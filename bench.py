@@ -23,6 +23,11 @@ K/V projections are computed on one rank only and the per-GPU K/V reuse does not
 by query block instead); ranks all-gather (position, score) pairs and every rank re-sorts.  After the timed region rank 0
 re-scores a sample of rows alone (single-GPU path) and the line carries the comparison (`cross_rank_check`).
 `--impl reference` times the reference's CPU implementation of the path instead (rank 0 only).
+
+`--dump-outputs DIR` writes what the last timed step returned, so that two builds can be compared output for output on
+the same seeded inputs: scores.npy [Q,K] float32, order.npy [Q,K] (re-ranked positions, as float32),
+recall_hits_at_10_50.npy [2] float64 and rows.npy (the query rows written, float64).  Above 64 MB in all, a fixed
+seeded sample of the query rows is written.
 """
 from __future__ import annotations
 
@@ -61,7 +66,12 @@ def parse():
     ap.add_argument("--cpu-sample-queries", type=int, default=4)      # ~13 s of CPU work on the box's 16 cores
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     q, k = JOBS[a.job]
     a.queries = a.queries or q
     a.k = a.k or k
@@ -133,6 +143,28 @@ def synth_workload(args, seed=0):
     return ref.int(), tgt, ids.int(), mask.int(), cand, labels
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, scores, order, hits, limit=DUMP_LIMIT_BYTES):
+    """Write one step's outputs as .npy files (float32 / float64).  When all rows would exceed ``limit`` bytes, a fixed
+    seeded sample of query rows is written instead; rows.npy names them."""
+    scores = np.asarray(scores, dtype=np.float32)
+    order = np.asarray(order, dtype=np.float32)          # positions < K <= 2**24: exact in float32
+    Q, K = scores.shape
+    per_row = K * 4 * 2 + 8
+    fixed = 16 + 4 * 128                                  # recall counters + .npy headers
+    rows = np.arange(Q)
+    if fixed + Q * per_row > limit:
+        n = max(0, (limit - fixed) // per_row)
+        rows = np.sort(np.random.default_rng(0).choice(Q, size=n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), scores[rows])
+    np.save(os.path.join(out_dir, "order.npy"), order[rows])
+    np.save(os.path.join(out_dir, "recall_hits_at_10_50.npy"), np.asarray(hits, dtype=np.float64))
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+
+
 def workload_text(args):
     return (f"stage2_rerank_{args.job}_shape: Q={args.queries} queries x K={args.k} candidates (whole job), L={args.length} tokens, "
             f"G={args.gallery} gallery images (577 ViT-B/16 tokens each, resident), z_t + stage-II + re-sort + recall")
@@ -140,8 +172,8 @@ def workload_text(args):
 
 # ----------------------------------------------------------------------------------------------- CPU arms
 def find_reference():
-    """The reference's own sources, if reachable (never on the GPU box): $CIR_REFERENCE, /root/reference, ./baseline/_ref."""
-    for p in (os.environ.get("CIR_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
+    """The reference's own sources, if reachable: $CIR_REFERENCE or ./baseline/_ref."""
+    for p in (os.environ.get("CIR_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
         if p and os.path.exists(os.path.join(p, "src", "blip_stage2.py")):
             return p
     return None
@@ -203,7 +235,7 @@ def run_reference(args, rank, emit):
     t0 = time.perf_counter()
     for i in range(args.steps):
         one(args.warmup + i)
-    dt = (time.perf_counter() - t0) / max(1, args.steps)
+    dt = (time.perf_counter() - t0) / args.steps
     v = K / dt
     sample = f"1 query x K={K} candidates per step (z_t + stage-II + sort), fp32, torch CPU {cores} threads; {note}"
     emit({"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -337,12 +369,14 @@ def main():
     prof = {k: eng.profile_read(k) for k in (N.PROF_GEMM, N.PROF_ATTN_TC, N.PROF_ATTN_SELF, N.PROF_LAYERNORM, N.PROF_QKV_ATTN)}
     gemm_ms, gemm_flops, gemm_n = prof[N.PROF_GEMM]
     plan = dict(eng.last_plan)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores_last.cpu().numpy(), order_last.cpu().numpy(), hits_last.cpu().numpy())
     step_e2e()
     eng.h2d_bytes = 0
-    ms_e2e, (r10, r50, order_host) = timed(step_e2e, max(1, args.steps))
+    ms_e2e, (r10, r50, order_host) = timed(step_e2e, args.steps)
     # bytes per step counted from the tensors the call copies: engine uploads (per-chunk lists, counted by the engine) +
     # int64 ids/mask (tokenize) + bool labels; D2H: the order [Q,K] int32 and two int64 counters
-    h2d = eng.h2d_bytes // max(1, args.steps) + 2 * Q * L * 8 + 2 * Q * L * 4 + Q * 4 + Q * K
+    h2d = eng.h2d_bytes // args.steps + 2 * Q * L * 8 + 2 * Q * L * 4 + Q * 4 + Q * K
     d2h = Q * K * 4 + 2 * 8
     sampler.stop_flag = True
     sampler.join(timeout=2)

@@ -42,12 +42,14 @@ def test_config1_scores_and_features_bf16(config1):
     rank_err = np.abs(d - d.mean(1, keepdims=True)).max()
     print(f"config1: max|dscore|={err.max():.2e} mean={err.mean():.2e} max in-row ranking error={rank_err:.2e} "
           f"(planted margin/2 = {float(g['margins'].min()) / 2:.2e})")
-    # 1536-d pre-head features of all 400 triplets, relative Frobenius error
+    # 1536-d pre-head features of all 400 triplets, relative Frobenius error over the fixture's seeded column sample
     ch = cir.schedule.plan_chunks(g["cand_idx"], None, 4096, 64)[0]
     assert ch.flat_pos.size == Q * K
     _, f = m2.engine.stage2_score_chunk(m2._w, tokens2, ch.cand_list, z_t, ids.cuda(), mask.cuda(), ch.trip_query, ch.trip_slot, want_feats=True)
-    want = torch.tensor(g["feats"].astype(np.float32)).reshape(-1, 1536)[torch.from_numpy(ch.flat_pos)]
-    rel = ((f.cpu() - want).norm() / want.norm()).item()
+    assert f.shape[1] == 1536
+    cols = torch.from_numpy(g["feats_cols"])
+    want = torch.tensor(g["feats"].astype(np.float32)).reshape(-1, cols.numel())[torch.from_numpy(ch.flat_pos)]
+    rel = ((f.cpu()[:, cols] - want).norm() / want.norm()).item()
     assert rel < 3e-2, rel
 
 
@@ -87,10 +89,10 @@ def test_config1_fp32_check_mode(config1):
     m2 = cir.blip_stage2.blip_stage2(image_size=384, state_dict=sd2, precision="fp32")
     tokens = m2.img_embed(golden_images(g))
     assert np.abs(tokens[:, 0, :].cpu().numpy() - g["tokens2_cls"]).max() < 2e-4
-    rows = [0, 5]
+    rows = g["z_t_rows"].tolist()                                            # queries 0 and 5
     ids, mask = torch.tensor(g["ids"][rows]), torch.tensor(g["mask"][rows])
     z_t, _ = m1.encode_queries(tokens, torch.tensor(g["ref_idx"][rows]).int(), ids, mask, want_z=True, want_emb=False)
-    assert np.abs(z_t.cpu().numpy() - g["z_t"][rows]).max() < 3e-4
+    assert np.abs(z_t.cpu().numpy() - g["z_t"]).max() < 3e-4
     s = m2.score_triplets(z_t, ids, mask, tokens, g["cand_idx"][rows])
     assert np.abs(s.cpu().numpy() - g["scores"][rows]).max() <= 1e-4
 
