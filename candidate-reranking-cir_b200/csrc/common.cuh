@@ -125,8 +125,15 @@ int cir_make_map_3d(cir_ctx* ctx, CUtensorMap* map, const void* base, int64_t d0
                     int b0, int b1, int b2);
 int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a);
 bool cir_qkv_attention_supported(const cir_ctx* ctx, int64_t L);   // qkv_attention.cu
-// stage1_topk_tc.cu: tensor-core candidate filter + exact fp32 re-check; *overflowed = 1 -> results invalid, use the fp32 path
+// stage1_topk_tc.cu: tensor-core candidate filter + exact fp32 re-check, per-query exact fallback on the device (never synchronises).
+// A gallery "view" is the fp32 rows, their bf16 copy and gmax = {max ||g||, max ||g - bf16(g)||} as float bits.
 bool cir_stage1_topk_tc_supported(const cir_ctx* ctx, int64_t Q, int64_t G, int64_t K);
-size_t cir_stage1_topk_tc_workspace_bytes(int64_t Q, int64_t G, int64_t K);
+size_t cir_stage1_topk_tc_workspace_bytes(int64_t Q, int64_t G, int64_t K);    // transient view + search
+size_t cir_stage1_tc_search_bytes(int64_t Q, int64_t K);
+// n more rows of a view: g_bf16[0..n) = bf16(g_emb[0..n)), gmax raised to cover them
+int cir_stage1_tc_convert(cir_ctx* ctx, const float* g_emb, int64_t n, bf16* g_bf16, uint32_t* gmax);
+int cir_stage1_tc_search(cir_ctx* ctx, const float* q_emb, int64_t Q, const float* g_emb, const bf16* g_bf16, int64_t G, const uint32_t* gmax,
+                         const int32_t* exclude, int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                         void* workspace, size_t workspace_bytes);
 int cir_stage1_topk_tc(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G, const int32_t* exclude, int64_t col_offset,
-                       int64_t K, float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes, int* overflowed);
+                       int64_t K, float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes);

@@ -4,6 +4,7 @@
 //   cir_rerank_sort      argsort(scores, descending)                 src/validate_stage2.py:53,174,190
 //   cir_topk_from_dist   K smallest of a distance row, minus `exclude` src/validate.py:58,203-210,257
 //   cir_stage1_topk      fused 1 - q @ G^T tiles + running top-K       src/validate.py:57-58,202-203
+//   cir_stage1_index_*   the same search over a resident gallery index (built once, grown by appends)
 //   cir_topk_merge       merge of per-shard (dist, idx) lists after the NCCL all-gather
 //   cir_recall_counts    sum(labels[:, :k]) over sorted labels         src/validate_stage2.py:56-62,178-203
 #include <algorithm>
@@ -248,20 +249,9 @@ extern "C" size_t cir_stage1_topk_workspace_bytes(int64_t Q, int64_t G, int64_t 
   return a > b ? a : b;
 }
 
-extern "C" int cir_stage1_topk(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G,
-                               const int32_t* exclude, int64_t col_offset, int64_t K,
-                               float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes) {
-  CIR_ENTER(ctx);
-  if (Q == 0) return CIR_OK;
-  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "stage1_topk: K=%lld out of range [1,%d]", (long long)K, MAXK);
-  if (workspace_bytes < cir_stage1_topk_workspace_bytes(Q, G, K)) { cir_set_error("stage1_topk: workspace too small"); return CIR_EWORKSPACE; }
-  if (cir_stage1_topk_tc_supported(ctx, Q, G, K)) {
-    // large gallery: candidate filter on the tensor cores + exact fp32 re-check (bit-identical results); an overflowing
-    // candidate list (adversarial gallery order / thousands of near-duplicates) falls through to the fp32 path below
-    int overflowed = 0;
-    CIR_TRY(cir_stage1_topk_tc(ctx, q_emb, g_emb, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace, workspace_bytes, &overflowed));
-    if (!overflowed) return CIR_OK;
-  }
+// fp32 CUDA-core path: similarity tiles of kSimChunk columns + running top-K (workspace: stage1_fp32_workspace_bytes)
+static int stage1_fp32(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G, const int32_t* exclude, int64_t col_offset,
+                       int64_t K, float* top_dist, int32_t* top_idx, void* workspace) {
   uint64_t* best = (uint64_t*)workspace;
   float* sim = (float*)((char*)workspace + cir_topk_workspace_bytes(Q, G, K));
   const int64_t gc = G < kSimChunk ? G : kSimChunk;
@@ -289,6 +279,86 @@ extern "C" int cir_stage1_topk(cir_ctx* ctx, const float* q_emb, const float* g_
     CIR_LAUNCH_CHECK(ctx);
   }
   return CIR_OK;
+}
+
+extern "C" int cir_stage1_topk(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G,
+                               const int32_t* exclude, int64_t col_offset, int64_t K,
+                               float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes) {
+  CIR_ENTER(ctx);
+  if (Q == 0) return CIR_OK;
+  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "stage1_topk: K=%lld out of range [1,%d]", (long long)K, MAXK);
+  if (workspace_bytes < cir_stage1_topk_workspace_bytes(Q, G, K)) { cir_set_error("stage1_topk: workspace too small"); return CIR_EWORKSPACE; }
+  // large gallery: candidate filter on the tensor cores + exact fp32 re-check (bit-identical results); queries whose candidate
+  // list overflows (adversarial gallery order / thousands of near-duplicates) get an exact scan on the device
+  if (cir_stage1_topk_tc_supported(ctx, Q, G, K))
+    return cir_stage1_topk_tc(ctx, q_emb, g_emb, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace, workspace_bytes);
+  return stage1_fp32(ctx, q_emb, g_emb, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace);
+}
+
+// ---- resident stage-I index: blob = [capacity,256] fp32 rows | [capacity,256] bf16 copy (bf16 contexts) | gmax (256 B)
+static const int64_t kTcMinRows = 16384;    // cir_stage1_topk_tc_supported's gallery threshold
+
+extern "C" size_t cir_stage1_index_bytes(const cir_ctx* ctx, int64_t capacity) {
+  if (!ctx || capacity < 0) return 0;
+  const size_t b = ctx->dtype == CIR_DTYPE_BF16 ? align_up((size_t)capacity * CIR_EMBED * 2, 256) : 0;
+  return align_up((size_t)capacity * CIR_EMBED * 4, 256) + b + 256;
+}
+
+extern "C" int cir_stage1_index_init(cir_ctx* ctx, void* blob, size_t bytes, int64_t capacity, cir_stage1_index* out) {
+  CIR_CHECK_ARG(ctx && out && blob, "stage1_index_init: null argument");
+  CIR_CHECK_ARG(capacity >= 0 && capacity < (1ll << 31), "stage1_index_init: capacity=%lld out of range [0,2^31)", (long long)capacity);
+  CIR_CHECK_ARG(((uintptr_t)blob & 255) == 0, "stage1_index_init: blob must be 256-byte aligned");
+  const size_t need = cir_stage1_index_bytes(ctx, capacity);
+  if (bytes < need) { cir_set_error("stage1_index_init: blob %zu < %zu bytes", bytes, need); return CIR_EWORKSPACE; }
+  CIR_ENTER(ctx);
+  char* base = (char*)blob;
+  const size_t f32 = align_up((size_t)capacity * CIR_EMBED * 4, 256);
+  out->capacity = capacity;
+  out->rows = 0;
+  out->g_f32 = (float*)base;
+  out->g_bf16 = ctx->dtype == CIR_DTYPE_BF16 ? (void*)(base + f32) : nullptr;
+  out->gmax = (uint32_t*)(base + need - 256);
+  CIR_CUDA(cudaMemsetAsync(out->gmax, 0, 2 * sizeof(uint32_t), ctx->stream));
+  return CIR_OK;
+}
+
+extern "C" int cir_stage1_index_add(cir_ctx* ctx, cir_stage1_index* index, const float* g_emb, int64_t n) {
+  CIR_CHECK_ARG(ctx && index && (g_emb || n == 0), "stage1_index_add: null argument");
+  CIR_CHECK_ARG(n >= 0 && index->rows + n <= index->capacity, "stage1_index_add: %lld rows + %lld exceed the capacity %lld",
+                (long long)index->rows, (long long)n, (long long)index->capacity);
+  if (n == 0) return CIR_OK;
+  CIR_ENTER(ctx);
+  float* dst = index->g_f32 + index->rows * CIR_EMBED;
+  CIR_CUDA(cudaMemcpyAsync(dst, g_emb, (size_t)n * CIR_EMBED * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+  if (index->g_bf16) CIR_TRY(cir_stage1_tc_convert(ctx, dst, n, (bf16*)index->g_bf16 + index->rows * CIR_EMBED, index->gmax));
+  index->rows += n;
+  return CIR_OK;
+}
+
+extern "C" size_t cir_stage1_index_topk_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* index, int64_t Q, int64_t K) {
+  (void)ctx;
+  if (!index || Q < 0 || K < 1 || K > MAXK) return 0;
+  // sized for every row count up to the capacity, so that a workspace stays valid while the index grows
+  const size_t a = stage1_fp32_workspace_bytes(Q, index->capacity, K);
+  const size_t b = (index->g_bf16 && index->capacity >= kTcMinRows) ? cir_stage1_tc_search_bytes(Q, K) : 0;
+  return a > b ? a : b;
+}
+
+extern "C" int cir_stage1_index_topk(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const int32_t* exclude,
+                                     int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                                     void* workspace, size_t workspace_bytes) {
+  CIR_CHECK_ARG(ctx && index, "stage1_index_topk: null argument");
+  CIR_ENTER(ctx);
+  if (Q == 0) return CIR_OK;
+  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "stage1_index_topk: K=%lld out of range [1,%d]", (long long)K, MAXK);
+  const size_t need = cir_stage1_index_topk_workspace_bytes(ctx, index, Q, K);
+  if (workspace_bytes < need) { cir_set_error("stage1_index_topk: workspace %zu < %zu bytes", workspace_bytes, need); return CIR_EWORKSPACE; }
+  const int64_t G = index->rows;
+  if (index->g_bf16 && cir_stage1_topk_tc_supported(ctx, Q, G, K))
+    return cir_stage1_tc_search(ctx, q_emb, Q, index->g_f32, (const bf16*)index->g_bf16, G, index->gmax, exclude, col_offset, K, top_dist,
+                                top_idx, exact_rows, workspace, workspace_bytes);
+  if (exact_rows) CIR_CUDA(cudaMemsetAsync(exact_rows, 0, (size_t)Q * sizeof(int32_t), ctx->stream));
+  return stage1_fp32(ctx, q_emb, index->g_f32, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace);
 }
 
 __global__ void divide_rows_kernel(float* __restrict__ x, int64_t n, float d) {

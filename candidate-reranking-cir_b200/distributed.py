@@ -10,7 +10,8 @@ independent, the stage-I gallery splits by rows; ranks exchange only (score, ind
              (b) query partition: each rank scores its [Q_r, K] block (K/V of a candidate recomputed on every rank whose
              queries name it); one all-gather of the padded score blocks.
   stage I  : gallery rows block-partitioned; each rank computes a local top-K with global column ids
-             (``col_offset``); one all-gather of [Q, K] (distance, index) lists; ``cir_topk_merge``.
+             (``col_offset``); one all-gather of [Q, K] (distance, index) lists; ``cir_topk_merge``.  ``ShardedStage1Index``
+             keeps each rank's block resident (built once from that block only) for repeated query batches.
 
 The compute steps are injected callables so the same code runs under ``gloo`` on CPU in the tests
 (with the oracle standing in for the kernels) and under ``nccl`` on GPUs (with the engine).
@@ -145,3 +146,24 @@ def stage1_topk_gpu(engine, q_emb, g_emb, k: int, exclude=None):
     def local(rows: slice):
         return engine.stage1_topk(q_emb, g_emb[rows], k, exclude=exclude, col_offset=rows.start)
     return sharded_stage1_topk(local, engine.topk_merge, g_emb.shape[0])
+
+
+class ShardedStage1Index:
+    """Resident stage-I index over the ranks of the default process group: each rank indexes only its ``shard_rows`` block of
+    the gallery, searches it with ``col_offset = block.start`` (global row ids), and the lists meet in ``sharded_stage1_topk``
+    + ``topk_merge``.  No rank holds the full gallery.  ``rows_of(block)`` -> fp32 [len(block), 256] gallery rows of that block
+    (e.g. a slice of ``extract_index_features`` output, or rows read from storage)."""
+
+    def __init__(self, engine, gallery_rows: int, rows_of: Callable[[slice], torch.Tensor]):
+        rank, ws = world()
+        self.engine, self.gallery_rows = engine, gallery_rows
+        self.block = shard_rows(gallery_rows, rank, ws)
+        self.index = engine.stage1_index(self.block.stop - self.block.start)
+        self.index.add(rows_of(self.block))
+
+    def topk(self, q_emb, k: int, exclude=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """-> merged (dist [Q,k], idx [Q,k]) on every rank; ``q_emb`` and ``exclude`` cover all Q queries (global row ids)."""
+        def local(rows: slice):
+            assert rows == self.block
+            return self.index.topk(q_emb, k, exclude=exclude, col_offset=rows.start)
+        return sharded_stage1_topk(local, self.engine.topk_merge, self.gallery_rows)

@@ -477,6 +477,11 @@ class Engine:
                                           N.ptr(ti), N.ptr(ws), ws.numel()), "cir_stage1_topk")
         return td, ti
 
+    def stage1_index(self, capacity: int) -> "Stage1Index":
+        """An empty resident stage-I gallery index for up to ``capacity`` rows (cir_stage1_index): fill it with
+        :meth:`Stage1Index.add` once, search it with :meth:`Stage1Index.topk` for every query batch."""
+        return Stage1Index(self, capacity)
+
     def stage1_rank_members(self, q_emb: torch.Tensor, g_emb: torch.Tensor, members):
         """members int [Q,P] gallery rows -> (dist fp32 [Q,P], order int32 [Q,P]: slot of the r-th closest member)."""
         q_emb = q_emb.to(self.device, torch.float32).contiguous()
@@ -607,6 +612,72 @@ class Engine:
             N.ptr(gamma.float().contiguous()), N.ptr(beta.float().contiguous()), rows_per_group or rows, N.ptr(y),
             1 if y.dtype == torch.float32 else 0, rows, eps), "cir_add_layernorm")
         return y
+
+
+class Stage1Index:
+    """Resident stage-I gallery index (``cir_stage1_index`` in include/cir_b200.h): gallery embeddings fp32 [n,256] are copied
+    and, in bf16 engines, converted to bf16 once, when they are added; every search reuses them.  ``topk`` returns exactly what
+    :meth:`Engine.stage1_topk` returns over the same rows, bit for bit.
+
+    ``topk`` never synchronises.  Given device tensors (q_emb fp32 contiguous, exclude int32) and ``out=``, it allocates and
+    uploads nothing once its workspace exists for that (Q, k) -- run it once before ``torch.cuda.graph`` capture.  A captured
+    graph searches the rows the index had at capture time."""
+
+    def __init__(self, eng: Engine, capacity: int):
+        self.eng = eng
+        self._blob = torch.empty(max(1, eng._lib.cir_stage1_index_bytes(eng.ctx, capacity)), dtype=torch.uint8, device=eng.device)
+        self._s = N.Stage1Index()
+        self._ws: Optional[torch.Tensor] = None
+        self._retired: List[torch.Tensor] = []    # outgrown workspaces stay alive: a captured graph may still point at one
+        eng._sync_stream()
+        N.check(eng._lib.cir_stage1_index_init(eng.ctx, N.ptr(self._blob), self._blob.numel(), capacity, C.byref(self._s)),
+                "cir_stage1_index_init")
+
+    @property
+    def capacity(self) -> int:
+        return int(self._s.capacity)
+
+    @property
+    def rows(self) -> int:
+        return int(self._s.rows)
+
+    @property
+    def g_f32(self) -> torch.Tensor:
+        """fp32 [rows, 256] view of the indexed rows (the blob starts with them; no copy)."""
+        n = self.rows
+        return self._blob[: n * EMBED * 4].view(torch.float32).view(n, EMBED)
+
+    def add(self, g_emb: torch.Tensor) -> "Stage1Index":
+        """Append gallery rows fp32 [n,256] (host or device); only the new rows are converted."""
+        g = g_emb.to(self.eng.device, torch.float32).contiguous()
+        assert g.dim() == 2 and g.shape[1] == EMBED, g.shape
+        self.eng._sync_stream()
+        N.check(self.eng._lib.cir_stage1_index_add(self.eng.ctx, C.byref(self._s), N.ptr(g), g.shape[0]), "cir_stage1_index_add")
+        return self
+
+    def topk(self, q_emb: torch.Tensor, k: int, exclude=None, col_offset: int = 0, out=None, exact_rows: Optional[torch.Tensor] = None):
+        """-> (dist fp32 [Q,k], idx int32 [Q,k]) of the k nearest indexed rows (global index = col_offset + row), skipping
+        exclude[q] (-1 = none).  ``out``: optional (dist, idx) to fill.  ``exact_rows``: optional int32 [Q] device tensor, set to 1
+        for the queries whose list came from the exact fallback scan."""
+        eng = self.eng
+        q = q_emb.to(eng.device, torch.float32).contiguous()
+        Q = q.shape[0]
+        if out is None:
+            out = (torch.empty(Q, k, dtype=torch.float32, device=eng.device), torch.empty(Q, k, dtype=torch.int32, device=eng.device))
+        td, ti = out
+        assert td.shape == ti.shape == (Q, k) and td.dtype == torch.float32 and ti.dtype == torch.int32
+        assert td.is_contiguous() and ti.is_contiguous()
+        assert exact_rows is None or (exact_rows.dtype == torch.int32 and exact_rows.numel() == Q and exact_rows.is_contiguous())
+        ex = None if exclude is None else eng._i32(exclude)
+        need = eng._lib.cir_stage1_index_topk_workspace_bytes(eng.ctx, C.byref(self._s), Q, k)
+        if self._ws is None or self._ws.numel() < need:
+            if self._ws is not None:
+                self._retired.append(self._ws)
+            self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=eng.device)
+        eng._sync_stream()
+        N.check(eng._lib.cir_stage1_index_topk(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(ex), col_offset, k, N.ptr(td), N.ptr(ti),
+                                               N.ptr(exact_rows), N.ptr(self._ws), self._ws.numel()), "cir_stage1_index_topk")
+        return td, ti
 
 
 _engines: Dict[Tuple[int, str], Engine] = {}

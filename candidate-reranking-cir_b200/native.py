@@ -49,6 +49,10 @@ class QkvAttnArgs(C.Structure):
                 ("key_mask", vp), ("mask_index", vp), ("captions", i64), ("L", i32), ("batch", i32), ("scale", C.c_float)]
 
 
+class Stage1Index(C.Structure):
+    _fields_ = [("capacity", i64), ("rows", i64), ("g_f32", vp), ("g_bf16", vp), ("gmax", vp)]
+
+
 _A = vp * LAYERS
 
 
@@ -148,6 +152,11 @@ _SIGS = {
     "cir_topk_workspace_bytes": (C.c_size_t, [i64, i64, i64]),
     "cir_stage1_topk": (C.c_int, [vp, vp, vp, i64, i64, vp, i64, i64, vp, vp, vp, C.c_size_t]),
     "cir_stage1_topk_workspace_bytes": (C.c_size_t, [i64, i64, i64]),
+    "cir_stage1_index_bytes": (C.c_size_t, [vp, i64]),
+    "cir_stage1_index_init": (C.c_int, [vp, vp, C.c_size_t, i64, C.POINTER(Stage1Index)]),
+    "cir_stage1_index_add": (C.c_int, [vp, C.POINTER(Stage1Index), vp, i64]),
+    "cir_stage1_index_topk_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage1Index), i64, i64]),
+    "cir_stage1_index_topk": (C.c_int, [vp, C.POINTER(Stage1Index), vp, i64, vp, i64, i64, vp, vp, vp, vp, C.c_size_t]),
     "cir_stage1_logits": (C.c_int, [vp, vp, vp, i64, i64, C.c_float, vp]),
     "cir_stage1_rank_members": (C.c_int, [vp, vp, vp, vp, i64, i64, vp, vp]),
     "cir_topk_merge": (C.c_int, [vp, vp, vp, i64, i64, i64, vp, vp, vp, C.c_size_t]),

@@ -72,14 +72,30 @@ def query_embeddings(blip_model, dataset, index_features, index_names, cirr: boo
     return q_emb, ref_idx
 
 
+def _stage1_search(eng, q_emb, g_emb, k, exclude, index):
+    """top-k of the gallery rows: through the resident ``index`` (engine.Stage1Index) when given, else over ``g_emb``."""
+    if index is not None:
+        return index.topk(q_emb, k, exclude=exclude)
+    return eng.stage1_topk(q_emb, g_emb, k, exclude=exclude)
+
+
+def _gallery(index_features_normed_pooled, index_names, index):
+    """fp32 gallery embeddings ("already normed", :55,:199): the index's own rows when an index is given."""
+    if index is None:
+        return index_features_normed_pooled.float()
+    assert index.rows == len(index_names), f"stage-I index holds {index.rows} rows, the gallery has {len(index_names)} names"
+    return index.g_f32
+
+
 def retrieve_topk(blip_model, dataset, index_features, index_features_normed_pooled, index_names, k: int, cirr: bool,
-                  return_embeddings: bool = False):
+                  return_embeddings: bool = False, index=None):
     """Query embeddings + fused distance/top-K (src/validate.py:57-58,202-210,257).  Returns (top_dist fp32 [Q,k],
-    top_idx int32 [Q,k]) on device; CIRR excludes each query's own reference image."""
+    top_idx int32 [Q,k]) on device; CIRR excludes each query's own reference image.  ``index``: an engine.Stage1Index built
+    from ``index_features_normed_pooled`` (which may then be None) -- same results, without per-call gallery conversion."""
     eng = blip_model.engine
     q_emb, ref_idx = query_embeddings(blip_model, dataset, index_features, index_names, cirr)
-    g_emb = index_features_normed_pooled.float()                                    # "already normed" (:55,:199)
-    td, ti = eng.stage1_topk(q_emb, g_emb, k, exclude=ref_idx if cirr else None)
+    g_emb = _gallery(index_features_normed_pooled, index_names, index)
+    td, ti = _stage1_search(eng, q_emb, g_emb, k, ref_idx if cirr else None, index)
     return (td, ti, q_emb, g_emb, ref_idx) if return_embeddings else (td, ti)
 
 
@@ -96,11 +112,12 @@ def _names_of(index_names, top_idx: torch.Tensor) -> np.ndarray:
     return np.array(index_names)[idx]
 
 
-def fiq_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k: int = 100):
-    """-> ((recall@10, recall@50), top-K dict shaped like the file written at src/validate.py:87-94)."""
+def fiq_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k: int = 100, index=None):
+    """-> ((recall@10, recall@50), top-K dict shaped like the file written at src/validate.py:87-94).  ``index``: see retrieve_topk."""
     eng = blip_model.engine
     k = min(max(k, 50), len(index_names))
-    _, top_idx = retrieve_topk(blip_model, relative_val_dataset, index_features, index_features_normed_pooled, index_names, k, cirr=False)
+    _, top_idx = retrieve_topk(blip_model, relative_val_dataset, index_features, index_features_normed_pooled, index_names, k, cirr=False,
+                               index=index)
     n2i = _name_index(index_names)
     tgt = np.array([n2i[n] for n in relative_val_dataset.target_names])
     labels, (r10, r50) = _labels_and_recalls(eng, top_idx, tgt, (10, 50))
@@ -110,13 +127,16 @@ def fiq_val_topk(relative_val_dataset, blip_model, index_features, index_feature
     return (r10, r50), topk
 
 
-def cirr_topk_from_embeddings(eng, q_emb, g_emb, ref_idx, target_idx, group_idx_noref, k: int):
+def cirr_topk_from_embeddings(eng, q_emb, g_emb, ref_idx, target_idx, group_idx_noref, k: int, index=None):
     """The index arithmetic of src/validate.py:202-226 on the GPU, from query / gallery embeddings:
     top-k gallery rows per query without the reference (ascending distance), labels, and ``group_labels`` [Q,5] = the labels
-    of the group members in stage-I ranking order (``labels[group_mask]``, :213-218).
+    of the group members in stage-I ranking order (``labels[group_mask]``, :213-218).  ``index``: an engine.Stage1Index of
+    the gallery, searched instead of ``g_emb`` (which may then be None).
     -> (top_idx int32 [Q,k], labels bool [Q,k], group_labels bool [Q,P], group_order int32 [Q,P]) on device."""
     ref_idx = np.asarray(ref_idx, dtype=np.int32)
-    _, top_idx = eng.stage1_topk(q_emb, g_emb, k, exclude=ref_idx)
+    if index is not None:
+        g_emb = index.g_f32
+    _, top_idx = _stage1_search(eng, q_emb, g_emb, k, ref_idx, index)
     tgt = torch.as_tensor(np.asarray(target_idx), device=eng.device)
     labels = top_idx.to(torch.int64) == tgt[:, None]
     members = torch.as_tensor(np.asarray(group_idx_noref), dtype=torch.int64)
@@ -126,21 +146,21 @@ def cirr_topk_from_embeddings(eng, q_emb, g_emb, ref_idx, target_idx, group_idx_
     return top_idx, labels, group_labels, gorder
 
 
-def cirr_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k: int = 50):
+def cirr_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k: int = 50, index=None):
     """-> ((group_recall@1,2,3, recall@1,5,10,50), top-K dict shaped like the file written at src/validate.py:256-263,
-    including ``group_labels``, which the reference's CIRR reader requires: src/data_utils.py:301)."""
+    including ``group_labels``, which the reference's CIRR reader requires: src/data_utils.py:301).  ``index``: see retrieve_topk."""
     ds = relative_val_dataset
     eng = blip_model.engine
     k = min(max(k, 50), len(index_names) - 1)          # the reference image is removed from every row (:207-210)
     q_emb, ref_idx = query_embeddings(blip_model, ds, index_features, index_names, cirr=True)
-    g_emb = index_features_normed_pooled.float()
+    g_emb = _gallery(index_features_normed_pooled, index_names, index)
     n2i = _name_index(index_names)
     tgt = np.array([n2i[n] for n in ds.target_names])
     gm = np.asarray(ds.group_members)
     refs = np.asarray(ds.reference_names)
     group_noref = [[n2i[m] for m in row if m != r] for row, r in zip(gm.tolist(), refs.tolist())]   # the reference never matches (:214)
     assert all(len(g) == len(group_noref[0]) for g in group_noref), "every img_set must have the same number of members"
-    top_idx, labels, group_labels, _ = cirr_topk_from_embeddings(eng, q_emb, g_emb, ref_idx, tgt, group_noref, k)
+    top_idx, labels, group_labels, _ = cirr_topk_from_embeddings(eng, q_emb, g_emb, ref_idx, tgt, group_noref, k, index=index)
     Q = len(tgt)
     if k == len(index_names) - 1:                       # the reference asserts on the FULL ranking (:221-222)
         assert torch.equal(labels.sum(-1).int().cpu(), torch.ones(Q).int())
@@ -156,19 +176,22 @@ def cirr_val_topk(relative_val_dataset, blip_model, index_features, index_featur
 
 
 def compute_fiq_val_metrics(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names,
-                            k: int = 100, save_topk_path: Optional[str] = None) -> Tuple[float, float]:
+                            k: int = 100, save_topk_path: Optional[str] = None, index=None) -> Tuple[float, float]:
     """src/validate.py:33-99 -> (recall@10, recall@50).  ``save_topk_path`` plays the role of the reference's SAVE_TOPK /
-    K_VALUE globals (:82-97): the top-``k`` file is written there."""
-    metrics, topk = fiq_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k)
+    K_VALUE globals (:82-97): the top-``k`` file is written there.  ``index``: see retrieve_topk."""
+    metrics, topk = fiq_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k, index=index)
     if save_topk_path:
         save_topk(save_topk_path, topk)
     return metrics
 
 
 def compute_cirr_val_metrics(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names,
-                             k: int = 50, save_topk_path: Optional[str] = None) -> Tuple[float, float, float, float, float, float, float]:
-    """src/validate.py:176-268 -> (group_recall@1, @2, @3, recall@1, @5, @10, @50), the reference's order (:268)."""
-    metrics, topk = cirr_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k)
+                             k: int = 50, save_topk_path: Optional[str] = None,
+                             index=None) -> Tuple[float, float, float, float, float, float, float]:
+    """src/validate.py:176-268 -> (group_recall@1, @2, @3, recall@1, @5, @10, @50), the reference's order (:268).
+    ``index``: see retrieve_topk."""
+    metrics, topk = cirr_val_topk(relative_val_dataset, blip_model, index_features, index_features_normed_pooled, index_names, k,
+                                  index=index)
     if save_topk_path:
         save_topk(save_topk_path, topk)
     return metrics

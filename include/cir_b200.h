@@ -79,9 +79,9 @@ int  cir_set_dedup_first_layer(cir_ctx* ctx, int enable);
 /* bf16 mode, captions of 8, 16, 24 or 32 tokens: the query/key/value Linears and the masked text self-attention run as ONE kernel
  * (cir_qkv_attention) -- the [rows, 2304] projection never reaches HBM.  Default on; 0 = GEMM + attention kernel (bit-equal). */
 int  cir_set_fuse_qkv_attention(cir_ctx* ctx, int enable);
-/* bf16 contexts, galleries of >= 16,384 rows: cir_stage1_topk computes the similarities on the tensor cores (bf16 operands) only to
- * FILTER candidates with a rigorous error margin, then re-computes the survivors in fp32 -- results are bit-identical to the
- * fp32 path.  Default on; 0 = fp32 CUDA-core similarities for every gallery row. */
+/* bf16 contexts, galleries of >= 16,384 rows: cir_stage1_topk and cir_stage1_index_topk compute the similarities on the tensor
+ * cores (bf16 operands) only to FILTER candidates with a rigorous error margin, then re-compute the survivors in fp32 -- results
+ * are bit-identical to the fp32 path.  Default on; 0 = fp32 CUDA-core similarities for every gallery row. */
 int  cir_set_stage1_tensor_cores(cir_ctx* ctx, int enable);
 /* 1 (default): bf16 GEMM outputs leave the tcgen05 epilogue through TMA bulk tensor stores; 0: per-lane 16 B stores. */
 int  cir_set_gemm_tma_store(cir_ctx* ctx, int enable);
@@ -209,6 +209,31 @@ int cir_stage1_topk(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_
                     const int32_t* exclude, int64_t col_offset, int64_t K,
                     float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes);
 size_t cir_stage1_topk_workspace_bytes(int64_t Q, int64_t G, int64_t K);
+
+/* Resident stage-I gallery index: the gallery embeddings (the `index_features` of src/utils.py:56-70, pooled and normalised)
+ * converted once and searched by many query batches (src/validate.py:198-203).  A search returns exactly what cir_stage1_topk
+ * returns over the same rows, bit for bit.  The blob (cir_stage1_index_bytes, 256-byte aligned) is owned by the caller; the struct
+ * points into it.  _init and _add enqueue work on the context's stream.
+ *   _add appends n rows (device fp32 [n,256]): copies them and, in bf16 contexts, converts only the new rows to bf16 and raises
+ *        the gallery maxima the filter bound uses.  Past `capacity`: CIR_EINVAL.  `rows` counts on the host.
+ *   _topk searches the first `rows` rows with the tensor-core filter (bf16 context, cir_set_stage1_tensor_cores on, rows >= 16,384)
+ *        or the fp32 tile loop, chosen per call.  It never synchronises and never copies to the host, so it can be captured in a
+ *        CUDA graph; a graph captured before an _add still searches the row count of its capture.  exact_rows (optional, [Q]):
+ *        1 where a query's candidate list overflowed and its list came from the exact scan of the whole index, else 0.
+ *        The workspace size depends on the capacity, not on `rows`: one workspace serves the index as it grows. */
+typedef struct cir_stage1_index {
+  int64_t capacity, rows;   /* rows added so far (host-side count) */
+  float*  g_f32;            /* [capacity,256] fp32 rows, owned copy (the exact re-check reads them) */
+  void*   g_bf16;           /* [capacity,256] bf16 copy; NULL in fp32 contexts */
+  uint32_t* gmax;           /* device: {max ||g||, max ||g - bf16(g)||} as float bits, updated by _add only */
+} cir_stage1_index;
+size_t cir_stage1_index_bytes(const cir_ctx* ctx, int64_t capacity);
+int    cir_stage1_index_init(cir_ctx* ctx, void* blob, size_t bytes, int64_t capacity, cir_stage1_index* out);
+int    cir_stage1_index_add(cir_ctx* ctx, cir_stage1_index* index, const float* g_emb, int64_t n);
+size_t cir_stage1_index_topk_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* index, int64_t Q, int64_t K);
+int    cir_stage1_index_topk(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const int32_t* exclude,
+                             int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                             void* workspace, size_t workspace_bytes);
 
 /* In-batch contrastive logits of the stage-I forward: logits[Q, G] = q_emb[Q,256] @ t_emb[G,256]^T / temp, all fp32.
  * Replaces `predicted_features @ target_features.T / self.temp` (src/blip_stage1.py:90-91), forward only. */
