@@ -109,11 +109,14 @@ __device__ __forceinline__ float warp_max(float v) {
 
 // Threshold filter of the tcgen05 similarity tiles (stage-I top-K): every accumulator S[row, col] >= thr[row] is appended to the
 // row's candidate list, cand[row * cap + atomicAdd(count[row])] = {col_base + col, float bits of S}; a full list raises *overflow.
+// col_tags [N] / row_masks [M] (both or neither): only columns with (col_tags[col] & row_masks[row]) != 0 are appended (a separate
+// kernel instantiation, so the untagged filter keeps its code).
 struct cir_gemm_filter {
   const float* thr; int32_t* count; uint2* cand; int32_t* overflow;
   int64_t cap; int64_t col_base;
 };
-int cir_gemm_tcgen05_filter(cir_ctx* ctx, const void* A, const void* W, int64_t M, int64_t N, int64_t K, const cir_gemm_filter* f);
+int cir_gemm_tcgen05_filter(cir_ctx* ctx, const void* A, const void* W, int64_t M, int64_t N, int64_t K, const cir_gemm_filter* f,
+                            const uint32_t* col_tags = nullptr, const uint32_t* row_masks = nullptr);
 
 // internal cross-file entry points
 int cir_gemm_simt(cir_ctx* ctx, const cir_gemm_args* a);
@@ -132,8 +135,9 @@ size_t cir_stage1_topk_tc_workspace_bytes(int64_t Q, int64_t G, int64_t K);    /
 size_t cir_stage1_tc_search_bytes(int64_t Q, int64_t K);
 // n more rows of a view: g_bf16[0..n) = bf16(g_emb[0..n)), gmax raised to cover them
 int cir_stage1_tc_convert(cir_ctx* ctx, const float* g_emb, int64_t n, bf16* g_bf16, uint32_t* gmax);
+// row_tags [G] / query_masks [Q] (both or neither): only rows with (row_tags[r] & query_masks[q]) != 0 are searched for query q
 int cir_stage1_tc_search(cir_ctx* ctx, const float* q_emb, int64_t Q, const float* g_emb, const bf16* g_bf16, int64_t G, const uint32_t* gmax,
-                         const int32_t* exclude, int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
-                         void* workspace, size_t workspace_bytes);
+                         const uint32_t* row_tags, const uint32_t* query_masks, const int32_t* exclude, int64_t col_offset, int64_t K,
+                         float* top_dist, int32_t* top_idx, int32_t* exact_rows, void* workspace, size_t workspace_bytes);
 int cir_stage1_topk_tc(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G, const int32_t* exclude, int64_t col_offset,
                        int64_t K, float* top_dist, int32_t* top_idx, void* workspace, size_t workspace_bytes);

@@ -52,6 +52,9 @@ struct Params {
   // to the row's candidate list as (global column, value bits)
   cir_gemm_filter flt;
   int32_t n_major;         // 1: tiles ordered n-block major (all m-blocks of a W block side by side: W streams from HBM once)
+  // tagged filter (TAGS kernels): column c may enter row r's list only if (flt_col_tags[c] & flt_row_masks[r]) != 0.
+  // Last in the struct: the offsets of every other field, hence the untagged kernels, do not move.
+  const uint32_t* flt_col_tags; const uint32_t* flt_row_masks;
 };
 
 // tile sequence of one worker: plain round-robin over tiles
@@ -103,10 +106,12 @@ __device__ __forceinline__ void gelu_fast2(float& x0, float& x1) {
 }
 
 // ----------------------------------------------------------------------------- the kernel
-template <int BN, bool PAIR, bool FILT>
+// TAGS (FILT only): the threshold filter also tests the column's tag against the row's mask before a hit reserves a slot
+template <int BN, bool PAIR, bool FILT, bool TAGS>
 __global__ void __launch_bounds__(THREADS, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w,
                     const __grid_constant__ CUtensorMap map_c, const Params p) {
+  static_assert(FILT || !TAGS, "tags belong to the threshold filter");
   using C = Cfg<BN, PAIR>;
   constexpr int TILE_M = PAIR ? 2 * BM : BM;                 // rows of one scheduled tile
   const uint32_t rank = PAIR ? cluster_ctarank() : 0u;       // 0 = leader (issues the MMAs)
@@ -258,6 +263,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
       const int64_t ntile0 = (int64_t)n_blk * BN;
       float flt_thr = INFINITY;
       if constexpr (FILT) { if (row_ok) flt_thr = __ldg(p.flt.thr + row); }
+      uint32_t flt_mask = 0u;
+      if constexpr (TAGS) { if (row_ok) flt_mask = __ldg(p.flt_row_masks + row); }
       if (!FILT && etid < BN) {
         const int64_t n = ntile0 + etid;
         sbias[acc * BN + etid] = (p.bias && n < p.N) ? __ldg(p.bias + b * p.bias_bstride + n) : 0.f;
@@ -319,10 +326,32 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
               c3 = fmaxf(fmaxf(c3, __uint_as_float(v[24 + j])), __uint_as_float(v[24 + (j + 1 < 8 ? j + 1 : j)]));
             }
             const float mx = fmaxf(fmaxf(c0, c1), fmaxf(c2, c3));
+            // TAGS: the chunk's 32 column tags (one 128-byte load by the whole warp, only when some lane passed the max test) are
+            // staged in this warp's slot of the (unused) bias area, where each hit lane reads them by index
+            const uint32_t* stags = reinterpret_cast<const uint32_t*>(sbias) + ew * 32;
+            if constexpr (TAGS) {
+              if (__any_sync(0xffffffffu, mx >= flt_thr)) {
+                const int64_t c = nbase + lane;
+                const uint32_t t = c < p.N ? __ldg(p.flt_col_tags + c) : 0u;
+                __syncwarp();                                                // the previous chunk's readers are done
+                const_cast<uint32_t*>(stags)[lane] = t;
+                __syncwarp();
+              }
+            }
             if (mx >= flt_thr) {
               uint32_t mask = 0u;
 #pragma unroll
               for (int j = 0; j < 32; j++) mask |= (__uint_as_float(v[j]) >= flt_thr ? 1u : 0u) << j;
+              if constexpr (TAGS) {                                          // eligibility before the atomicAdd reserves slots
+                uint32_t elig = 0u;
+#pragma unroll
+                for (int j = 0; j < 32; j += 4) {
+                  const uint4 t = *reinterpret_cast<const uint4*>(stags + j);
+                  elig |= ((t.x & flt_mask) ? 1u : 0u) << j | ((t.y & flt_mask) ? 1u : 0u) << (j + 1) |
+                          ((t.z & flt_mask) ? 1u : 0u) << (j + 2) | ((t.w & flt_mask) ? 1u : 0u) << (j + 3);
+                }
+                mask &= elig;
+              }
               const int64_t left = p.N - nbase;                              // columns of this chunk inside the matrix
               if (left < 32) mask &= left <= 0 ? 0u : ((1u << left) - 1u);
               const uint32_t mine = stg + (uint32_t)lane * 128;
@@ -583,13 +612,15 @@ static int make_map_c(cir_ctx* ctx, CUtensorMap* map, const void* base, int64_t 
   return cir_make_map_3d(ctx, map, base, N, M, batch, ldc, c_bstride, 64, 32, 1);
 }
 
-template <int BN, bool PAIR, bool FILT = false>
+template <int BN, bool PAIR, bool FILT = false, bool TAGS = false>
 static int launch_tc(cir_ctx* ctx, const tc::Params& p, const CUtensorMap& ma, const CUtensorMap& mw, const CUtensorMap& mc) {
   using C = tc::Cfg<BN, PAIR>;
-  const unsigned bit = FILT ? 1u << (26 + (BN == 128 ? 0 : 1) + (PAIR ? 1 : 0))
+  const auto kernel = tc::gemm_tcgen05_kernel<BN, PAIR, FILT, TAGS>;
+  const unsigned bit = TAGS ? 1u << (12 + (PAIR ? 1 : 0))
+                     : FILT ? 1u << (26 + (BN == 128 ? 0 : 1) + (PAIR ? 1 : 0))
                             : 1u << (8 + (BN == 128 ? 0 : 1) + (PAIR ? 2 : 0));   // per context: the attribute is per device
   if (!(ctx->func_attr_mask & bit)) {
-    CIR_CUDA(cudaFuncSetAttribute(tc::gemm_tcgen05_kernel<BN, PAIR, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+    CIR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     ctx->func_attr_mask |= bit;
   }
   const int slots = PAIR ? ctx->num_sms / 2 : ctx->num_sms;
@@ -607,7 +638,7 @@ static int launch_tc(cir_ctx* ctx, const tc::Params& p, const CUtensorMap& ma, c
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   cir_prof_gemm_begin(ctx, 2.0 * (double)p.M * (double)p.N * (double)p.K * (double)p.batch);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, tc::gemm_tcgen05_kernel<BN, PAIR, FILT>, ma, mw, mc, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, ma, mw, mc, p);
   cir_prof_gemm_end(ctx);
   if (e != cudaSuccess) { cir_set_error("tcgen05 GEMM launch failed: %s", cudaGetErrorString(e)); return CIR_ECUDA; }
   CIR_LAUNCH_CHECK(ctx);
@@ -664,14 +695,17 @@ int cir_gemm_tcgen05(cir_ctx* ctx, const cir_gemm_args* a) {
 
 // Similarity tiles with a threshold filter instead of an output matrix (stage-I top-K): S = A W^T is computed tile by tile on the
 // tensor cores (bf16 operands, fp32 accumulation) and never stored; see cir_gemm_filter in common.cuh.
-int cir_gemm_tcgen05_filter(cir_ctx* ctx, const void* A, const void* W, int64_t M, int64_t N, int64_t K, const cir_gemm_filter* f) {
+int cir_gemm_tcgen05_filter(cir_ctx* ctx, const void* A, const void* W, int64_t M, int64_t N, int64_t K, const cir_gemm_filter* f,
+                            const uint32_t* col_tags, const uint32_t* row_masks) {
   if (M == 0 || N == 0) return CIR_OK;
   CIR_CHECK_ARG(ctx->dtype == CIR_DTYPE_BF16 && K % 64 == 0 && ((uintptr_t)A & 15) == 0 && ((uintptr_t)W & 15) == 0, "gemm_filter: bf16 context, K % 64 == 0, aligned operands");
   CIR_CHECK_ARG(M < (1ll << 31) && N < (1ll << 31) && f && f->thr && f->count && f->cand && f->overflow && f->cap > 0, "gemm_filter: bad argument");
+  CIR_CHECK_ARG(!col_tags == !row_masks, "gemm_filter: column tags and row masks go together");
   tc::Params p{};
   p.M = M; p.N = N; p.K = K; p.batch = 1;
   p.flt = *f;
   p.n_major = 1;
+  p.flt_col_tags = col_tags; p.flt_row_masks = row_masks;
   const int64_t pair_tiles = ((M + 2 * tc::BM - 1) / (2 * tc::BM)) * ((N + 255) / 256);
   const bool use_pair = ctx->gemm_pair && pair_tiles >= ctx->num_sms / 2;
   const int tile_m = use_pair ? 2 * tc::BM : tc::BM;
@@ -684,5 +718,6 @@ int cir_gemm_tcgen05_filter(cir_ctx* ctx, const void* A, const void* W, int64_t 
   CUtensorMap ma, mw;
   CIR_TRY(cir_make_map_2d(ctx, &ma, A, M, K, K, tc::BM));
   CIR_TRY(cir_make_map_2d(ctx, &mw, W, N, K, K, use_pair ? 128 : 256));
+  if (col_tags) return use_pair ? launch_tc<256, true, true, true>(ctx, p, ma, mw, ma) : launch_tc<256, false, true, true>(ctx, p, ma, mw, ma);
   return use_pair ? launch_tc<256, true, true>(ctx, p, ma, mw, ma) : launch_tc<256, false, true>(ctx, p, ma, mw, ma);
 }

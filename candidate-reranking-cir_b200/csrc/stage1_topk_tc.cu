@@ -17,6 +17,9 @@
 //      the host, so a search can be captured in a CUDA graph.
 // The gallery side (bf16 copy + the maxima {max ||g||, max ||g - bf16(g)||}) is a "view": cir_stage1_index keeps one resident and
 // grows it row block by row block (the maxima only grow), cir_stage1_topk builds a transient one in its workspace per call.
+// Filtered search (row tags, per-query masks): the tagged FILT GEMM drops ineligible columns before a hit reserves a slot and the exact
+// scan skips them, so the lists, thresholds and counts of select_kernel / finalize_kernel only ever hold eligible rows (those two
+// kernels are shared unchanged).  gmax stays a valid bound: it covers a superset of the eligible rows.
 #include "common.cuh"
 
 namespace s1tc {
@@ -268,12 +271,14 @@ finalize_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__ coun
 // on exact_dist keys.  Fixed grid, independent of the data: blockIdx.x = one of `parts` gallery slices of `slice` rows, blockIdx.y
 // strides over the flagged queries; every CTA exits at once when nothing is flagged.  Slice p's Kp best keys go to the query's own
 // candidate row at [p * Kp, (p + 1) * Kp) (parts * Kp <= cap), which the filter no longer needs.
+// TAGS: rows with (row_tags[r] & query_masks[q]) == 0 are skipped next to the excluded one.
 constexpr int SCAN_CH = 2048;                  // gallery rows per compaction round
 constexpr int MAX_PARTS = 64;
-__global__ void __launch_bounds__(THREADS, 2)
-exact_scan_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__ flagged, const float* __restrict__ q_emb,
-                  const float* __restrict__ g_emb, int64_t G, int64_t slice, const int32_t* __restrict__ exclude, int64_t col_offset,
-                  int K, int Kp, uint2* __restrict__ cand, int64_t cap) {
+template <bool TAGS>
+__device__ __forceinline__ void exact_scan(const int32_t* __restrict__ flags, const int32_t* __restrict__ flagged, const float* __restrict__ q_emb,
+                                           const float* __restrict__ g_emb, int64_t G, int64_t slice, const int32_t* __restrict__ exclude,
+                                           int64_t col_offset, int K, int Kp, uint2* __restrict__ cand, int64_t cap,
+                                           const uint32_t* __restrict__ row_tags, const uint32_t* __restrict__ query_masks) {
   __shared__ __align__(16) float sq[E];
   __shared__ uint64_t sbest[1024];
   __shared__ uint64_t schunk[SCAN_CH];
@@ -287,6 +292,7 @@ exact_scan_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__
     for (int i = tid; i < E; i += THREADS) sq[i] = q_emb[q * E + i];
     for (int i = tid; i < Kp; i += THREADS) sbest[i] = KEY_MAX;
     const int64_t excl = exclude ? (int64_t)exclude[q] : -1;
+    const uint32_t qmask = TAGS ? query_masks[q] : 0u;
     __syncthreads();
     for (int64_t c0 = r0; c0 < r1; c0 += SCAN_CH) {
       if (tid == 0) s_n = 0;
@@ -294,7 +300,7 @@ exact_scan_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__
       const uint64_t thresh = sbest[K - 1];                  // current K-th best (KEY_MAX while not full)
       for (int i = tid; i < SCAN_CH; i += THREADS) {
         const int64_t r = c0 + i;
-        if (r < r1) {
+        if (r < r1 && (!TAGS || (row_tags[r] & qmask) != 0)) {
           const int64_t global = col_offset + r;
           const uint64_t key = ((uint64_t)ordered_bits(exact_dist(sq, g_emb + r * E)) << 32) | (uint32_t)global;
           if (global != excl && key < thresh) schunk[atomicAdd(&s_n, 1)] = key;
@@ -318,6 +324,19 @@ exact_scan_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__
     uint64_t* out = reinterpret_cast<uint64_t*>(cand + q * cap) + (int64_t)blockIdx.x * Kp;
     for (int i = tid; i < Kp; i += THREADS) out[i] = sbest[i];
   }
+}
+__global__ void __launch_bounds__(THREADS, 2)
+exact_scan_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__ flagged, const float* __restrict__ q_emb,
+                  const float* __restrict__ g_emb, int64_t G, int64_t slice, const int32_t* __restrict__ exclude, int64_t col_offset,
+                  int K, int Kp, uint2* __restrict__ cand, int64_t cap) {
+  exact_scan<false>(flags, flagged, q_emb, g_emb, G, slice, exclude, col_offset, K, Kp, cand, cap, nullptr, nullptr);
+}
+__global__ void __launch_bounds__(THREADS, 2)
+exact_scan_filtered_kernel(const int32_t* __restrict__ flags, const int32_t* __restrict__ flagged, const float* __restrict__ q_emb,
+                           const float* __restrict__ g_emb, int64_t G, int64_t slice, const int32_t* __restrict__ exclude, int64_t col_offset,
+                           int K, int Kp, uint2* __restrict__ cand, int64_t cap, const uint32_t* __restrict__ row_tags,
+                           const uint32_t* __restrict__ query_masks) {
+  exact_scan<true>(flags, flagged, q_emb, g_emb, G, slice, exclude, col_offset, K, Kp, cand, cap, row_tags, query_masks);
 }
 
 // The flagged queries' `n` = parts * Kp slice keys (a power of two) -> sorted, first K out.
@@ -381,8 +400,8 @@ int cir_stage1_tc_convert(cir_ctx* ctx, const float* g_emb, int64_t n, bf16* g_b
 }
 
 int cir_stage1_tc_search(cir_ctx* ctx, const float* q_emb, int64_t Q, const float* g_emb, const bf16* g_bf16, int64_t G, const uint32_t* gmax,
-                         const int32_t* exclude, int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
-                         void* workspace, size_t workspace_bytes) {
+                         const uint32_t* row_tags, const uint32_t* query_masks, const int32_t* exclude, int64_t col_offset, int64_t K,
+                         float* top_dist, int32_t* top_idx, int32_t* exact_rows, void* workspace, size_t workspace_bytes) {
   using namespace s1tc;
   const int64_t cap = capacity(K);
   Ws w = plan(workspace, Q, cap);
@@ -408,7 +427,7 @@ int cir_stage1_tc_search(cir_ctx* ctx, const float* q_emb, int64_t Q, const floa
     if (n > G - g0) n = G - g0;
     cir_gemm_filter f{};
     f.thr = w.thr; f.count = w.count; f.cand = w.cand; f.overflow = w.flags; f.cap = cap; f.col_base = g0;
-    CIR_TRY(cir_gemm_tcgen05_filter(ctx, w.qb, g_bf16 + g0 * E, Q, n, E, &f));
+    CIR_TRY(cir_gemm_tcgen05_filter(ctx, w.qb, g_bf16 + g0 * E, Q, n, E, &f, row_tags ? row_tags + g0 : nullptr, query_masks));
     g0 += n;
     if (g0 < G) {
       select_kernel<<<(unsigned)Q, THREADS, (size_t)cap * 8, st>>>(w.cand, w.count, w.thr, cap, (int)K, exclude, w.q_err, w.q_nrm, gmax);
@@ -424,8 +443,12 @@ int cir_stage1_tc_search(cir_ctx* ctx, const float* q_emb, int64_t Q, const floa
   const int64_t slice = (G + parts - 1) / parts;
   const int64_t ys = (2 * (int64_t)ctx->num_sms + parts - 1) / parts;
   const unsigned gy = (unsigned)(Q < ys ? Q : ys);
-  exact_scan_kernel<<<dim3((unsigned)parts, gy), THREADS, 0, st>>>(w.flags, w.flagged, q_emb, g_emb, G, slice, exclude, col_offset, (int)K, Kp,
-                                                                    w.cand, cap);
+  if (row_tags)
+    exact_scan_filtered_kernel<<<dim3((unsigned)parts, gy), THREADS, 0, st>>>(w.flags, w.flagged, q_emb, g_emb, G, slice, exclude, col_offset,
+                                                                               (int)K, Kp, w.cand, cap, row_tags, query_masks);
+  else
+    exact_scan_kernel<<<dim3((unsigned)parts, gy), THREADS, 0, st>>>(w.flags, w.flagged, q_emb, g_emb, G, slice, exclude, col_offset, (int)K, Kp,
+                                                                      w.cand, cap);
   CIR_LAUNCH_CHECK(ctx);
   const unsigned gm = (unsigned)(Q < 2 * ctx->num_sms ? Q : 2 * ctx->num_sms);
   exact_merge_kernel<<<gm, THREADS, (size_t)parts * Kp * 8, st>>>(w.flags, w.flagged, w.cand, cap, parts * Kp, (int)K, top_dist, top_idx);
@@ -442,6 +465,6 @@ int cir_stage1_topk_tc(cir_ctx* ctx, const float* q_emb, const float* g_emb, int
   uint32_t* gmax = (uint32_t*)((char*)workspace + vb - 256);
   CIR_CUDA(cudaMemsetAsync(gmax, 0, 2 * sizeof(uint32_t), ctx->stream));
   CIR_TRY(cir_stage1_tc_convert(ctx, g_emb, G, gb, gmax));
-  return cir_stage1_tc_search(ctx, q_emb, Q, g_emb, gb, G, gmax, exclude, col_offset, K, top_dist, top_idx, nullptr, (char*)workspace + vb,
-                              workspace_bytes - vb);
+  return cir_stage1_tc_search(ctx, q_emb, Q, g_emb, gb, G, gmax, nullptr, nullptr, exclude, col_offset, K, top_dist, top_idx, nullptr,
+                              (char*)workspace + vb, workspace_bytes - vb);
 }

@@ -4,7 +4,8 @@
 //   cir_rerank_sort      argsort(scores, descending)                 src/validate_stage2.py:53,174,190
 //   cir_topk_from_dist   K smallest of a distance row, minus `exclude` src/validate.py:58,203-210,257
 //   cir_stage1_topk      fused 1 - q @ G^T tiles + running top-K       src/validate.py:57-58,202-203
-//   cir_stage1_index_*   the same search over a resident gallery index (built once, grown by appends)
+//   cir_stage1_index_*   the same search over a resident gallery index (built once, grown by appends); _filtered restricts each
+//                        query to the rows whose tag shares a bit with its mask
 //   cir_topk_merge       merge of per-shard (dist, idx) lists after the NCCL all-gather
 //   cir_recall_counts    sum(labels[:, :k]) over sorted labels         src/validate_stage2.py:56-62,178-203
 #include <algorithm>
@@ -81,10 +82,13 @@ struct TopkParams {
   uint64_t* best;                                    // [Q][Kp] running sorted lists
   int init;                                          // 1: start from empty lists
   float* out_dist; int32_t* out_idx;                 // optional final outputs [Q][K]
+  // topk_rows_filtered_kernel only: column c of row q is a candidate iff (row_tags[c] & query_masks[q]) != 0 (row_tags starts at
+  // this slab's column 0).  Last in the struct, so the other fields keep their offsets in topk_rows_kernel.
+  const uint32_t* row_tags; const uint32_t* query_masks;
 };
 
-__global__ void __launch_bounds__(THREADS)
-topk_rows_kernel(TopkParams p) {
+template <bool TAGS>
+__device__ __forceinline__ void topk_rows(const TopkParams& p) {
   __shared__ uint64_t sbest[MAXK];
   __shared__ uint64_t schunk[CH];
   __shared__ int s_any;
@@ -94,6 +98,7 @@ topk_rows_kernel(TopkParams p) {
   const int64_t excl = p.exclude ? (int64_t)p.exclude[q] : -1;
   const float* row = p.vals + q * p.ld;
   const int32_t* irow = p.col_idx ? p.col_idx + q * p.ld : nullptr;
+  const uint32_t qmask = TAGS ? p.query_masks[q] : 0u;
   __syncthreads();
   for (int64_t c0 = 0; c0 < p.ncols; c0 += CH) {
     if (tid == 0) s_any = 0;
@@ -102,7 +107,7 @@ topk_rows_kernel(TopkParams p) {
     // compact the keys that can still enter the top-K (usually a handful once the lists have warmed up)
     for (int i = tid; i < CH; i += THREADS) {
       const int64_t c = c0 + i;
-      if (c < p.ncols) {
+      if (c < p.ncols && (!TAGS || (p.row_tags[c] & qmask) != 0)) {
         float v = row[c];
         if (p.one_minus) v = 1.0f - v;
         const int64_t gi = irow ? (int64_t)irow[c] : p.col_base + c;
@@ -135,6 +140,8 @@ topk_rows_kernel(TopkParams p) {
     }
   }
 }
+__global__ void __launch_bounds__(THREADS) topk_rows_kernel(TopkParams p) { topk_rows<false>(p); }
+__global__ void __launch_bounds__(THREADS) topk_rows_filtered_kernel(TopkParams p) { topk_rows<true>(p); }
 
 // Merge of P per-shard lists in ONE pass: the P*K composite keys of a query (<= 8192) are sorted once in shared memory and the first K
 // leave.  Keys are unique across shards (disjoint global indices), so the result equals the sequential merge bit for bit.
@@ -249,9 +256,11 @@ extern "C" size_t cir_stage1_topk_workspace_bytes(int64_t Q, int64_t G, int64_t 
   return a > b ? a : b;
 }
 
-// fp32 CUDA-core path: similarity tiles of kSimChunk columns + running top-K (workspace: stage1_fp32_workspace_bytes)
+// fp32 CUDA-core path: similarity tiles of kSimChunk columns + running top-K (workspace: stage1_fp32_workspace_bytes).
+// row_tags [G] / query_masks [Q] (both or neither): query q ranks only the rows with (row_tags[r] & query_masks[q]) != 0.
 static int stage1_fp32(cir_ctx* ctx, const float* q_emb, const float* g_emb, int64_t Q, int64_t G, const int32_t* exclude, int64_t col_offset,
-                       int64_t K, float* top_dist, int32_t* top_idx, void* workspace) {
+                       int64_t K, float* top_dist, int32_t* top_idx, void* workspace, const uint32_t* row_tags = nullptr,
+                       const uint32_t* query_masks = nullptr) {
   uint64_t* best = (uint64_t*)workspace;
   float* sim = (float*)((char*)workspace + cir_topk_workspace_bytes(Q, G, K));
   const int64_t gc = G < kSimChunk ? G : kSimChunk;
@@ -275,7 +284,12 @@ static int stage1_fp32(cir_ctx* ctx, const float* q_emb, const float* g_emb, int
     p.one_minus = 1; p.K = (int)K; p.Kp = pow2_at_least(K); p.best = best; p.init = (g0 == 0);
     const bool last = g0 + gc >= G;
     p.out_dist = last ? top_dist : nullptr; p.out_idx = last ? top_idx : nullptr;
-    topk_rows_kernel<<<(unsigned)Q, THREADS, 0, ctx->stream>>>(p);
+    if (row_tags) {
+      p.row_tags = row_tags + g0; p.query_masks = query_masks;
+      topk_rows_filtered_kernel<<<(unsigned)Q, THREADS, 0, ctx->stream>>>(p);
+    } else {
+      topk_rows_kernel<<<(unsigned)Q, THREADS, 0, ctx->stream>>>(p);
+    }
     CIR_LAUNCH_CHECK(ctx);
   }
   return CIR_OK;
@@ -344,21 +358,39 @@ extern "C" size_t cir_stage1_index_topk_workspace_bytes(const cir_ctx* ctx, cons
   return a > b ? a : b;
 }
 
+// cir_stage1_index_topk (row_tags == query_masks == NULL) and cir_stage1_index_topk_filtered; `fn` names the entry point in errors
+static int index_topk(const char* fn, cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const uint32_t* row_tags,
+                      const uint32_t* query_masks, const int32_t* exclude, int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx,
+                      int32_t* exact_rows, void* workspace, size_t workspace_bytes) {
+  CIR_ENTER(ctx);
+  if (Q == 0) return CIR_OK;
+  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "%s: K=%lld out of range [1,%d]", fn, (long long)K, MAXK);
+  const size_t need = cir_stage1_index_topk_workspace_bytes(ctx, index, Q, K);
+  if (workspace_bytes < need) { cir_set_error("%s: workspace %zu < %zu bytes", fn, workspace_bytes, need); return CIR_EWORKSPACE; }
+  const int64_t G = index->rows;
+  if (index->g_bf16 && cir_stage1_topk_tc_supported(ctx, Q, G, K))
+    return cir_stage1_tc_search(ctx, q_emb, Q, index->g_f32, (const bf16*)index->g_bf16, G, index->gmax, row_tags, query_masks, exclude,
+                                col_offset, K, top_dist, top_idx, exact_rows, workspace, workspace_bytes);
+  if (exact_rows) CIR_CUDA(cudaMemsetAsync(exact_rows, 0, (size_t)Q * sizeof(int32_t), ctx->stream));
+  return stage1_fp32(ctx, q_emb, index->g_f32, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace, row_tags, query_masks);
+}
+
 extern "C" int cir_stage1_index_topk(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const int32_t* exclude,
                                      int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
                                      void* workspace, size_t workspace_bytes) {
   CIR_CHECK_ARG(ctx && index, "stage1_index_topk: null argument");
-  CIR_ENTER(ctx);
-  if (Q == 0) return CIR_OK;
-  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "stage1_index_topk: K=%lld out of range [1,%d]", (long long)K, MAXK);
-  const size_t need = cir_stage1_index_topk_workspace_bytes(ctx, index, Q, K);
-  if (workspace_bytes < need) { cir_set_error("stage1_index_topk: workspace %zu < %zu bytes", workspace_bytes, need); return CIR_EWORKSPACE; }
-  const int64_t G = index->rows;
-  if (index->g_bf16 && cir_stage1_topk_tc_supported(ctx, Q, G, K))
-    return cir_stage1_tc_search(ctx, q_emb, Q, index->g_f32, (const bf16*)index->g_bf16, G, index->gmax, exclude, col_offset, K, top_dist,
-                                top_idx, exact_rows, workspace, workspace_bytes);
-  if (exact_rows) CIR_CUDA(cudaMemsetAsync(exact_rows, 0, (size_t)Q * sizeof(int32_t), ctx->stream));
-  return stage1_fp32(ctx, q_emb, index->g_f32, Q, G, exclude, col_offset, K, top_dist, top_idx, workspace);
+  return index_topk("stage1_index_topk", ctx, index, q_emb, Q, nullptr, nullptr, exclude, col_offset, K, top_dist, top_idx, exact_rows,
+                    workspace, workspace_bytes);
+}
+
+extern "C" int cir_stage1_index_topk_filtered(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q,
+                                              const uint32_t* row_tags, const uint32_t* query_masks, const int32_t* exclude,
+                                              int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                                              void* workspace, size_t workspace_bytes) {
+  CIR_CHECK_ARG(ctx && index, "stage1_index_topk_filtered: null argument");
+  CIR_CHECK_ARG(row_tags && query_masks, "stage1_index_topk_filtered: row_tags and query_masks are required (all bits set = no filter)");
+  return index_topk("stage1_index_topk_filtered", ctx, index, q_emb, Q, row_tags, query_masks, exclude, col_offset, K, top_dist, top_idx,
+                    exact_rows, workspace, workspace_bytes);
 }
 
 __global__ void divide_rows_kernel(float* __restrict__ x, int64_t n, float d) {

@@ -20,6 +20,7 @@ from __future__ import annotations
 
 from typing import Callable, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -152,18 +153,30 @@ class ShardedStage1Index:
     """Resident stage-I index over the ranks of the default process group: each rank indexes only its ``shard_rows`` block of
     the gallery, searches it with ``col_offset = block.start`` (global row ids), and the lists meet in ``sharded_stage1_topk``
     + ``topk_merge``.  No rank holds the full gallery.  ``rows_of(block)`` -> fp32 [len(block), 256] gallery rows of that block
-    (e.g. a slice of ``extract_index_features`` output, or rows read from storage)."""
+    (e.g. a slice of ``extract_index_features`` output, or rows read from storage); ``tags_of(block)`` (optional) -> their row
+    tags (see ``Stage1Index.add``)."""
 
-    def __init__(self, engine, gallery_rows: int, rows_of: Callable[[slice], torch.Tensor]):
+    def __init__(self, engine, gallery_rows: int, rows_of: Callable[[slice], torch.Tensor],
+                 tags_of: Optional[Callable[[slice], object]] = None):
         rank, ws = world()
         self.engine, self.gallery_rows = engine, gallery_rows
         self.block = shard_rows(gallery_rows, rank, ws)
         self.index = engine.stage1_index(self.block.stop - self.block.start)
-        self.index.add(rows_of(self.block))
+        self.index.add(rows_of(self.block), tags=None if tags_of is None else tags_of(self.block))
 
-    def topk(self, q_emb, k: int, exclude=None) -> Tuple[torch.Tensor, torch.Tensor]:
-        """-> merged (dist [Q,k], idx [Q,k]) on every rank; ``q_emb`` and ``exclude`` cover all Q queries (global row ids)."""
+    def topk(self, q_emb, k: int, exclude=None, tags=None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """-> merged (dist [Q,k], idx [Q,k]) on every rank; ``q_emb``, ``exclude`` (global row ids) and the query masks ``tags``
+        (optional, see ``Stage1Index.topk``) cover all Q queries."""
         def local(rows: slice):
             assert rows == self.block
-            return self.index.topk(q_emb, k, exclude=exclude, col_offset=rows.start)
+            return self.index.topk(q_emb, k, exclude=exclude, col_offset=rows.start, tags=tags)
         return sharded_stage1_topk(local, self.engine.topk_merge, self.gallery_rows)
+
+    def remove(self, global_rows) -> None:
+        """Remove gallery rows (global row ids, the same list on every rank): each rank removes those in its block."""
+        g = global_rows.cpu() if isinstance(global_rows, torch.Tensor) else global_rows
+        g = np.asarray(g, dtype=np.int64).reshape(-1)
+        if g.size and (g.min() < 0 or g.max() >= self.gallery_rows):
+            raise ValueError(f"remove: rows outside [0, {self.gallery_rows})")
+        mine = g[(g >= self.block.start) & (g < self.block.stop)]
+        self.index.remove(mine - self.block.start)

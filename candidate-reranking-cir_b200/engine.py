@@ -614,14 +614,34 @@ class Engine:
         return y
 
 
+ALL_TAGS = 0xFFFFFFFF
+
+
+def tag_bits(tags) -> np.ndarray:
+    """Row tags / query masks (a Python int, a sequence of ints or a numpy integer array, e.g. uint32) -> int32 bit patterns
+    (0xFFFFFFFF -> -1), the form the device tensors keep.  Values outside [0, 2^32) raise ValueError."""
+    a = np.asarray(tags)
+    if a.dtype == object:            # ints beyond 64 bits
+        raise ValueError("tags must lie in [0, 2^32)")
+    if a.dtype == bool or not np.issubdtype(a.dtype, np.integer):
+        raise TypeError(f"tags must be integers, got {a.dtype}")
+    if a.size and (a.min() < 0 or a.max() > ALL_TAGS):
+        raise ValueError(f"tags must lie in [0, 2^32), got [{a.min()}, {a.max()}]")
+    return a.astype(np.uint32).view(np.int32)
+
+
 class Stage1Index:
     """Resident stage-I gallery index (``cir_stage1_index`` in include/cir_b200.h): gallery embeddings fp32 [n,256] are copied
     and, in bf16 engines, converted to bf16 once, when they are added; every search reuses them.  ``topk`` returns exactly what
     :meth:`Engine.stage1_topk` returns over the same rows, bit for bit.
 
-    ``topk`` never synchronises.  Given device tensors (q_emb fp32 contiguous, exclude int32) and ``out=``, it allocates and
-    uploads nothing once its workspace exists for that (Q, k) -- run it once before ``torch.cuda.graph`` capture.  A captured
-    graph searches the rows the index had at capture time."""
+    Every row carries a 32-bit tag (all bits set unless given).  ``topk(..., tags=masks)`` searches, for query q, only the rows
+    whose tag shares a bit with masks[q] (cir_stage1_index_topk_filtered); :meth:`remove` sets tags to 0, so removed rows are
+    never returned.  Tags are kept as a device int32 tensor of uint32 bit patterns.
+
+    ``topk`` never synchronises.  Given device tensors (q_emb fp32 contiguous, exclude and masks int32) and ``out=``, it allocates
+    and uploads nothing once its workspace exists for that (Q, k) -- run it once before ``torch.cuda.graph`` capture.  A captured
+    graph searches the rows the index had at capture time, with the tags and masks those tensors hold at replay."""
 
     def __init__(self, eng: Engine, capacity: int):
         self.eng = eng
@@ -629,6 +649,7 @@ class Stage1Index:
         self._s = N.Stage1Index()
         self._ws: Optional[torch.Tensor] = None
         self._retired: List[torch.Tensor] = []    # outgrown workspaces stay alive: a captured graph may still point at one
+        self._tags = torch.full((max(1, capacity),), -1, dtype=torch.int32, device=eng.device)
         eng._sync_stream()
         N.check(eng._lib.cir_stage1_index_init(eng.ctx, N.ptr(self._blob), self._blob.numel(), capacity, C.byref(self._s)),
                 "cir_stage1_index_init")
@@ -647,18 +668,65 @@ class Stage1Index:
         n = self.rows
         return self._blob[: n * EMBED * 4].view(torch.float32).view(n, EMBED)
 
-    def add(self, g_emb: torch.Tensor) -> "Stage1Index":
-        """Append gallery rows fp32 [n,256] (host or device); only the new rows are converted."""
+    @property
+    def row_tags(self) -> torch.Tensor:
+        """int32 [rows] tag bit patterns of the indexed rows (a view: change tags through :meth:`set_tags` / :meth:`remove`)."""
+        return self._tags[: self.rows]
+
+    def _tag_tensor(self, tags, n: int, what: str) -> torch.Tensor:
+        """One int (broadcast), n values (see tag_bits) or an int32 tensor of n bit patterns -> contiguous device int32 [n]."""
+        if isinstance(tags, torch.Tensor):
+            if tags.dtype != torch.int32:
+                raise TypeError(f"{what}: a tag tensor holds int32 bit patterns, got {tags.dtype}")
+            if tags.dim() != 1 or tags.numel() != n:
+                raise ValueError(f"{what}: expected {n} tags, got shape {tuple(tags.shape)}")
+            return tags.to(self.eng.device).contiguous()
+        bits = tag_bits(tags)
+        if bits.ndim == 0:
+            return torch.full((n,), int(bits), dtype=torch.int32, device=self.eng.device)
+        if bits.shape != (n,):
+            raise ValueError(f"{what}: expected {n} tags, got shape {bits.shape}")
+        return torch.from_numpy(np.ascontiguousarray(bits)).to(self.eng.device)
+
+    def add(self, g_emb: torch.Tensor, tags=None) -> "Stage1Index":
+        """Append gallery rows fp32 [n,256] (host or device); only the new rows are converted.  ``tags``: the new rows' tags
+        (one int or n values; default all bits set, so every non-zero mask sees them)."""
         g = g_emb.to(self.eng.device, torch.float32).contiguous()
         assert g.dim() == 2 and g.shape[1] == EMBED, g.shape
+        n, r0 = g.shape[0], self.rows
+        t = None if tags is None else self._tag_tensor(tags, n, "Stage1Index.add")
         self.eng._sync_stream()
-        N.check(self.eng._lib.cir_stage1_index_add(self.eng.ctx, C.byref(self._s), N.ptr(g), g.shape[0]), "cir_stage1_index_add")
+        N.check(self.eng._lib.cir_stage1_index_add(self.eng.ctx, C.byref(self._s), N.ptr(g), n), "cir_stage1_index_add")
+        if t is None:
+            self._tags[r0:r0 + n].fill_(-1)
+        else:
+            self._tags[r0:r0 + n].copy_(t)
         return self
 
-    def topk(self, q_emb: torch.Tensor, k: int, exclude=None, col_offset: int = 0, out=None, exact_rows: Optional[torch.Tensor] = None):
+    def set_tags(self, rows, tags) -> "Stage1Index":
+        """Set the tags of indexed rows (local row numbers: a device int tensor, or host ints range-checked here) to one int or
+        one value per row.  An on-stream tensor write: with device tensors it can be captured in a CUDA graph."""
+        if isinstance(rows, torch.Tensor) and rows.is_cuda:
+            r = rows.reshape(-1).long()
+        else:
+            r_np = np.asarray(rows, dtype=np.int64).reshape(-1)
+            self.eng._check_range(r_np, self.rows, "Stage1Index.set_tags rows")
+            r = torch.from_numpy(r_np).to(self.eng.device)
+        t = self._tag_tensor(tags, r.numel(), "Stage1Index.set_tags")
+        self._tags.index_copy_(0, r, t)
+        return self
+
+    def remove(self, rows) -> "Stage1Index":
+        """Remove indexed rows: their tags become 0, so no filtered search returns them (search with ``tags=ALL_TAGS`` for
+        everything not removed; ``tags=None`` ignores tags).  Row numbers stay; ``set_tags`` restores a row."""
+        return self.set_tags(rows, 0)
+
+    def topk(self, q_emb: torch.Tensor, k: int, exclude=None, col_offset: int = 0, out=None, exact_rows: Optional[torch.Tensor] = None,
+             tags=None):
         """-> (dist fp32 [Q,k], idx int32 [Q,k]) of the k nearest indexed rows (global index = col_offset + row), skipping
         exclude[q] (-1 = none).  ``out``: optional (dist, idx) to fill.  ``exact_rows``: optional int32 [Q] device tensor, set to 1
-        for the queries whose list came from the exact fallback scan."""
+        for the queries whose list came from the exact fallback scan.  ``tags``: per-query masks [Q] (or one int for all queries):
+        query q then ranks only the rows with (row tag & tags[q]) != 0 and pads a short list with (+inf, -1)."""
         eng = self.eng
         q = q_emb.to(eng.device, torch.float32).contiguous()
         Q = q.shape[0]
@@ -669,14 +737,20 @@ class Stage1Index:
         assert td.is_contiguous() and ti.is_contiguous()
         assert exact_rows is None or (exact_rows.dtype == torch.int32 and exact_rows.numel() == Q and exact_rows.is_contiguous())
         ex = None if exclude is None else eng._i32(exclude)
+        masks = None if tags is None else self._tag_tensor(tags, Q, "Stage1Index.topk")
         need = eng._lib.cir_stage1_index_topk_workspace_bytes(eng.ctx, C.byref(self._s), Q, k)
         if self._ws is None or self._ws.numel() < need:
             if self._ws is not None:
                 self._retired.append(self._ws)
             self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=eng.device)
         eng._sync_stream()
-        N.check(eng._lib.cir_stage1_index_topk(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(ex), col_offset, k, N.ptr(td), N.ptr(ti),
-                                               N.ptr(exact_rows), N.ptr(self._ws), self._ws.numel()), "cir_stage1_index_topk")
+        if masks is None:
+            N.check(eng._lib.cir_stage1_index_topk(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(ex), col_offset, k, N.ptr(td), N.ptr(ti),
+                                                   N.ptr(exact_rows), N.ptr(self._ws), self._ws.numel()), "cir_stage1_index_topk")
+        else:
+            N.check(eng._lib.cir_stage1_index_topk_filtered(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(self._tags), N.ptr(masks),
+                                                            N.ptr(ex), col_offset, k, N.ptr(td), N.ptr(ti), N.ptr(exact_rows),
+                                                            N.ptr(self._ws), self._ws.numel()), "cir_stage1_index_topk_filtered")
         return td, ti
 
 

@@ -234,6 +234,21 @@ size_t cir_stage1_index_topk_workspace_bytes(const cir_ctx* ctx, const cir_stage
 int    cir_stage1_index_topk(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const int32_t* exclude,
                              int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
                              void* workspace, size_t workspace_bytes);
+/* Filtered search: row r of the index is eligible for query q iff (row_tags[r] & query_masks[q]) != 0; otherwise as
+ * cir_stage1_index_topk.  The result is exactly what cir_stage1_topk returns over the eligible rows compacted in their original
+ * order, with indices mapped back (col_offset + local row), ties to the lowest eligible row; a query with fewer than K eligible
+ * rows gets (+inf, -1) in the remaining slots (a mask of 0: all of them).  `exclude` applies on top of eligibility; exact_rows
+ * flags queries whose eligible-row candidate list overflowed.  Eligibility is applied before a row enters a query's candidate
+ * list (tensor-core filter, exact scan and fp32 path alike).  The workspace is cir_stage1_index_topk_workspace_bytes, so one
+ * workspace (and one captured graph) serves both calls.  Tags and masks belong to the caller and are read when the search runs:
+ * a captured graph follows in-place edits of both, which is how rows are removed (tag 0) or re-categorised.  Never synchronises.
+ * NULL row_tags or query_masks: CIR_EINVAL. */
+int    cir_stage1_index_topk_filtered(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q,
+                                      const uint32_t* row_tags,     /* device [index->rows], local row order */
+                                      const uint32_t* query_masks,  /* device [Q] */
+                                      const int32_t* exclude, int64_t col_offset, int64_t K,
+                                      float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                                      void* workspace, size_t workspace_bytes);
 
 /* In-batch contrastive logits of the stage-I forward: logits[Q, G] = q_emb[Q,256] @ t_emb[G,256]^T / temp, all fp32.
  * Replaces `predicted_features @ target_features.T / self.temp` (src/blip_stage1.py:90-91), forward only. */
