@@ -393,6 +393,217 @@ extern "C" int cir_stage1_index_topk_filtered(cir_ctx* ctx, const cir_stage1_ind
                     exact_rows, workspace, workspace_bytes);
 }
 
+// ---- compaction and permanent row ids.  Compaction is stable (kept rows keep their order), so the ids stay strictly increasing along
+// the physical rows and a search over physical rows ranks ties exactly as a search over ids would.
+namespace {
+
+constexpr int CPT_ROWS = 1024;            // rows per block of the count / gather kernels (4 consecutive rows per thread)
+
+__device__ __forceinline__ int kept_row(const uint32_t* __restrict__ tags, int64_t r, int64_t n, uint32_t mask) {
+  return r < n && (tags[r] & mask) != 0;
+}
+
+// block b: how many rows of [b * CPT_ROWS, (b + 1) * CPT_ROWS) are kept
+__global__ void __launch_bounds__(THREADS)
+compact_count_kernel(const uint32_t* __restrict__ tags, int64_t n, uint32_t mask, int32_t* __restrict__ block_count) {
+  __shared__ int s_count;
+  if (threadIdx.x == 0) s_count = 0;
+  __syncthreads();
+  const int64_t r0 = (int64_t)blockIdx.x * CPT_ROWS;
+  int c = 0;
+  for (int i = threadIdx.x; i < CPT_ROWS; i += THREADS) c += kept_row(tags, r0 + i, n, mask);
+  c = __reduce_add_sync(0xffffffffu, c);
+  if ((threadIdx.x & 31) == 0) atomicAdd(&s_count, c);
+  __syncthreads();
+  if (threadIdx.x == 0) block_count[blockIdx.x] = s_count;
+}
+
+// one block: block_off[b] = sum of block_count[0..b), block_off[nb] = the kept total
+__global__ void __launch_bounds__(1024)
+compact_scan_kernel(const int32_t* __restrict__ block_count, int64_t nb, int32_t* __restrict__ block_off) {
+  __shared__ int s_warp[32];
+  __shared__ int s_carry;
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  if (tid == 0) s_carry = 0;
+  for (int64_t b0 = 0; b0 < nb; b0 += 1024) {
+    const int64_t b = b0 + tid;
+    const int v = b < nb ? block_count[b] : 0;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
+    if (lane == 31) s_warp[w] = incl;
+    __syncthreads();
+    if (w == 0) {
+      const int t = s_warp[lane];
+      int x = t;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += u; }
+      s_warp[lane] = x - t;                                  // warps before this one
+    }
+    __syncthreads();
+    const int excl = s_carry + s_warp[w] + incl - v;
+    if (b < nb) block_off[b] = excl;
+    __syncthreads();                                         // everyone has read s_carry / s_warp
+    if (tid == 1023) s_carry = excl + v;
+    __syncthreads();
+  }
+  if (tid == 0) block_off[nb] = s_carry;
+}
+
+// Kept row r (in order) -> dst row block_off[b] + (kept rows before it in its block): the 1 KB fp32 row, its tag and its id
+// (src_ids[r], or r when src_ids is NULL).  One warp copies a row with two 16-byte loads per lane.
+__global__ void __launch_bounds__(THREADS)
+compact_gather_kernel(const float* __restrict__ src, const uint32_t* __restrict__ src_tags, const int32_t* __restrict__ src_ids, int64_t n,
+                      uint32_t mask, const int32_t* __restrict__ block_off, float* __restrict__ dst, uint32_t* __restrict__ dst_tags,
+                      int32_t* __restrict__ dst_ids) {
+  __shared__ int s_dst[CPT_ROWS];
+  __shared__ int s_warp[THREADS / 32];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const int64_t b0 = (int64_t)blockIdx.x * CPT_ROWS;
+  int k[4], c = 0;
+#pragma unroll
+  for (int j = 0; j < 4; j++) { k[j] = kept_row(src_tags, b0 + 4 * tid + j, n, mask); c += k[j]; }
+  int incl = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
+  if (lane == 31) s_warp[w] = incl;
+  __syncthreads();
+  int d = block_off[blockIdx.x] + incl - c;
+  for (int i = 0; i < w; i++) d += s_warp[i];
+#pragma unroll
+  for (int j = 0; j < 4; j++) s_dst[4 * tid + j] = k[j] ? d++ : -1;
+  __syncthreads();
+  for (int i = w; i < CPT_ROWS; i += THREADS / 32) {
+    const int to = s_dst[i];
+    if (to < 0) continue;
+    const int64_t r = b0 + i;
+    const float4* s4 = reinterpret_cast<const float4*>(src + r * CIR_EMBED);
+    float4* d4 = reinterpret_cast<float4*>(dst + (int64_t)to * CIR_EMBED);
+    const float4 a = __ldg(s4 + lane), b = __ldg(s4 + lane + 32);
+    d4[lane] = a;
+    d4[lane + 32] = b;
+    if (lane == 0) { dst_tags[to] = src_tags[r]; dst_ids[to] = src_ids ? src_ids[r] : (int32_t)r; }
+  }
+}
+
+// exclude[q] (col_offset + id, -1 = none) -> the physical row holding that id (binary search of the strictly increasing row_ids), -1 when
+// no row holds it
+__global__ void map_exclude_kernel(const int32_t* __restrict__ exclude, int64_t Q, const int32_t* __restrict__ row_ids, int64_t rows,
+                                   int64_t col_offset, int32_t* __restrict__ out) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= Q) return;
+  const int64_t id = exclude[q] < 0 ? -1 : (int64_t)exclude[q] - col_offset;
+  int32_t p = -1;
+  if (id >= 0) {
+    int64_t lo = 0, hi = rows;
+    while (lo < hi) {
+      const int64_t mid = (lo + hi) >> 1;
+      if ((int64_t)row_ids[mid] < id) lo = mid + 1; else hi = mid;
+    }
+    if (lo < rows && (int64_t)row_ids[lo] == id) p = (int32_t)lo;
+  }
+  out[q] = p;
+}
+
+// physical rows of a finished search -> col_offset + id; -1 (empty slot) passes through
+__global__ void map_ids_kernel(int32_t* __restrict__ idx, int64_t n, const int32_t* __restrict__ row_ids, int64_t col_offset) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t v = idx[i];
+    if (v >= 0) idx[i] = (int32_t)(col_offset + row_ids[v]);
+  }
+}
+
+}  // namespace
+
+extern "C" size_t cir_stage1_index_compact_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* src) {
+  (void)ctx;
+  if (!src) return 0;
+  const int64_t nb = (src->rows + CPT_ROWS - 1) / CPT_ROWS;
+  return align_up((size_t)nb * 4, 256) + align_up((size_t)(nb + 1) * 4, 256);
+}
+
+extern "C" int cir_stage1_index_compact(cir_ctx* ctx, const cir_stage1_index* src, const uint32_t* src_tags, const int32_t* src_ids,
+                                        uint32_t keep_mask, cir_stage1_index* dst, uint32_t* dst_tags, int32_t* dst_ids, void* workspace,
+                                        size_t workspace_bytes) {
+  CIR_CHECK_ARG(ctx && src && dst && dst_tags && dst_ids, "stage1_index_compact: null argument");
+  CIR_CHECK_ARG(src_tags || src->rows == 0, "stage1_index_compact: src_tags is required");
+  CIR_CHECK_ARG(dst->rows == 0, "stage1_index_compact: dst holds %lld rows; it must be an empty index", (long long)dst->rows);
+  const bool bf = ctx->dtype == CIR_DTYPE_BF16;
+  CIR_CHECK_ARG((src->g_bf16 != nullptr) == bf && (dst->g_bf16 != nullptr) == bf,
+                "stage1_index_compact: src and dst must both be indexes of the context's dtype (%s)", bf ? "bf16" : "fp32");
+  // a blob spans [g_f32, gmax + 256): a parallel stable compaction in place would read rows other blocks already overwrote
+  const char *s_lo = (const char*)src->g_f32, *s_hi = (const char*)src->gmax + 256;
+  const char *d_lo = (const char*)dst->g_f32, *d_hi = (const char*)dst->gmax + 256;
+  CIR_CHECK_ARG(s_hi <= d_lo || d_hi <= s_lo, "stage1_index_compact: src and dst blobs overlap; compact into a different blob");
+  const size_t need = cir_stage1_index_compact_workspace_bytes(ctx, src);
+  if (workspace_bytes < need) { cir_set_error("stage1_index_compact: workspace %zu < %zu bytes", workspace_bytes, need); return CIR_EWORKSPACE; }
+  CIR_ENTER(ctx);
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  CIR_CUDA(cudaStreamIsCapturing(ctx->stream, &cs));
+  CIR_CHECK_ARG(cs == cudaStreamCaptureStatusNone, "stage1_index_compact: synchronises the stream and cannot be captured in a CUDA graph");
+  const int64_t n = src->rows, nb = (n + CPT_ROWS - 1) / CPT_ROWS;
+  int32_t* count = (int32_t*)workspace;
+  int32_t* off = (int32_t*)((char*)workspace + align_up((size_t)nb * 4, 256));
+  int32_t kept = 0;
+  if (n > 0) {
+    compact_count_kernel<<<(unsigned)nb, THREADS, 0, ctx->stream>>>(src_tags, n, keep_mask, count);
+    CIR_LAUNCH_CHECK(ctx);
+    compact_scan_kernel<<<1, 1024, 0, ctx->stream>>>(count, nb, off);
+    CIR_LAUNCH_CHECK(ctx);
+    CIR_CUDA(cudaMemcpyAsync(&kept, off + nb, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CIR_CUDA(cudaStreamSynchronize(ctx->stream));             // the one synchronisation: dst->rows is a host-side count
+  }
+  CIR_CHECK_ARG(kept <= dst->capacity, "stage1_index_compact: %lld kept rows exceed the capacity %lld of dst (nothing written)",
+                (long long)kept, (long long)dst->capacity);
+  CIR_CUDA(cudaMemsetAsync(dst->gmax, 0, 2 * sizeof(uint32_t), ctx->stream));
+  if (kept > 0) {
+    compact_gather_kernel<<<(unsigned)nb, THREADS, 0, ctx->stream>>>(src->g_f32, src_tags, src_ids, n, keep_mask, off, dst->g_f32, dst_tags,
+                                                                      dst_ids);
+    CIR_LAUNCH_CHECK(ctx);
+    // the bf16 copy and the maxima of the kept rows only, as cir_stage1_index_add of those rows builds them
+    if (dst->g_bf16) CIR_TRY(cir_stage1_tc_convert(ctx, dst->g_f32, kept, (bf16*)dst->g_bf16, dst->gmax));
+  }
+  dst->rows = kept;
+  return CIR_OK;
+}
+
+extern "C" size_t cir_stage1_index_topk_ids_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* index, int64_t Q, int64_t K) {
+  const size_t s = cir_stage1_index_topk_workspace_bytes(ctx, index, Q, K);
+  return s ? align_up(s, 256) + align_up((size_t)Q * sizeof(int32_t), 256) : 0;
+}
+
+extern "C" int cir_stage1_index_topk_ids(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q, const int32_t* row_ids,
+                                         int64_t id_end, const uint32_t* row_tags, const uint32_t* query_masks, const int32_t* exclude,
+                                         int64_t col_offset, int64_t K, float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                                         void* workspace, size_t workspace_bytes) {
+  CIR_CHECK_ARG(ctx && index, "stage1_index_topk_ids: null argument");
+  CIR_CHECK_ARG(row_ids || index->rows == 0, "stage1_index_topk_ids: row_ids is required");
+  CIR_CHECK_ARG((row_tags == nullptr) == (query_masks == nullptr),
+                "stage1_index_topk_ids: row_tags and query_masks are both NULL (unfiltered) or both set (filtered)");
+  CIR_CHECK_ARG(col_offset >= 0 && id_end >= index->rows && col_offset + id_end <= (1ll << 31),
+                "stage1_index_topk_ids: col_offset %lld + ids up to %lld do not fit int32 indices", (long long)col_offset,
+                (long long)id_end - 1);
+  CIR_ENTER(ctx);
+  if (Q == 0) return CIR_OK;
+  CIR_CHECK_ARG(K >= 1 && K <= MAXK, "stage1_index_topk_ids: K=%lld out of range [1,%d]", (long long)K, MAXK);
+  const size_t need = cir_stage1_index_topk_ids_workspace_bytes(ctx, index, Q, K);
+  if (workspace_bytes < need) { cir_set_error("stage1_index_topk_ids: workspace %zu < %zu bytes", workspace_bytes, need); return CIR_EWORKSPACE; }
+  const size_t search = align_up(cir_stage1_index_topk_workspace_bytes(ctx, index, Q, K), 256);
+  int32_t* ex = nullptr;
+  if (exclude) {
+    ex = (int32_t*)((char*)workspace + search);
+    map_exclude_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, ctx->stream>>>(exclude, Q, row_ids, index->rows, col_offset, ex);
+    CIR_LAUNCH_CHECK(ctx);
+  }
+  CIR_TRY(index_topk("stage1_index_topk_ids", ctx, index, q_emb, Q, row_tags, query_masks, ex, 0, K, top_dist, top_idx, exact_rows,
+                     workspace, search));
+  const int64_t n = Q * K;
+  const unsigned blocks = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)ctx->num_sms * 8);
+  map_ids_kernel<<<blocks, 256, 0, ctx->stream>>>(top_idx, n, row_ids, col_offset);
+  CIR_LAUNCH_CHECK(ctx);
+  return CIR_OK;
+}
+
 __global__ void divide_rows_kernel(float* __restrict__ x, int64_t n, float d) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) x[i] = x[i] / d;
 }

@@ -163,13 +163,14 @@ class ShardedStage1Index:
         self.block = shard_rows(gallery_rows, rank, ws)
         self.index = engine.stage1_index(self.block.stop - self.block.start)
         self.index.add(rows_of(self.block), tags=None if tags_of is None else tags_of(self.block))
+        self.col_offset = self.block.start        # global id of the rank's row id 0: block.start, 0 once compact() made ids global
 
     def topk(self, q_emb, k: int, exclude=None, tags=None) -> Tuple[torch.Tensor, torch.Tensor]:
         """-> merged (dist [Q,k], idx [Q,k]) on every rank; ``q_emb``, ``exclude`` (global row ids) and the query masks ``tags``
         (optional, see ``Stage1Index.topk``) cover all Q queries."""
         def local(rows: slice):
             assert rows == self.block
-            return self.index.topk(q_emb, k, exclude=exclude, col_offset=rows.start, tags=tags)
+            return self.index.topk(q_emb, k, exclude=exclude, col_offset=self.col_offset, tags=tags)
         return sharded_stage1_topk(local, self.engine.topk_merge, self.gallery_rows)
 
     def remove(self, global_rows) -> None:
@@ -179,4 +180,10 @@ class ShardedStage1Index:
         if g.size and (g.min() < 0 or g.max() >= self.gallery_rows):
             raise ValueError(f"remove: rows outside [0, {self.gallery_rows})")
         mine = g[(g >= self.block.start) & (g < self.block.stop)]
-        self.index.remove(mine - self.block.start)
+        self.index.remove(mine - self.col_offset)
+
+    def compact(self) -> None:
+        """Each rank drops the removed rows of its block (``Stage1Index.compact``).  The rank's row ids become the global rows
+        (block.start + local row), so it then searches with col_offset 0; results, ``remove`` and the merge are unchanged."""
+        self.index._compact(None, self.col_offset)
+        self.col_offset = 0

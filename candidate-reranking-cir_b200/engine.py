@@ -641,15 +641,24 @@ class Stage1Index:
 
     ``topk`` never synchronises.  Given device tensors (q_emb fp32 contiguous, exclude and masks int32) and ``out=``, it allocates
     and uploads nothing once its workspace exists for that (Q, k) -- run it once before ``torch.cuda.graph`` capture.  A captured
-    graph searches the rows the index had at capture time, with the tags and masks those tensors hold at replay."""
+    graph searches the rows the index had at capture time, with the tags and masks those tensors hold at replay.
+
+    Row ids: every row keeps the id it was given when it was added (0, 1, 2, ... in the order of ``add``).  ``topk`` returns ids
+    (plus ``col_offset``), ``exclude``, ``set_tags`` and ``remove`` take them.  :meth:`compact` drops the removed rows and
+    :meth:`subset` copies the rows of some tags into a new index; both keep the ids, so they change speed and memory but no search
+    result.  Until the first compaction the ids are the physical row numbers and the index keeps no id table."""
 
     def __init__(self, eng: Engine, capacity: int):
         self.eng = eng
-        self._blob = torch.empty(max(1, eng._lib.cir_stage1_index_bytes(eng.ctx, capacity)), dtype=torch.uint8, device=eng.device)
-        self._s = N.Stage1Index()
         self._ws: Optional[torch.Tensor] = None
         self._retired: List[torch.Tensor] = []    # outgrown workspaces stay alive: a captured graph may still point at one
-        self._tags = torch.full((max(1, capacity),), -1, dtype=torch.int32, device=eng.device)
+        self._ids: Optional[torch.Tensor] = None  # device int32 [capacity + 1] id per physical row, from the first compaction on
+        self._ids_host: Optional[np.ndarray] = None   # host mirror of _ids[:rows] (checks host ids without a synchronisation)
+        self._next_id = 0                         # rows ever added: the id of the next added row
+        self._blob = torch.empty(max(1, eng._lib.cir_stage1_index_bytes(eng.ctx, capacity)), dtype=torch.uint8, device=eng.device)
+        self._s = N.Stage1Index()
+        # one spare slot past the capacity: set_tags with device ids sends the writes of ids that no row holds there
+        self._tags = torch.full((capacity + 1,), -1, dtype=torch.int32, device=eng.device)
         eng._sync_stream()
         N.check(eng._lib.cir_stage1_index_init(eng.ctx, N.ptr(self._blob), self._blob.numel(), capacity, C.byref(self._s)),
                 "cir_stage1_index_init")
@@ -673,6 +682,18 @@ class Stage1Index:
         """int32 [rows] tag bit patterns of the indexed rows (a view: change tags through :meth:`set_tags` / :meth:`remove`)."""
         return self._tags[: self.rows]
 
+    @property
+    def row_ids(self) -> torch.Tensor:
+        """int32 [rows] id of each physical row, strictly increasing (a view after a compaction, ``arange(rows)`` before)."""
+        if self._ids is None:
+            return torch.arange(self.rows, dtype=torch.int32, device=self.eng.device)
+        return self._ids[: self.rows]
+
+    @property
+    def next_id(self) -> int:
+        """The id the next added row gets: the number of rows ever added (compactions do not lower it)."""
+        return self._next_id
+
     def _tag_tensor(self, tags, n: int, what: str) -> torch.Tensor:
         """One int (broadcast), n values (see tag_bits) or an int32 tensor of n bit patterns -> contiguous device int32 [n]."""
         if isinstance(tags, torch.Tensor):
@@ -694,6 +715,8 @@ class Stage1Index:
         g = g_emb.to(self.eng.device, torch.float32).contiguous()
         assert g.dim() == 2 and g.shape[1] == EMBED, g.shape
         n, r0 = g.shape[0], self.rows
+        if self._next_id + n > 1 << 31:
+            raise N.CirError(f"Stage1Index.add: ids {self._next_id}..{self._next_id + n - 1} do not fit int32")
         t = None if tags is None else self._tag_tensor(tags, n, "Stage1Index.add")
         self.eng._sync_stream()
         N.check(self.eng._lib.cir_stage1_index_add(self.eng.ctx, C.byref(self._s), N.ptr(g), n), "cir_stage1_index_add")
@@ -701,32 +724,103 @@ class Stage1Index:
             self._tags[r0:r0 + n].fill_(-1)
         else:
             self._tags[r0:r0 + n].copy_(t)
+        if self._ids is not None:
+            new = np.arange(self._next_id, self._next_id + n, dtype=np.int32)
+            self._ids[r0:r0 + n].copy_(torch.from_numpy(new))
+            self._ids_host = np.concatenate([self._ids_host, new])
+        self._next_id += n
         return self
 
+    def _rows_of(self, ids, what: str, missing_ok: bool) -> torch.Tensor:
+        """Row ids -> device int64 physical rows.  Host ids outside [0, next_id) raise; host ids that no row holds any more (dropped
+        by a compaction) raise unless ``missing_ok``, else they are left out.  Device ids are mapped on the device without a
+        synchronisation; those no row holds go to the spare tag slot past the capacity, so they change no row."""
+        if self._ids is None:                     # ids are physical rows
+            if isinstance(ids, torch.Tensor) and ids.is_cuda:
+                return ids.reshape(-1).long()
+            r_np = np.asarray(ids, dtype=np.int64).reshape(-1)
+            self.eng._check_range(r_np, self.rows, what)
+            return torch.from_numpy(r_np).to(self.eng.device)
+        n = self.rows
+        if isinstance(ids, torch.Tensor) and ids.is_cuda:
+            want = ids.reshape(-1).to(torch.int32)
+            pos = torch.searchsorted(self._ids[:n], want)
+            hit = self._ids[:n][pos.clamp(max=max(n - 1, 0))] == want if n else torch.zeros_like(want, dtype=torch.bool)
+            return torch.where(hit & (pos < n), pos, torch.full_like(pos, self.capacity))
+        i_np = np.asarray(ids, dtype=np.int64).reshape(-1)
+        self.eng._check_range(i_np, self._next_id, what)
+        pos = np.searchsorted(self._ids_host, i_np)
+        hit = (pos < n) & (self._ids_host[np.minimum(pos, max(n - 1, 0))] == i_np) if n else np.zeros(i_np.shape, dtype=bool)
+        if not hit.all():
+            if not missing_ok:
+                raise ValueError(f"{what}: ids {i_np[~hit][:8].tolist()} are no longer in the index (dropped by a compaction)")
+            pos = pos[hit]
+        return torch.from_numpy(pos.astype(np.int64)).to(self.eng.device)
+
     def set_tags(self, rows, tags) -> "Stage1Index":
-        """Set the tags of indexed rows (local row numbers: a device int tensor, or host ints range-checked here) to one int or
-        one value per row.  An on-stream tensor write: with device tensors it can be captured in a CUDA graph."""
-        if isinstance(rows, torch.Tensor) and rows.is_cuda:
-            r = rows.reshape(-1).long()
-        else:
-            r_np = np.asarray(rows, dtype=np.int64).reshape(-1)
-            self.eng._check_range(r_np, self.rows, "Stage1Index.set_tags rows")
-            r = torch.from_numpy(r_np).to(self.eng.device)
+        """Set the tags of indexed rows (row ids: a device int tensor, or host ints checked here) to one int or one value per row.
+        An on-stream tensor write: with device tensors it can be captured in a CUDA graph.  After a compaction, host ids that no
+        row holds any more raise ValueError, device ones are ignored."""
+        r = self._rows_of(rows, "Stage1Index.set_tags rows", missing_ok=False)
         t = self._tag_tensor(tags, r.numel(), "Stage1Index.set_tags")
         self._tags.index_copy_(0, r, t)
         return self
 
     def remove(self, rows) -> "Stage1Index":
-        """Remove indexed rows: their tags become 0, so no filtered search returns them (search with ``tags=ALL_TAGS`` for
-        everything not removed; ``tags=None`` ignores tags).  Row numbers stay; ``set_tags`` restores a row."""
-        return self.set_tags(rows, 0)
+        """Remove indexed rows (row ids): their tags become 0, so no filtered search returns them (search with ``tags=ALL_TAGS``
+        for everything not removed; ``tags=None`` ignores tags until :meth:`compact` drops them).  Ids stay; ``set_tags``
+        restores a row that has not been compacted away.  Removing an id that a compaction already dropped does nothing."""
+        r = self._rows_of(rows, "Stage1Index.remove rows", missing_ok=True)
+        self._tags.index_fill_(0, r, 0)
+        return self
+
+    def _compact_into(self, dst: "Stage1Index", keep_mask: int, id_offset: int = 0) -> None:
+        """cir_stage1_index_compact of this index into the empty index ``dst`` (rows with tag & keep_mask != 0, ids kept)."""
+        eng = self.eng
+        ids = self._ids
+        if ids is None and id_offset:
+            ids = torch.arange(id_offset, id_offset + self.rows, dtype=torch.int32, device=eng.device)
+        dst._ids = torch.zeros(dst.capacity + 1, dtype=torch.int32, device=eng.device)
+        ws = eng.workspace(eng._lib.cir_stage1_index_compact_workspace_bytes(eng.ctx, C.byref(self._s)))
+        eng._sync_stream()
+        N.check(eng._lib.cir_stage1_index_compact(eng.ctx, C.byref(self._s), N.ptr(self._tags), N.ptr(ids), int(keep_mask) & ALL_TAGS,
+                                                  C.byref(dst._s), N.ptr(dst._tags), N.ptr(dst._ids), N.ptr(ws), ws.numel()),
+                "cir_stage1_index_compact")
+        dst._ids_host = dst._ids[: dst.rows].cpu().numpy()
+        dst._next_id = self._next_id + id_offset
+
+    def compact(self, capacity: Optional[int] = None) -> "Stage1Index":
+        """Drop the removed rows (tag 0): the kept rows move, in their order, into a new blob of the same capacity (or of
+        ``capacity``, e.g. to shrink the index), which replaces the old one; their bf16 copy and the gallery maxima are rebuilt
+        from the kept rows.  Ids, tags and every filtered search result stay as they were; a search without tags no longer
+        sees the removed rows.  Synchronises once.  While it runs the index takes two blobs of memory.  CUDA graphs captured
+        before ``compact()`` point at the old blob and must be captured again."""
+        return self._compact(capacity, 0)
+
+    def _compact(self, capacity: Optional[int], id_offset: int) -> "Stage1Index":
+        """:meth:`compact`; ``id_offset`` (first compaction only) is added to the row numbers that serve as ids until then."""
+        assert id_offset == 0 or self._ids is None
+        new = Stage1Index(self.eng, self.capacity if capacity is None else capacity)
+        self._compact_into(new, ALL_TAGS, id_offset)
+        self._blob, self._s, self._tags, self._ids = new._blob, new._s, new._tags, new._ids
+        self._ids_host, self._next_id = new._ids_host, new._next_id
+        return self
+
+    def subset(self, mask, capacity: Optional[int] = None) -> "Stage1Index":
+        """A new index of the rows whose tag shares a bit with ``mask``, in their order, with their ids and tags; this index is
+        unchanged.  ``sub.topk(q, k, exclude=ex)`` equals ``self.topk(q, k, exclude=ex, tags=mask)`` bit for bit.  Capacity: this
+        index's unless given (the subset can grow by ``add``; its new rows get ids from ``next_id`` on).  Synchronises once."""
+        sub = Stage1Index(self.eng, self.capacity if capacity is None else capacity)
+        self._compact_into(sub, int(tag_bits(mask)) & ALL_TAGS)
+        return sub
 
     def topk(self, q_emb: torch.Tensor, k: int, exclude=None, col_offset: int = 0, out=None, exact_rows: Optional[torch.Tensor] = None,
              tags=None):
-        """-> (dist fp32 [Q,k], idx int32 [Q,k]) of the k nearest indexed rows (global index = col_offset + row), skipping
+        """-> (dist fp32 [Q,k], idx int32 [Q,k]) of the k nearest indexed rows (global index = col_offset + row id), skipping
         exclude[q] (-1 = none).  ``out``: optional (dist, idx) to fill.  ``exact_rows``: optional int32 [Q] device tensor, set to 1
         for the queries whose list came from the exact fallback scan.  ``tags``: per-query masks [Q] (or one int for all queries):
-        query q then ranks only the rows with (row tag & tags[q]) != 0 and pads a short list with (+inf, -1)."""
+        query q then ranks only the rows with (row tag & tags[q]) != 0 and pads a short list with (+inf, -1).  After a
+        compaction the search maps ids on the device (cir_stage1_index_topk_ids); it still never synchronises."""
         eng = self.eng
         q = q_emb.to(eng.device, torch.float32).contiguous()
         Q = q.shape[0]
@@ -738,13 +832,19 @@ class Stage1Index:
         assert exact_rows is None or (exact_rows.dtype == torch.int32 and exact_rows.numel() == Q and exact_rows.is_contiguous())
         ex = None if exclude is None else eng._i32(exclude)
         masks = None if tags is None else self._tag_tensor(tags, Q, "Stage1Index.topk")
-        need = eng._lib.cir_stage1_index_topk_workspace_bytes(eng.ctx, C.byref(self._s), Q, k)
+        ws_bytes = eng._lib.cir_stage1_index_topk_workspace_bytes if self._ids is None else eng._lib.cir_stage1_index_topk_ids_workspace_bytes
+        need = ws_bytes(eng.ctx, C.byref(self._s), Q, k)
         if self._ws is None or self._ws.numel() < need:
             if self._ws is not None:
                 self._retired.append(self._ws)
             self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=eng.device)
         eng._sync_stream()
-        if masks is None:
+        if self._ids is not None:
+            N.check(eng._lib.cir_stage1_index_topk_ids(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(self._ids), self._next_id,
+                                                       N.ptr(None if masks is None else self._tags), N.ptr(masks), N.ptr(ex), col_offset,
+                                                       k, N.ptr(td), N.ptr(ti), N.ptr(exact_rows), N.ptr(self._ws), self._ws.numel()),
+                    "cir_stage1_index_topk_ids")
+        elif masks is None:
             N.check(eng._lib.cir_stage1_index_topk(eng.ctx, C.byref(self._s), N.ptr(q), Q, N.ptr(ex), col_offset, k, N.ptr(td), N.ptr(ti),
                                                    N.ptr(exact_rows), N.ptr(self._ws), self._ws.numel()), "cir_stage1_index_topk")
         else:

@@ -158,6 +158,10 @@ _SIGS = {
     "cir_stage1_index_topk_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage1Index), i64, i64]),
     "cir_stage1_index_topk": (C.c_int, [vp, C.POINTER(Stage1Index), vp, i64, vp, i64, i64, vp, vp, vp, vp, C.c_size_t]),
     "cir_stage1_index_topk_filtered": (C.c_int, [vp, C.POINTER(Stage1Index), vp, i64, vp, vp, vp, i64, i64, vp, vp, vp, vp, C.c_size_t]),
+    "cir_stage1_index_compact_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage1Index)]),
+    "cir_stage1_index_compact": (C.c_int, [vp, C.POINTER(Stage1Index), vp, vp, C.c_uint32, C.POINTER(Stage1Index), vp, vp, vp, C.c_size_t]),
+    "cir_stage1_index_topk_ids_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage1Index), i64, i64]),
+    "cir_stage1_index_topk_ids": (C.c_int, [vp, C.POINTER(Stage1Index), vp, i64, vp, i64, vp, vp, vp, i64, i64, vp, vp, vp, vp, C.c_size_t]),
     "cir_stage1_logits": (C.c_int, [vp, vp, vp, i64, i64, C.c_float, vp]),
     "cir_stage1_rank_members": (C.c_int, [vp, vp, vp, vp, i64, i64, vp, vp]),
     "cir_topk_merge": (C.c_int, [vp, vp, vp, i64, i64, i64, vp, vp, vp, C.c_size_t]),

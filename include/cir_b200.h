@@ -249,6 +249,31 @@ int    cir_stage1_index_topk_filtered(cir_ctx* ctx, const cir_stage1_index* inde
                                       const int32_t* exclude, int64_t col_offset, int64_t K,
                                       float* top_dist, int32_t* top_idx, int32_t* exact_rows,
                                       void* workspace, size_t workspace_bytes);
+/* Compaction and subsets: copy the rows r of `src` with (src_tags[r] & keep_mask) != 0, in their order, into `dst` -- an initialised,
+ * EMPTY index in a different blob (overlap: CIR_EINVAL) of the context's dtype -- with their tags in dst_tags and their ids in dst_ids
+ * (device [dst->capacity]).  The id of row r is src_ids[r], or r when src_ids is NULL.  keep_mask 0xFFFFFFFF drops the removed rows
+ * (tag 0); a narrower mask extracts a subset.  dst's blob is byte for byte what cir_stage1_index_add of the kept rows builds: fp32 rows,
+ * bf16 copy and the maxima of the kept rows only.  The call synchronises the stream ONCE to read the kept count (dst->rows is a host
+ * count): a maintenance call, not capturable in a CUDA graph (CIR_EINVAL while the stream captures).  More kept rows than
+ * dst->capacity: CIR_EINVAL and nothing written.  Zero kept rows is valid.  workspace: _compact_workspace_bytes(src). */
+size_t cir_stage1_index_compact_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* src);
+int    cir_stage1_index_compact(cir_ctx* ctx, const cir_stage1_index* src, const uint32_t* src_tags, const int32_t* src_ids,
+                                uint32_t keep_mask, cir_stage1_index* dst, uint32_t* dst_tags, int32_t* dst_ids,
+                                void* workspace, size_t workspace_bytes);
+/* Search an index whose physical row p carries the permanent id row_ids[p] (device [index->rows], strictly increasing, all < id_end --
+ * e.g. the number of rows ever added; compaction keeps the order, so its ids stay increasing).  exclude[q] and the returned indices
+ * are col_offset + id; an excluded id that no row holds excludes nothing.  row_tags and query_masks: both NULL (unfiltered, as
+ * cir_stage1_index_topk) or both set (as cir_stage1_index_topk_filtered).  Because ids increase with the physical rows, ties resolve
+ * as they would over the ids: the result equals the same search over an index that was never compacted, bit for bit.  Never
+ * synchronises (graph-capturable).  col_offset + id_end > 2^31: CIR_EINVAL.  workspace: _topk_ids_workspace_bytes, which is
+ * cir_stage1_index_topk_workspace_bytes plus 4 bytes per query (256-byte aligned). */
+size_t cir_stage1_index_topk_ids_workspace_bytes(const cir_ctx* ctx, const cir_stage1_index* index, int64_t Q, int64_t K);
+int    cir_stage1_index_topk_ids(cir_ctx* ctx, const cir_stage1_index* index, const float* q_emb, int64_t Q,
+                                 const int32_t* row_ids, int64_t id_end,
+                                 const uint32_t* row_tags, const uint32_t* query_masks,   /* both NULL or both set */
+                                 const int32_t* exclude, int64_t col_offset, int64_t K,
+                                 float* top_dist, int32_t* top_idx, int32_t* exact_rows,
+                                 void* workspace, size_t workspace_bytes);
 
 /* In-batch contrastive logits of the stage-I forward: logits[Q, G] = q_emb[Q,256] @ t_emb[G,256]^T / temp, all fp32.
  * Replaces `predicted_features @ target_features.T / self.temp` (src/blip_stage1.py:90-91), forward only. */
