@@ -18,6 +18,7 @@ struct cir_ctx {
   int gemm_impl;        // CIR_GEMM_*
   int attn_impl;        // 0 = auto (tensor cores in bf16 mode), 1 = force the CUDA-core kernel
   int gemm_pair;        // 1 = allow cta_group::2 pair tiles for large GEMMs (default)
+  int gemm_force_pair;  // 1 = take the pair tile whenever gemm_pair allows it, whatever M is (stage-II K/V cache fill)
   int prune_last;       // 1 = stage II computes the last layer for the CLS rows only (default)
   int gemm_tma_store;   // 1 = bf16 GEMM outputs leave through TMA bulk tensor stores (default)
   int fuse_qkv;         // 1 = QKV projection + masked text self-attention as one kernel where eligible (default)

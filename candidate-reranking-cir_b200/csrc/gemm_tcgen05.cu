@@ -667,7 +667,7 @@ int cir_gemm_tcgen05(cir_ctx* ctx, const cir_gemm_args* a) {
   // that is what it takes for the persistent grid to cover the SMs
   const int64_t tiles256 = ((a->M + tc::BM - 1) / tc::BM) * ((a->N + 255) / 256) * a->batch;
   const int64_t pair_tiles = ((a->M + 2 * tc::BM - 1) / (2 * tc::BM)) * ((a->N + 255) / 256) * a->batch;
-  const bool use_pair = ctx->gemm_pair && pair_tiles >= ctx->num_sms / 2;
+  const bool use_pair = ctx->gemm_pair && (ctx->gemm_force_pair || pair_tiles >= ctx->num_sms / 2);
   const bool use128 = !use_pair && ((a->N <= 128) || (tiles256 < ctx->num_sms));
   const int BN = use128 ? 128 : 256;
   const int tile_m = use_pair ? 2 * tc::BM : tc::BM;

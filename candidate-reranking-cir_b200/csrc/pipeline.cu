@@ -73,6 +73,7 @@ extern "C" int cir_create(cir_ctx** out, int device, int dtype) {
   c->gemm_impl = CIR_GEMM_AUTO;
   c->attn_impl = 0;
   c->gemm_pair = 1;
+  c->gemm_force_pair = 0;
   c->prune_last = 1;
   c->dedup_first = 1;
   c->fuse_qkv = 1;
@@ -363,14 +364,15 @@ extern "C" int cir_stage1_gallery_embed(cir_ctx* ctx, const cir_stage1_weights* 
 }
 
 // ========================================================================================== stage II
-struct S2Ws { void *cand, *kv, *emb, *h, *qkv, *ctx, *pre, *a, *qc, *ctxc, *m, *x, *f, *feats; float *hid; size_t total; };
-static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64_t C, int64_t Q, int64_t L, int64_t N) {
+// cached = K/V read from a cir_stage2_kv_cache: no candidate tokens / K/V rows in the workspace, one int32 cache row per triplet
+struct S2Ws { void *cand, *kv, *emb, *h, *qkv, *ctx, *pre, *a, *qc, *ctxc, *m, *x, *f, *feats; float *hid; int32_t* kv_row; size_t total; };
+static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64_t C, int64_t Q, int64_t L, int64_t N, bool cached = false) {
   const size_t es = act_size(ctx);
   const int64_t M = T * L;
   Bump b(ws, bytes);
   S2Ws w;
-  w.cand = b.take(C * N * D * es);
-  w.kv = b.take(C * N * 4 * D * es);
+  w.cand = cached ? nullptr : b.take(C * N * D * es);
+  w.kv = cached ? nullptr : b.take(C * N * 4 * D * es);
   w.emb = b.take(Q * L * D * es);
   w.h = b.take(2 * M * D * es);
   w.qkv = b.take(2 * M * 3 * D * es);
@@ -384,6 +386,7 @@ static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64
   w.f = b.take(2 * M * F * es);
   w.feats = b.take(T * 2 * D * es);
   w.hid = (float*)b.take(T * D * 4);
+  w.kv_row = cached ? (int32_t*)b.take(T * 4) : nullptr;
   w.total = align_up(b.off, 256);
   return w;
 }
@@ -437,6 +440,20 @@ extern "C" int cir_stage2_prefix(cir_ctx* ctx, const cir_stage2_weights* w, cons
   return stage2_query_block(ctx, w, ws.hq, mask, Q, L, ws.qkv, ws.ctx, ws.scratch, a0, qc0);
 }
 
+// kv_row[t] = cand_list[trip_slot[t]] - row0: the cache row of each triplet's candidate (the attention's kv_index)
+__global__ void stage2_kv_rows_kernel(const int32_t* __restrict__ cand_list, const int32_t* __restrict__ trip_slot, int64_t row0,
+                                      int64_t T, int32_t* __restrict__ kv_row) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < T) kv_row[t] = (int32_t)(cand_list[trip_slot[t]] - row0);
+}
+
+// K/V rows of layer i in a cache: act [rows * N][4 * 768]
+static const void* kv_cache_layer(const cir_stage2_kv_cache* c, int i, size_t es) {
+  return (const char*)c->kv + (int64_t)i * c->rows * c->num_tokens * 4 * D * (int64_t)es;
+}
+
+// cache == NULL: the chunk's candidate tokens are gathered and their K/V projected per layer into the workspace (attention reads
+// K/V batch trip_slot[t] of C); otherwise the K/V rows come from the cache (K/V batch kv_row[t] of cache->rows)
 static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const void* gallery_tokens,
                              const int32_t* cand_list, int64_t C, const void* z_t, const int32_t* ids,
                              const int32_t* mask, int64_t Q, int64_t L, int64_t N,
@@ -445,16 +462,26 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                              const int32_t* attn_tiles, int64_t num_attn_tiles,
                              const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                              float* scores, float* feats, void* workspace, size_t workspace_bytes,
-                             const void* a0, const void* qc0) {             // optional cir_stage2_prefix results of the Q queries
+                             const void* a0, const void* qc0,              // optional cir_stage2_prefix results of the Q queries
+                             const cir_stage2_kv_cache* cache) {
   if (T == 0) return CIR_OK;
   CIR_CHECK_ARG(C >= 1 && Q >= 1, "stage2: need at least one candidate and one query");
   CIR_CHECK_ARG(L >= 1 && L <= 512 && N >= 1 && N <= 1024, "stage2: L=%lld N=%lld out of range", (long long)L, (long long)N);
-  S2Ws ws = s2_plan(ctx, workspace, workspace_bytes, T, C, Q, L, N);
+  S2Ws ws = s2_plan(ctx, workspace, workspace_bytes, T, C, Q, L, N, cache != nullptr);
   if (workspace_bytes < ws.total) { cir_set_error("stage2: workspace %zu < %zu", workspace_bytes, ws.total); return CIR_EWORKSPACE; }
   const size_t es = act_size(ctx);
   const int64_t M = T * L;
-  // candidate tokens of this chunk, contiguous [C*N, 768] (validate_stage2.py:251 gather, once per unique image)
-  CIR_TRY(cir_gather_rows(ctx, gallery_tokens, cand_list, ws.cand, C, N * D));
+  const int32_t* kv_index = trip_slot;
+  int32_t kv_batches = (int32_t)C;
+  if (cache) {
+    stage2_kv_rows_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(cand_list, trip_slot, cache->row0, T, ws.kv_row);
+    CIR_LAUNCH_CHECK(ctx);
+    kv_index = ws.kv_row;
+    kv_batches = (int32_t)cache->rows;
+  } else {
+    // candidate tokens of this chunk, contiguous [C*N, 768] (validate_stage2.py:251 gather, once per unique image)
+    CIR_TRY(cir_gather_rows(ctx, gallery_tokens, cand_list, ws.cand, C, N * D));
+  }
   // stream 1 = embeddings (nlvr_encoder.py:880-886), stream 0 = z_t WITHOUT embedding LayerNorm (:892);
   // both expanded over the query's triplets (blip_stage2.py:118-124)
   const int full_layers = ctx->prune_last ? CIR_LAYERS - 1 : CIR_LAYERS;
@@ -501,16 +528,18 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                  M, D, D, 2, CIR_ACT_NONE));
     }   // !per_query
     // K/V projections once per candidate image: rows K0|V0|K1|V1 (:158-159)
-    CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
-                 C * N, 4 * D, D, 1, CIR_ACT_NONE));
+    void* kv = cache ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
+    if (!cache)
+      CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
+                   C * N, 4 * D, D, 1, CIR_ACT_NONE));
     for (int s = 0; s < 2; s++) {
       cir_attn_args c{};
-      c.q = at(ws.qc, s * M * D, es); c.k = at(ws.kv, s * 2 * D, es); c.v = at(ws.kv, s * 2 * D + D, es);
+      c.q = at(ws.qc, s * M * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
       c.o = at(ws.ctxc, s * D, es);
       c.q_bs = L * D; c.q_rs = D; c.k_bs = c.v_bs = N * 4 * D; c.k_rs = c.v_rs = 4 * D; c.o_bs = L * 2 * D; c.o_rs = 2 * D;
-      c.kv_index = trip_slot;
+      c.kv_index = kv_index;
       c.work = attn_work; c.num_work = (int32_t)num_attn_work;
-      c.tiles = attn_tiles; c.num_tiles = (int32_t)num_attn_tiles; c.kv_batches = (int32_t)C;
+      c.tiles = attn_tiles; c.num_tiles = (int32_t)num_attn_tiles; c.kv_batches = kv_batches;
       c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = (int32_t)L; c.Lk = (int32_t)N; c.scale = 0.125f;
       CIR_TRY(cir_attention(ctx, &c));
     }
@@ -548,15 +577,17 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
     CIR_TRY(cir_add_layernorm(ctx, ws.pre, 0, 2 * T, nullptr, w->self_ln_g[i], w->self_ln_b[i], T, ws.a, 0, 2 * T, BERT_EPS));
     CIR_TRY(gemm(ctx, ws.a, D, T * D, w->cross_q_w[i], D, D * D, w->cross_q_b[i], D, ws.qc, D, T * D, 0, nullptr, 0, 0, 0,
                  T, D, D, 2, CIR_ACT_NONE));
-    CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
-                 C * N, 4 * D, D, 1, CIR_ACT_NONE));
+    void* kv = cache ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
+    if (!cache)
+      CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
+                   C * N, 4 * D, D, 1, CIR_ACT_NONE));
     for (int s = 0; s < 2; s++) {
       cir_attn_args c{};
-      c.q = at(ws.qc, s * T * D, es); c.k = at(ws.kv, s * 2 * D, es); c.v = at(ws.kv, s * 2 * D + D, es);
+      c.q = at(ws.qc, s * T * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
       c.o = at(ws.ctxc, s * D, es);
       c.q_bs = D; c.q_rs = D; c.k_bs = c.v_bs = N * 4 * D; c.k_rs = c.v_rs = 4 * D; c.o_bs = 2 * D; c.o_rs = 2 * D;
-      c.kv_index = trip_slot;
-      c.tiles = attn_tiles_cls; c.num_tiles = (int32_t)num_attn_tiles_cls; c.kv_batches = (int32_t)C;
+      c.kv_index = kv_index;
+      c.tiles = attn_tiles_cls; c.num_tiles = (int32_t)num_attn_tiles_cls; c.kv_batches = kv_batches;
       c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = 1; c.Lk = (int32_t)N; c.scale = 0.125f;
       CIR_TRY(cir_attention(ctx, &c));
     }
@@ -586,7 +617,7 @@ extern "C" int cir_stage2_score(cir_ctx* ctx, const cir_stage2_weights* w, const
   CIR_CHECK_ARG(T == 0 || (z_t && ids), "stage2: z_t and ids are required");
   return stage2_score_impl(ctx, w, gallery_tokens, cand_list, C, z_t, ids, mask, Q, L, N, trip_query, trip_slot, T, attn_work, num_attn_work,
                            attn_tiles, num_attn_tiles, attn_tiles_cls, num_attn_tiles_cls, scores, feats, workspace, workspace_bytes,
-                           nullptr, nullptr);
+                           nullptr, nullptr, nullptr);
 }
 
 extern "C" int cir_stage2_score_prefixed(cir_ctx* ctx, const cir_stage2_weights* w, const void* gallery_tokens,
@@ -601,5 +632,71 @@ extern "C" int cir_stage2_score_prefixed(cir_ctx* ctx, const cir_stage2_weights*
   CIR_CHECK_ARG(T == 0 || (a0 && qc0), "stage2_score_prefixed: a0 and qc0 are required");
   return stage2_score_impl(ctx, w, gallery_tokens, cand_list, C, nullptr, nullptr, mask, Q, L, N, trip_query, trip_slot, T, attn_work,
                            num_attn_work, attn_tiles, num_attn_tiles, attn_tiles_cls, num_attn_tiles_cls, scores, feats, workspace,
-                           workspace_bytes, a0, qc0);
+                           workspace_bytes, a0, qc0, nullptr);
+}
+
+// ------------------------------------------------------------------------------------------ resident K/V gallery
+extern "C" size_t cir_stage2_kv_cache_bytes(const cir_ctx* ctx, int64_t rows, int64_t N) {
+  if (rows < 0 || N < 0) return 0;
+  return align_up((size_t)CIR_LAYERS * rows * N * 4 * D * act_size(ctx), 256);
+}
+
+extern "C" int cir_stage2_kv_cache_init(cir_ctx* ctx, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N,
+                                        cir_stage2_kv_cache* out) {
+  CIR_CHECK_ARG(out != nullptr, "stage2_kv_cache_init: out is NULL");
+  CIR_CHECK_ARG(row0 >= 0 && rows >= 0 && row0 + rows <= (1ll << 31) && N >= 1 && N <= 1024,
+                "stage2_kv_cache_init: bad range row0=%lld rows=%lld N=%lld", (long long)row0, (long long)rows, (long long)N);
+  CIR_CHECK_ARG(rows * N < (1ll << 31), "stage2_kv_cache_init: rows * N must stay below 2^31 (attention row index)");
+  const size_t need = cir_stage2_kv_cache_bytes(ctx, rows, N);
+  CIR_CHECK_ARG(rows == 0 || (blob && ((uintptr_t)blob & 255) == 0), "stage2_kv_cache_init: blob must be 256-byte aligned");
+  CIR_CHECK_ARG(bytes >= need, "stage2_kv_cache_init: blob %zu < %zu bytes", bytes, need);
+  out->row0 = row0; out->rows = rows; out->num_tokens = N; out->dtype = ctx->dtype; out->kv = blob;
+  return CIR_OK;
+}
+
+extern "C" int cir_stage2_kv_cache_fill(cir_ctx* ctx, const cir_stage2_weights* w, cir_stage2_kv_cache* cache, const void* tokens,
+                                        int64_t first, int64_t n) {
+  CIR_ENTER(ctx);
+  CIR_CHECK_ARG(w && cache, "stage2_kv_cache_fill: NULL weights or cache");
+  CIR_CHECK_ARG(cache->dtype == ctx->dtype, "stage2_kv_cache_fill: cache dtype %d, context dtype %d", cache->dtype, ctx->dtype);
+  CIR_CHECK_ARG(n >= 0 && first >= cache->row0 && first + n <= cache->row0 + cache->rows,
+                "stage2_kv_cache_fill: rows [%lld, %lld) outside the cache's [%lld, %lld)", (long long)first, (long long)(first + n),
+                (long long)cache->row0, (long long)(cache->row0 + cache->rows));
+  if (n == 0) return CIR_OK;
+  CIR_CHECK_ARG(tokens != nullptr, "stage2_kv_cache_fill: tokens is NULL");
+  const size_t es = act_size(ctx);
+  const int64_t N = cache->num_tokens;
+  // the pair tile whatever n is: a row's bytes must not depend on how many rows share its call
+  ctx->gemm_force_pair = 1;
+  int rc = CIR_OK;
+  for (int i = 0; i < CIR_LAYERS && rc == CIR_OK; i++) {
+    void* dst = at(const_cast<void*>(kv_cache_layer(cache, i, es)), (first - cache->row0) * N * 4 * D, es);
+    rc = gemm(ctx, tokens, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, dst, 4 * D, 0, 0, nullptr, 0, 0, 0, n * N, 4 * D, D, 1,
+              CIR_ACT_NONE);
+  }
+  ctx->gemm_force_pair = 0;
+  return rc;
+}
+
+extern "C" size_t cir_stage2_score_cached_workspace_bytes(const cir_ctx* ctx, int64_t T, int64_t Q, int64_t L, int64_t N) {
+  return s2_plan(ctx, nullptr, 0, T, 0, Q, L, N, true).total;
+}
+
+extern "C" int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache,
+                                       const int32_t* cand_list, int64_t C, const void* z_t, const int32_t* ids,
+                                       const void* a0, const void* qc0,
+                                       const int32_t* mask, int64_t Q, int64_t L,
+                                       const int32_t* trip_query, const int32_t* trip_slot, int64_t T,
+                                       const int32_t* attn_work, int64_t num_attn_work, const int32_t* attn_tiles, int64_t num_attn_tiles,
+                                       const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
+                                       float* scores, float* feats, void* workspace, size_t workspace_bytes) {
+  CIR_ENTER(ctx);
+  CIR_CHECK_ARG(cache != nullptr, "stage2_score_cached: cache is NULL");
+  CIR_CHECK_ARG(cache->dtype == ctx->dtype, "stage2_score_cached: cache dtype %d, context dtype %d", cache->dtype, ctx->dtype);
+  CIR_CHECK_ARG(!a0 == !qc0, "stage2_score_cached: a0 and qc0 come as a pair");
+  CIR_CHECK_ARG(T == 0 || a0 || (z_t && ids), "stage2_score_cached: z_t and ids are required without the a0 / qc0 prefix");
+  CIR_CHECK_ARG(T == 0 || cache->rows >= 1, "stage2_score_cached: empty cache");
+  return stage2_score_impl(ctx, w, nullptr, cand_list, C, a0 ? nullptr : z_t, a0 ? nullptr : ids, mask, Q, L, cache->num_tokens,
+                           trip_query, trip_slot, T, attn_work, num_attn_work, attn_tiles, num_attn_tiles, attn_tiles_cls,
+                           num_attn_tiles_cls, scores, feats, workspace, workspace_bytes, a0, qc0, cache);
 }

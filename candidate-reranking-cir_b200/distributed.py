@@ -113,15 +113,17 @@ def encode_queries_sharded(m1, gallery_tokens, ref_idx, ids, mask) -> torch.Tens
     return all_gather_rows(z_loc, len(ref_idx))
 
 
-def score_matrix_sharded(m2, gallery_tokens, z_all, ids, mask, cand_idx, row_active=None) -> torch.Tensor:
-    """Stage-II scores of all Q*K triplets, candidate-range partitioned over the ranks -> [Q, K] on every rank."""
+def score_matrix_sharded(m2, gallery_tokens, z_all, ids, mask, cand_idx, row_active=None, kv_cache=None) -> torch.Tensor:
+    """Stage-II scores of all Q*K triplets, candidate-range partitioned over the ranks -> [Q, K] on every rank.
+    ``kv_cache``: this rank's Stage2KVCache; it must cover the candidates of the rank's share (e.g. the whole gallery)."""
     import numpy as np
     from .engine import NEG_FILL
     cand_np = cand_idx.cpu().numpy() if isinstance(cand_idx, torch.Tensor) else np.asarray(cand_idx)
     Q, K = cand_np.shape
 
     def pairs(part):
-        pos, sc = m2.engine.stage2_score_pairs(m2._w, gallery_tokens, z_all, ids, mask, cand_np, row_active, part=part)
+        pos, sc = m2.engine.stage2_score_pairs(m2._w, gallery_tokens, z_all, ids, mask, cand_np, row_active, part=part,
+                                               kv_cache=kv_cache)
         return pos, sc, m2.engine.last_plan["part_sizes"]
     return sharded_stage2_scores_by_candidate(pairs, Q, K, NEG_FILL)
 

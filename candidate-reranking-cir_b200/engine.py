@@ -306,25 +306,41 @@ class Engine:
         return out
 
     def stage2_score_chunk(self, w, gallery_tokens, cand_list, z_t, ids, mask, trip_query, trip_slot, want_feats=False,
-                           attn_work=None, attn_tiles=None, attn_tiles_cls=None, prefix=None, out=None):
+                           attn_work=None, attn_tiles=None, attn_tiles_cls=None, prefix=None, out=None, kv_cache=None):
         """One C-ABI call: T triplets sharing C candidates -> (scores fp32 [T], feats fp32 [T,1536] | None).
         ``attn_work``: optional int32 [W,4] K/V-sharing work list (schedule.build_attn_work).
-        ``prefix``: optional (a0, qc0) from :meth:`stage2_prefix` for the same Q queries as ids/mask (z_t is then unused)."""
+        ``prefix``: optional (a0, qc0) from :meth:`stage2_prefix` for the same Q queries as ids/mask (z_t is then unused).
+        ``kv_cache``: optional :class:`Stage2KVCache` holding every candidate of ``cand_list`` (cir_stage2_score_cached; not checked
+        here -- :meth:`stage2_score_pairs` checks it); ``gallery_tokens`` is then unused and may be None."""
         cand_list, ids, mask = self._i32(cand_list), self._i32(ids), self._i32(mask)
         trip_query, trip_slot = self._i32(trip_query), self._i32(trip_slot)
-        T, Cn, (Q, L), n_tok = trip_query.numel(), cand_list.numel(), ids.shape, gallery_tokens.shape[1]
+        T, Cn, (Q, L) = trip_query.numel(), cand_list.numel(), ids.shape
         if prefix is None:
             assert z_t.shape == (Q, L, HIDDEN) and z_t.dtype == self.act_dtype and z_t.is_contiguous()
-        assert gallery_tokens.dtype == self.act_dtype and gallery_tokens.is_contiguous()
+        if kv_cache is None:
+            n_tok = gallery_tokens.shape[1]
+            assert gallery_tokens.dtype == self.act_dtype and gallery_tokens.is_contiguous()
+            need = self._lib.cir_stage2_workspace_bytes(self.ctx, T, Cn, Q, L, n_tok)
+        else:
+            need = self._lib.cir_stage2_score_cached_workspace_bytes(self.ctx, T, Q, L, kv_cache.num_tokens)
         scores = torch.empty(T, dtype=torch.float32, device=self.device) if out is None else out
         assert scores.is_contiguous() and scores.numel() == T and scores.dtype == torch.float32
         feats = torch.empty(T, 2 * HIDDEN, dtype=torch.float32, device=self.device) if want_feats else None
-        need = self._lib.cir_stage2_workspace_bytes(self.ctx, T, Cn, Q, L, n_tok)
         ws = self.workspace(need)
         aw = None if attn_work is None or len(attn_work) == 0 else self._i32(attn_work)
         at = None if attn_tiles is None or len(attn_tiles) == 0 else self._i32(attn_tiles)
         ac = None if attn_tiles_cls is None or len(attn_tiles_cls) == 0 else self._i32(attn_tiles_cls)
         self._sync_stream()
+        if kv_cache is not None:
+            a0, qc0 = (None, None) if prefix is None else prefix
+            if prefix is not None:
+                assert a0.shape == (2, Q * L, HIDDEN) and qc0.shape == a0.shape and a0.dtype == self.act_dtype
+            N.check(self._lib.cir_stage2_score_cached(
+                self.ctx, C.byref(w), C.byref(kv_cache._s), N.ptr(cand_list), Cn, N.ptr(z_t if prefix is None else None), N.ptr(ids),
+                N.ptr(a0), N.ptr(qc0), N.ptr(mask), Q, L, N.ptr(trip_query), N.ptr(trip_slot), T, N.ptr(aw),
+                0 if aw is None else aw.shape[0], N.ptr(at), 0 if at is None else at.shape[0], N.ptr(ac), 0 if ac is None else ac.shape[0],
+                N.ptr(scores), N.ptr(feats), N.ptr(ws), ws.numel()), "cir_stage2_score_cached")
+            return scores, feats
         tail = (Q, L, n_tok, N.ptr(trip_query), N.ptr(trip_slot), T, N.ptr(aw), 0 if aw is None else aw.shape[0],
                 N.ptr(at), 0 if at is None else at.shape[0], N.ptr(ac), 0 if ac is None else ac.shape[0], N.ptr(scores), N.ptr(feats),
                 N.ptr(ws), ws.numel())
@@ -389,10 +405,13 @@ class Engine:
             out.append(t.view(torch.int64).view(a.shape) if a.dtype == np.int64 else t.view(a.shape))
         return out
 
-    def stage2_score_pairs(self, w, gallery_tokens, z_t, ids, mask, cand_idx, row_active=None, part=None):
+    def stage2_score_pairs(self, w, gallery_tokens, z_t, ids, mask, cand_idx, row_active=None, part=None, kv_cache=None):
         """Score this process's share of the Q*K triplets, candidate-major.  ``part=(rank, world)`` restricts the work to the
         rank's contiguous candidate range (schedule.candidate_partition): every candidate's K/V projections stay on ONE rank,
         so the per-GPU K/V reuse does not fall with the number of GPUs.  z_t act [Q,L,768] / ids / mask [Q,L] cover ALL Q queries.
+        ``kv_cache``: a :class:`Stage2KVCache` filled with ``w`` that holds every candidate this process scores: the chunks then
+        read their K/V from it (cir_stage2_score_cached) and are bounded by ``max_triplets`` only.  It is checked against ``w``,
+        the token count of ``gallery_tokens`` and the candidates before anything launches (CirError).
         -> (flat_pos int64 [n] = q*K+k of each scored triplet, scores fp32 [n]) on the device."""
         cand_np = cand_idx.cpu().numpy() if isinstance(cand_idx, torch.Tensor) else np.asarray(cand_idx)
         Q, K = cand_np.shape
@@ -400,7 +419,13 @@ class Engine:
         self._check_range(ids, getattr(self, "vocab_rows", None), "stage2_score_matrix token ids")
         act_np = None if row_active is None else np.asarray(row_active, dtype=bool)
         info: dict = {}
-        chunks = plan_chunks(cand_np, act_np, self.max_triplets, self.max_candidates, part=part, info=info)
+        if kv_cache is not None:
+            kv_cache._check_use(self, w, gallery_tokens.shape[1])
+        # the cached path keeps no per-chunk K/V, so nothing bounds the unique candidates of a chunk
+        max_cand = self.max_candidates if kv_cache is None else max(1, Q * K)
+        chunks = plan_chunks(cand_np, act_np, self.max_triplets, max_cand, part=part, info=info)
+        if kv_cache is not None and chunks:
+            kv_cache._check_rows(min(int(c.cand_list[0]) for c in chunks), max(int(c.cand_list[-1]) for c in chunks))
         self.last_plan = {"part_sizes": info["part_sizes"], "chunks": len(chunks), "triplets": int(sum(c.flat_pos.size for c in chunks)),
                           "candidate_loads": int(sum(c.cand_list.size for c in chunks))}
         ids_d, mask_d = self._i32(ids), self._i32(mask)
@@ -424,21 +449,22 @@ class Engine:
             lists = dict(attn_work=aw, attn_tiles=at, attn_tiles_cls=ac)
             n = ch.flat_pos.size
             if prefix is not None:                              # global query rows: no per-chunk selection of z_t / ids / mask
-                s, _ = self.stage2_score_chunk(w, gallery_tokens, cl, None, ids_d, mask_d, tq, ts, prefix=prefix, out=scores[o:o + n], **lists)
+                s, _ = self.stage2_score_chunk(w, gallery_tokens, cl, None, ids_d, mask_d, tq, ts, prefix=prefix, out=scores[o:o + n],
+                                               kv_cache=kv_cache, **lists)
             else:
                 s, _ = self.stage2_score_chunk(w, gallery_tokens, cl, z_t.index_select(0, ql).contiguous(), ids_d.index_select(0, ql),
-                                               mask_d.index_select(0, ql), tq, ts, out=scores[o:o + n], **lists)
+                                               mask_d.index_select(0, ql), tq, ts, out=scores[o:o + n], kv_cache=kv_cache, **lists)
             pos[o:o + n] = fp
             o += n
         return pos, scores
 
-    def stage2_score_matrix(self, w, gallery_tokens, z_t, ids, mask, cand_idx, row_active=None):
+    def stage2_score_matrix(self, w, gallery_tokens, z_t, ids, mask, cand_idx, row_active=None, kv_cache=None):
         """All Q*K triplets, candidate-major.  z_t act [Q,L,768]; ids/mask [Q,L]; cand_idx [Q,K] ->
         scores fp32 [Q,K]; inactive rows are filled with -99999.99 (src/validate_stage2.py:123,258).
         With more than one chunk, layer 0's query-only part is computed once for all Q queries (stage2_prefix) instead of
-        once per chunk for the chunk's unique queries."""
+        once per chunk for the chunk's unique queries.  ``kv_cache``: see :meth:`stage2_score_pairs` (same scores, bit for bit)."""
         Q, K = cand_idx.shape
-        pos, s = self.stage2_score_pairs(w, gallery_tokens, z_t, ids, mask, cand_idx, row_active)
+        pos, s = self.stage2_score_pairs(w, gallery_tokens, z_t, ids, mask, cand_idx, row_active, kv_cache=kv_cache)
         out = torch.full((Q * K,), NEG_FILL, dtype=torch.float32, device=self.device)
         out.index_copy_(0, pos, s)
         return out.view(Q, K)
@@ -476,6 +502,16 @@ class Engine:
         N.check(self._lib.cir_stage1_topk(self.ctx, N.ptr(q_emb), N.ptr(g_emb), Q, G, N.ptr(ex), col_offset, k, N.ptr(td),
                                           N.ptr(ti), N.ptr(ws), ws.numel()), "cir_stage1_topk")
         return td, ti
+
+    def stage2_kv_cache(self, w, gallery_tokens: torch.Tensor, row0: int = 0, rows: Optional[int] = None) -> "Stage2KVCache":
+        """A resident cross-attention K/V gallery (cir_stage2_kv_cache) of gallery rows [row0, row0 + rows) (default: to the end of
+        ``gallery_tokens``, act [G,N,768]), filled with the packed stage-II weights ``w``: 42.5 MB per image in bf16 at N = 577."""
+        G, n_tok = gallery_tokens.shape[0], gallery_tokens.shape[1]
+        rows = G - row0 if rows is None else rows
+        if row0 < 0 or rows < 0 or row0 + rows > G:
+            raise N.CirError(f"stage2_kv_cache: rows [{row0}, {row0 + rows}) outside the gallery's [0, {G})")
+        cache = Stage2KVCache(self, w, rows, n_tok, row0=row0)
+        return cache.fill(gallery_tokens[row0:row0 + rows], row0)
 
     def stage1_index(self, capacity: int) -> "Stage1Index":
         """An empty resident stage-I gallery index for up to ``capacity`` rows (cir_stage1_index): fill it with
@@ -612,6 +648,82 @@ class Engine:
             N.ptr(gamma.float().contiguous()), N.ptr(beta.float().contiguous()), rows_per_group or rows, N.ptr(y),
             1 if y.dtype == torch.float32 else 0, rows, eps), "cir_add_layernorm")
         return y
+
+
+def _kv_weights_key(w) -> tuple:
+    """The device pointers of the cross-attention K/V weights in a packed cir_stage2_weights: what a K/V cache depends on."""
+    return tuple(int(p or 0) for p in w.cross_kv_w) + tuple(int(p or 0) for p in w.cross_kv_b)
+
+
+class Stage2KVCache:
+    """Resident cross-attention K/V gallery (``cir_stage2_kv_cache`` in include/cir_b200.h): the K0|V0|K1|V1 rows of all 12
+    layers of gallery rows [row0, row0 + rows), computed once by :meth:`fill` and read by every scoring call that passes
+    ``kv_cache=`` (``Engine.stage2_score_matrix``, ``BLIP_NLVR.score_triplets``, the validation drivers).  Those calls then skip the
+    per-chunk token gather and K/V GEMMs (32.7 GF per candidate load) and return the same scores bit for bit.
+
+    The cache remembers the packed weights it is filled with (``weights``; their blob must stay alive, as for any scoring call)
+    and refuses to serve other weights.  ``blob``: optional caller-provided uint8 device tensor of at least ``nbytes``."""
+
+    def __init__(self, eng: Engine, w, rows: int, num_tokens: int, row0: int = 0, blob: Optional[torch.Tensor] = None):
+        self.eng, self.weights = eng, w
+        self._key = _kv_weights_key(w)
+        need = eng._lib.cir_stage2_kv_cache_bytes(eng.ctx, rows, num_tokens)
+        self._blob = torch.empty(max(need, 256), dtype=torch.uint8, device=eng.device) if blob is None else blob
+        if self._blob.device != eng.device or self._blob.dtype != torch.uint8:
+            raise N.CirError(f"Stage2KVCache: the blob must be a uint8 tensor on {eng.device}")
+        self._s = N.Stage2KVCache()
+        N.check(eng._lib.cir_stage2_kv_cache_init(eng.ctx, N.ptr(self._blob), self._blob.numel(), row0, rows, num_tokens,
+                                                  C.byref(self._s)), "cir_stage2_kv_cache_init")
+
+    @property
+    def row0(self) -> int:
+        return int(self._s.row0)
+
+    @property
+    def rows(self) -> int:
+        return int(self._s.rows)
+
+    @property
+    def num_tokens(self) -> int:
+        return int(self._s.num_tokens)
+
+    @property
+    def nbytes(self) -> int:
+        """Bytes of K/V the cache holds (12 layers x rows x N x 3072 activations)."""
+        return int(self.eng._lib.cir_stage2_kv_cache_bytes(self.eng.ctx, self.rows, self.num_tokens))
+
+    def layer(self, i: int) -> torch.Tensor:
+        """View of layer i's K/V rows: act [rows * N, 3072] (K0 | V0 | K1 | V1 columns)."""
+        n = self.rows * self.num_tokens * 4 * HIDDEN
+        es = 2 if self.eng.act_dtype == torch.bfloat16 else 4
+        return self._blob[i * n * es:(i + 1) * n * es].view(self.eng.act_dtype).view(self.rows * self.num_tokens, 4 * HIDDEN)
+
+    def fill(self, tokens: torch.Tensor, first: Optional[int] = None) -> "Stage2KVCache":
+        """Project gallery rows first .. first + n - 1 (``tokens`` act [n, N, 768]; ``first`` defaults to ``row0``) into the cache.
+        Slices may come in any order and any size: the bytes of a row do not depend on them."""
+        eng = self.eng
+        first = self.row0 if first is None else int(first)
+        if tokens.dim() != 3 or tokens.shape[1] != self.num_tokens or tokens.shape[2] != HIDDEN:
+            raise N.CirError(f"Stage2KVCache.fill: tokens {tuple(tokens.shape)} are not [n, {self.num_tokens}, {HIDDEN}]")
+        if tokens.dtype != eng.act_dtype or tokens.device != eng.device:
+            raise N.CirError(f"Stage2KVCache.fill: tokens must be {eng.act_dtype} on {eng.device}")
+        t = tokens.contiguous()
+        eng._sync_stream()
+        N.check(eng._lib.cir_stage2_kv_cache_fill(eng.ctx, C.byref(self.weights), C.byref(self._s), N.ptr(t), first, t.shape[0]),
+                "cir_stage2_kv_cache_fill")
+        return self
+
+    def _check_use(self, eng: Engine, w, num_tokens: int) -> None:
+        if eng.device != self.eng.device:
+            raise N.CirError(f"Stage2KVCache lives on {self.eng.device}, the engine on {eng.device}")
+        if _kv_weights_key(w) != self._key:
+            raise N.CirError("Stage2KVCache was filled with other stage-II weights")
+        if num_tokens != self.num_tokens:
+            raise N.CirError(f"Stage2KVCache holds {self.num_tokens} tokens per image, the gallery has {num_tokens}")
+
+    def _check_rows(self, lo: int, hi: int) -> None:
+        if lo < self.row0 or hi >= self.row0 + self.rows:
+            raise N.CirError(f"candidates [{lo}, {hi}] outside the K/V cache's rows [{self.row0}, {self.row0 + self.rows})")
 
 
 ALL_TAGS = 0xFFFFFFFF

@@ -53,6 +53,10 @@ class Stage1Index(C.Structure):
     _fields_ = [("capacity", i64), ("rows", i64), ("g_f32", vp), ("g_bf16", vp), ("gmax", vp)]
 
 
+class Stage2KVCache(C.Structure):
+    _fields_ = [("row0", i64), ("rows", i64), ("num_tokens", i64), ("dtype", i32), ("kv", vp)]
+
+
 _A = vp * LAYERS
 
 
@@ -176,6 +180,12 @@ _SIGS = {
     "cir_stage2_prefix_workspace_bytes": (C.c_size_t, [vp, i64, i64]),
     "cir_stage2_prefix": (C.c_int, [vp, C.POINTER(Stage2Weights), vp, vp, vp, i64, i64, vp, vp, vp, C.c_size_t]),
     "cir_stage2_score_prefixed": (C.c_int, [vp, C.POINTER(Stage2Weights), vp, vp, i64, vp, vp, vp, i64, i64, i64, vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, vp, vp, C.c_size_t]),
+    "cir_stage2_kv_cache_bytes": (C.c_size_t, [vp, i64, i64]),
+    "cir_stage2_kv_cache_init": (C.c_int, [vp, vp, C.c_size_t, i64, i64, i64, C.POINTER(Stage2KVCache)]),
+    "cir_stage2_kv_cache_fill": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, i64]),
+    "cir_stage2_score_cached_workspace_bytes": (C.c_size_t, [vp, i64, i64, i64, i64]),
+    "cir_stage2_score_cached": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, vp, vp, vp, vp, vp, i64, i64,
+                                          vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, vp, vp, C.c_size_t]),
 }
 
 _lib = None

@@ -83,8 +83,9 @@ def _length_buckets(mask: torch.Tensor, bucket: int):
 
 
 def _predict(blip_model, model_stage1, dataset, index_names, index_features, captions, cand_names, row_active,
-             extra_cand_names=None):
-    """-> (scores [Q,K], extra scores [Q,K'] | None).  z_t is computed once per query and shared by both lists."""
+             extra_cand_names=None, kv_cache=None):
+    """-> (scores [Q,K], extra scores [Q,K'] | None).  z_t is computed once per query and shared by both lists.
+    ``kv_cache``: optional ``blip_model.kv_cache(...)`` of the gallery rows the lists name (same scores, bit for bit)."""
     eng = blip_model.engine
     n2i = _name_index(index_names)
     ref_idx = np.array([n2i[n] for n in dataset.reference_names], dtype=np.int32)
@@ -104,25 +105,28 @@ def _predict(blip_model, model_stage1, dataset, index_names, index_features, cap
         # Under torch.distributed (one process per GPU) the queries' z_t and the candidate ranges are split over the ranks
         # and every rank ends up with the full score rows; single-process: plain calls.
         z_t = encode_queries_sharded(model_stage1, gallery, ref_idx[rows], ids_b, mask_b)
-        scores[r_t] = score_matrix_sharded(blip_model, gallery, z_t, ids_b, mask_b, cand_idx[rows], active[rows])
+        scores[r_t] = score_matrix_sharded(blip_model, gallery, z_t, ids_b, mask_b, cand_idx[rows], active[rows], kv_cache=kv_cache)
         if extra is not None:
-            extra[r_t] = score_matrix_sharded(blip_model, gallery, z_t, ids_b, mask_b, extra_idx[rows], None)
+            extra[r_t] = score_matrix_sharded(blip_model, gallery, z_t, ids_b, mask_b, extra_idx[rows], None, kv_cache=kv_cache)
     return scores, extra
 
 
-def generate_fiq_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features):
+def generate_fiq_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features, kv_cache=None):
     """src/validate_stage2.py:69-129 -> (predicted_logits [Q,K] fp32 on device, target_names)."""
     caps = _fiq_captions(relative_val_dataset.captions)
     active = np.asarray(relative_val_dataset.K_labels).any(axis=1)                  # `if True in K_labels` (:95)
     logits, _ = _predict(blip_model, model_stage1, relative_val_dataset, index_names, index_features, caps,
-                         relative_val_dataset.K_sorted_index_names, active)
+                         relative_val_dataset.K_sorted_index_names, active, kv_cache=kv_cache)
     return logits, list(relative_val_dataset.target_names)
 
 
-def compute_fiq_val_metrics(relative_val_dataset, blip_model, model_stage1, index_features, index_names, return_order: bool = False):
+def compute_fiq_val_metrics(relative_val_dataset, blip_model, model_stage1, index_features, index_names, return_order: bool = False,
+                            kv_cache=None):
     """src/validate_stage2.py:33-66 -> (recall@10, recall@50).  ``return_order=True`` appends the re-ranked order [Q,K] as a
-    HOST int32 array -- the ``sorted_indices`` the reference brings to the CPU at :53."""
-    predicted_logits, _ = generate_fiq_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features)
+    HOST int32 array -- the ``sorted_indices`` the reference brings to the CPU at :53.  ``kv_cache``: optional
+    ``blip_model.kv_cache(...)`` of the gallery (same metrics and order)."""
+    predicted_logits, _ = generate_fiq_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features,
+                                                       kv_cache=kv_cache)
     eng = blip_model.engine
     order = eng.rerank_sort(predicted_logits)                                       # argsort descending (:53)
     labels = torch.from_numpy(np.asarray(relative_val_dataset.K_labels))
@@ -133,7 +137,7 @@ def compute_fiq_val_metrics(relative_val_dataset, blip_model, model_stage1, inde
     return _percent(h10, Q), _percent(h50, Q)
 
 
-def generate_cirr_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features):
+def generate_cirr_val_predictions(blip_model, model_stage1, relative_val_dataset, index_names, index_features, kv_cache=None):
     """src/validate_stage2.py:209-278 -> (predicted_logits [Q,K], group_predicted_logits [Q,5],
     reference_names, target_names, group_members_noRef)."""
     ds = relative_val_dataset
@@ -144,14 +148,14 @@ def generate_cirr_val_predictions(blip_model, model_stage1, relative_val_dataset
     group_noref = [[m for m in row if m != r] for row, r in zip(gm.tolist(), refs.tolist())]
     assert all(len(g) == 5 for g in group_noref)
     logits, group_logits = _predict(blip_model, model_stage1, ds, index_names, index_features, list(ds.captions),
-                                    ds.K_sorted_index_names, active, extra_cand_names=group_noref)
+                                    ds.K_sorted_index_names, active, extra_cand_names=group_noref, kv_cache=kv_cache)
     return logits, group_logits, list(ds.reference_names), list(ds.target_names), group_noref
 
 
-def compute_cirr_val_metrics(relative_val_dataset, blip_model, model_stage1, index_features, index_names):
-    """src/validate_stage2.py:153-206 -> (group_recall@1,2,3, recall@1,5,10,50)."""
+def compute_cirr_val_metrics(relative_val_dataset, blip_model, model_stage1, index_features, index_names, kv_cache=None):
+    """src/validate_stage2.py:153-206 -> (group_recall@1,2,3, recall@1,5,10,50).  ``kv_cache``: as compute_fiq_val_metrics."""
     predicted_logits, group_logits, _, target_names, group_members = generate_cirr_val_predictions(
-        blip_model, model_stage1, relative_val_dataset, index_names, index_features)
+        blip_model, model_stage1, relative_val_dataset, index_names, index_features, kv_cache=kv_cache)
     eng = blip_model.engine
     order = eng.rerank_sort(predicted_logits)                                       # :174
     labels = torch.from_numpy(np.asarray(relative_val_dataset.K_labels))            # :178

@@ -410,6 +410,42 @@ int cir_stage2_score_prefixed(cir_ctx* ctx, const cir_stage2_weights* w, const v
                               const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                               float* scores, float* feats, void* workspace, size_t workspace_bytes);
 
+/* Resident cross-attention K/V gallery: the K0|V0|K1|V1 projections of every layer depend on the gallery image only
+ * (src/nlvr_encoder.py:158-159), so they can be computed once per image and read by every later scoring call.  The blob
+ * (cir_stage2_kv_cache_bytes, 256-byte aligned) is owned by the caller; the struct points into it.  Per layer i the cache holds
+ * act [rows * N][3072] at kv + i * rows * N * 3072 elements: row (r - row0) * N + t is token t of gallery row r, in exactly the
+ * layout cir_stage2_score projects per chunk.  12 * rows * N * 3072 elements: 42.5 MB per image in bf16 at N = 577.
+ *   _init records the row range, N and the context's dtype; it enqueues nothing.  Blob too small or misaligned: CIR_EINVAL.
+ *   _fill projects gallery rows [first, first + n) (tokens act [n, N, 768]) with the cross_kv_w GEMM of each layer, straight
+ *        into the cache; no workspace.  In bf16 contexts it always takes the cta_group::2 pair tile (unless cir_set_gemm_impl
+ *        chose CIR_GEMM_TCGEN05_1CTA), so the bytes do not depend on how the rows are sliced into calls.  Rows outside
+ *        [row0, row0 + rows) or a cache of the other dtype: CIR_EINVAL. */
+typedef struct cir_stage2_kv_cache {
+  int64_t row0, rows;     /* gallery rows [row0, row0 + rows) */
+  int64_t num_tokens;     /* N (577 at 384 px) */
+  int32_t dtype;          /* CIR_DTYPE_* of the context that initialised it */
+  void*   kv;             /* act dtype, per layer i: [rows * N][3072] = K0|V0|K1|V1, at kv + i * rows * N * 3072 */
+} cir_stage2_kv_cache;
+size_t cir_stage2_kv_cache_bytes(const cir_ctx* ctx, int64_t rows, int64_t N);
+int    cir_stage2_kv_cache_init(cir_ctx* ctx, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N, cir_stage2_kv_cache* out);
+int    cir_stage2_kv_cache_fill(cir_ctx* ctx, const cir_stage2_weights* w, cir_stage2_kv_cache* cache,
+                                const void* tokens /* act [n, N, 768]: gallery rows first..first+n-1 */, int64_t first, int64_t n);
+/* cir_stage2_score / cir_stage2_score_prefixed with the candidates' K/V read from a filled cache: no token gather and no K/V
+ * GEMMs, one small kernel maps each triplet to its cache row.  Same chunk description and results; N comes from the cache.
+ * PRECONDITION (not checked on the device): every cand_list entry lies in [cache->row0, cache->row0 + cache->rows) and the cache
+ * was filled with the K/V weights of `w`.  a0 / qc0: optional cir_stage2_prefix pair (then z_t / ids may be NULL); otherwise z_t
+ * and ids are required.  A missing half of the pair, missing z_t / ids or a cache of the other dtype: CIR_EINVAL.  The workspace
+ * has no candidate term.  Never synchronises. */
+size_t cir_stage2_score_cached_workspace_bytes(const cir_ctx* ctx, int64_t T, int64_t Q, int64_t L, int64_t N);
+int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache,
+                            const int32_t* cand_list, int64_t C, const void* z_t, const int32_t* ids,
+                            const void* a0, const void* qc0,
+                            const int32_t* mask, int64_t Q, int64_t L,
+                            const int32_t* trip_query, const int32_t* trip_slot, int64_t T,
+                            const int32_t* attn_work, int64_t num_attn_work, const int32_t* attn_tiles, int64_t num_attn_tiles,
+                            const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
+                            float* scores, float* feats, void* workspace, size_t workspace_bytes);
+
 
 /* ---- weight packing: reference state_dict tensors -> the packed structs above ------------------------------------------
  * A consumer that does not go through the Python host layer binds the reference's checkpoints here: every field of a
