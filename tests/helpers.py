@@ -1,4 +1,4 @@
-"""Shared test helpers: golden fixtures, seeded weights (cached), torch fp32 references for single ops."""
+"""Shared test helpers: golden fixtures, seeded weights (cached)."""
 import functools
 import os
 
@@ -30,20 +30,3 @@ def golden_images(g):
     """The gallery images a fixture was generated from (its ``images`` key names the generator)."""
     fn = syn.make_diverse_images if ("images" in g and str(g["images"]) == "diverse") else syn.make_images
     return fn(int(g["G"]), 384, seed=1)
-
-
-def ref_attention(q, k, v, key_mask=None, kv_index=None, scale=0.125):
-    """fp32 torch reference of cir_attention: q [B,Lq,H*64], k/v [Bk,Lk,H*64]."""
-    q, k, v = q.float(), k.float(), v.float()
-    if kv_index is not None:
-        k, v = k[kv_index.long()], v[kv_index.long()]
-    B, Lq, HD = q.shape
-    H = HD // 64
-    qh = q.view(B, Lq, H, 64).permute(0, 2, 1, 3)
-    kh = k.view(B, -1, H, 64).permute(0, 2, 1, 3)
-    vh = v.view(B, -1, H, 64).permute(0, 2, 1, 3)
-    s = qh @ kh.transpose(-1, -2) * scale
-    if key_mask is not None:
-        s = s + (1.0 - key_mask.float())[:, None, None, :] * -10000.0
-    o = torch.softmax(s, -1) @ vh
-    return o.permute(0, 2, 1, 3).reshape(B, Lq, HD)
