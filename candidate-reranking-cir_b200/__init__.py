@@ -19,7 +19,7 @@ def __getattr__(name):
     # importable on machines without the built extension.
     import importlib
     if name in ("native", "engine", "schedule", "blip", "blip_stage1", "blip_stage2", "validate",
-                "validate_stage2", "distributed", "topk_file", "checkpoint", "build"):
+                "validate_stage2", "distributed", "topk_file", "checkpoint", "build", "online"):
         return importlib.import_module(f"{__name__}.{name}")
     for mod in ("blip_stage1", "blip_stage2"):
         if name in ("BLIP_Retrieval", "BLIP_NLVR"):

@@ -90,6 +90,13 @@ class BLIP_NLVR(nn.Module):
         self._need_weights()
         return self.engine.stage2_score_matrix(self._w, gallery_tokens, z_t, ids, mask, cand_idx, row_active, kv_cache=kv_cache)
 
+    def rerank_topk(self, z_t, ids, mask, cand_idx, kv_cache, out=None):
+        """Re-rank a device-resident top-K list cand_idx int32 [Q,K] (e.g. the idx of engine.Stage1Index.topk) through ``kv_cache``
+        without the host (engine.Engine.stage2_rerank_cached) -> (scores fp32 [Q,K], order int32 [Q,K], ranked int32 [Q,K]).
+        The scores are those of :meth:`score_triplets` with ``kv_cache``; capturable in a CUDA graph."""
+        self._need_weights()
+        return self.engine.stage2_rerank_cached(self._w, kv_cache, z_t, ids, mask, cand_idx, out=out)
+
     def kv_cache(self, gallery_tokens, row0: int = 0, rows: Optional[int] = None):
         """The cross-attention K/V of gallery rows [row0, row0 + rows) under this model's weights, computed once
         (engine.Stage2KVCache): 42.5 MB per 384 px image in bf16.  Pass it as ``kv_cache=`` to score_triplets / the drivers."""

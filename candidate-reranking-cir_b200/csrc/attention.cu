@@ -479,3 +479,18 @@ extern "C" int cir_attention(cir_ctx* ctx, const cir_attn_args* a) {
   CIR_LAUNCH_CHECK(ctx);
   return CIR_OK;
 }
+
+// cir_attention for a tile list whose length the device wrote (a->tiles with at most a->num_tiles entries, the count at *ntiles_dev):
+// the tcgen05 kernel reads the count itself; every other kernel ignores tile and work lists and runs each batch as its own run.
+int cir_attention_counted(cir_ctx* ctx, const cir_attn_args* a, const int32_t* ntiles_dev) {
+  CIR_ENTER(ctx);
+  if (a->B == 0 || a->Lq == 0) return CIR_OK;
+  if (ctx->dtype == CIR_DTYPE_BF16 && ctx->attn_impl == 0) {
+    const int rc = cir_attention_tc_counted(ctx, a, ntiles_dev);
+    if (rc != CIR_EUNSUPPORTED) return rc;
+  }
+  cir_attn_args b = *a;
+  b.work = nullptr; b.num_work = 0;
+  b.tiles = nullptr; b.num_tiles = 0;
+  return cir_attention(ctx, &b);
+}

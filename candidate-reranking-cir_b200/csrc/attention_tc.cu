@@ -132,13 +132,21 @@ __device__ __forceinline__ Item decode_rows(const cir_attn_args& p, int w, int n
   return it;
 }
 
+// COUNTED: the tile count is read once from ntiles_dev (written on the device by an earlier kernel of the stream, e.g. the
+// on-device planner of cir_stage2_rerank_cached); the grid was sized from the host bound `ntiles`, and CTAs past the device
+// count have no items.  Every role derives its items from this one value.
+template <bool COUNTED>
 __global__ void __launch_bounds__(THREADS, 1)
 attention_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                     const __grid_constant__ CUtensorMap map_v, const __grid_constant__ CUtensorMap map_o, const cir_attn_args p,
-                    int cpb, int ntiles, int RB, int total) {
+                    int cpb, int ntiles, int RB, int total, const int32_t* __restrict__ ntiles_dev) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if (COUNTED) {
+    ntiles = __ldg(ntiles_dev);
+    total = ntiles * p.H;
+  }
   const int nch = (p.Lk + KC - 1) / KC;
   const int n_my = (int)blockIdx.x < total ? (total - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
   const int total_g = n_my * nch;
@@ -447,7 +455,9 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_cons
 
 }  // namespace fatc
 
-int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a) {
+// ntiles_dev == NULL: the tile count is a->num_tiles (or one tile per 256-row slice of every batch without a tile list).
+// Otherwise a->tiles is required, a->num_tiles bounds the count the kernel reads from ntiles_dev, and the grid is sized from that bound.
+static int attention_tc_launch(cir_ctx* ctx, const cir_attn_args* a, const int32_t* ntiles_dev) {
   // eligibility (the caller falls back to the mma.sync kernel on CIR_EUNSUPPORTED)
   if (ctx->dtype != CIR_DTYPE_BF16 || a->key_mask != nullptr || a->Lk < 16 || a->kv_batches <= 0 || a->H * 64 > 65536 ||
       a->k_bs != (int64_t)a->Lk * a->k_rs || a->v_bs != (int64_t)a->Lk * a->v_rs || (a->k_rs % 8) || (a->v_rs % 8) ||
@@ -466,9 +476,11 @@ int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a) {
   CIR_TRY(cir_make_map_3d(ctx, &mo, a->o, (int64_t)a->H * 64, a->Lq, a->B, a->o_rs, a->o_bs, 64, 32, 1));
   CIR_TRY(cir_make_map_2d(ctx, &mk, a->k, kv_rows, (int64_t)a->H * 64, a->k_rs, fatc::KC));
   CIR_TRY(cir_make_map_2d(ctx, &mv, a->v, kv_rows, (int64_t)a->H * 64, a->v_rs, fatc::KC));
-  if (!(ctx->func_attr_mask & (1u << 3))) {                  // per context: the attribute is per device
-    CIR_CUDA(cudaFuncSetAttribute(fatc::attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fatc::SMEM_BYTES));
-    ctx->func_attr_mask |= 1u << 3;
+  const unsigned bit = ntiles_dev ? 1u << 4 : 1u << 3;       // per context: the attribute is per device
+  if (!(ctx->func_attr_mask & bit)) {
+    CIR_CUDA(cudaFuncSetAttribute(ntiles_dev ? (const void*)fatc::attention_tc_kernel<true> : (const void*)fatc::attention_tc_kernel<false>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, fatc::SMEM_BYTES));
+    ctx->func_attr_mask |= bit;
   }
   const int cpb = (a->Lq + 255) / 256;
   const int64_t ntiles = a->tiles ? (int64_t)a->num_tiles : (int64_t)a->B * cpb;
@@ -477,8 +489,19 @@ int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a) {
   if (total >= (1ll << 31)) return CIR_EUNSUPPORTED;
   const unsigned gx = (unsigned)std::min<int64_t>(total, (int64_t)ctx->num_sms);      // persistent: one CTA per SM
   cir_prof_begin(ctx, CIR_PROF_ATTN_TC, 4.0 * (double)a->B * a->H * (double)a->Lq * (double)a->Lk * 64.0);
-  fatc::attention_tc_kernel<<<gx, fatc::THREADS, fatc::SMEM_BYTES, ctx->stream>>>(mq, mk, mv, mo, *a, cpb, (int)ntiles, RB, (int)total);
+  if (ntiles_dev)
+    fatc::attention_tc_kernel<true><<<gx, fatc::THREADS, fatc::SMEM_BYTES, ctx->stream>>>(mq, mk, mv, mo, *a, 1, 0, RB, 0, ntiles_dev);
+  else
+    fatc::attention_tc_kernel<false><<<gx, fatc::THREADS, fatc::SMEM_BYTES, ctx->stream>>>(mq, mk, mv, mo, *a, cpb, (int)ntiles, RB, (int)total,
+                                                                                          nullptr);
   cir_prof_end(ctx);
   CIR_LAUNCH_CHECK(ctx);
   return CIR_OK;
+}
+
+int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a) { return attention_tc_launch(ctx, a, nullptr); }
+
+int cir_attention_tc_counted(cir_ctx* ctx, const cir_attn_args* a, const int32_t* ntiles_dev) {
+  CIR_CHECK_ARG(a->tiles && ntiles_dev, "attention_tc_counted: needs a tile list and its device count");
+  return attention_tc_launch(ctx, a, ntiles_dev);
 }

@@ -128,6 +128,11 @@ int cir_make_map_2d(cir_ctx* ctx, CUtensorMap* map, const void* base, int64_t ro
 int cir_make_map_3d(cir_ctx* ctx, CUtensorMap* map, const void* base, int64_t d0, int64_t d1, int64_t d2, int64_t s1, int64_t s2,
                     int b0, int b1, int b2);
 int cir_attention_tc(cir_ctx* ctx, const cir_attn_args* a);
+int cir_attention_tc_counted(cir_ctx* ctx, const cir_attn_args* a, const int32_t* ntiles_dev);   // tile count read on the device
+int cir_attention_counted(cir_ctx* ctx, const cir_attn_args* a, const int32_t* ntiles_dev);      // attention.cu
+// stage2_plan.cu: the two kernels after the scoring of an on-device plan (cir_stage2_rerank_cached)
+int cir_stage2_scatter_scores(cir_ctx* ctx, const float* sorted, const int32_t* flat_pos, int64_t T, const int32_t* counts, float* scores);
+int cir_stage2_gather_ranked(cir_ctx* ctx, const int32_t* cand, const int32_t* order, int64_t Q, int64_t K, int32_t* ranked);
 bool cir_qkv_attention_supported(const cir_ctx* ctx, int64_t L);   // qkv_attention.cu
 // stage1_topk_tc.cu: tensor-core candidate filter + exact fp32 re-check, per-query exact fallback on the device (never synchronises).
 // A gallery "view" is the fp32 rows, their bf16 copy and gmax = {max ||g||, max ||g - bf16(g)||} as float bits.

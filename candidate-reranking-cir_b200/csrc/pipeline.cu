@@ -453,7 +453,10 @@ static const void* kv_cache_layer(const cir_stage2_kv_cache* c, int i, size_t es
 }
 
 // cache == NULL: the chunk's candidate tokens are gathered and their K/V projected per layer into the workspace (attention reads
-// K/V batch trip_slot[t] of C); otherwise the K/V rows come from the cache (K/V batch kv_row[t] of cache->rows)
+// K/V batch trip_slot[t] of C); otherwise the K/V rows come from the cache (K/V batch kv_row[t] of cache->rows).
+// tile_counts (cached only; NULL from every host-planned caller): device {tiles, cls tiles} of an on-device plan
+// (cir_stage2_plan_topk).  trip_slot then holds each triplet's cache row, and attn_tiles / attn_tiles_cls hold at most T entries,
+// of which the two cross-attentions read as many as the device counts say.
 static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const void* gallery_tokens,
                              const int32_t* cand_list, int64_t C, const void* z_t, const int32_t* ids,
                              const int32_t* mask, int64_t Q, int64_t L, int64_t N,
@@ -463,7 +466,7 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                              const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                              float* scores, float* feats, void* workspace, size_t workspace_bytes,
                              const void* a0, const void* qc0,              // optional cir_stage2_prefix results of the Q queries
-                             const cir_stage2_kv_cache* cache) {
+                             const cir_stage2_kv_cache* cache, const int32_t* tile_counts = nullptr) {
   if (T == 0) return CIR_OK;
   CIR_CHECK_ARG(C >= 1 && Q >= 1, "stage2: need at least one candidate and one query");
   CIR_CHECK_ARG(L >= 1 && L <= 512 && N >= 1 && N <= 1024, "stage2: L=%lld N=%lld out of range", (long long)L, (long long)N);
@@ -473,7 +476,9 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
   const int64_t M = T * L;
   const int32_t* kv_index = trip_slot;
   int32_t kv_batches = (int32_t)C;
-  if (cache) {
+  if (cache && tile_counts) {
+    kv_batches = (int32_t)cache->rows;               // trip_slot already holds the cache rows
+  } else if (cache) {
     stage2_kv_rows_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(cand_list, trip_slot, cache->row0, T, ws.kv_row);
     CIR_LAUNCH_CHECK(ctx);
     kv_index = ws.kv_row;
@@ -541,7 +546,7 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
       c.work = attn_work; c.num_work = (int32_t)num_attn_work;
       c.tiles = attn_tiles; c.num_tiles = (int32_t)num_attn_tiles; c.kv_batches = kv_batches;
       c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = (int32_t)L; c.Lk = (int32_t)N; c.scale = 0.125f;
-      CIR_TRY(cir_attention(ctx, &c));
+      CIR_TRY(tile_counts ? cir_attention_counted(ctx, &c, tile_counts) : cir_attention(ctx, &c));
     }
     // m = merge(dense0(c0), dense1(c1)) folded into one K=1536 GEMM (:250-258); x_s = LayerNorm{A,B}(m + a_s) (:256,:260)
     CIR_TRY(gemm(ctx, ws.ctxc, 2 * D, 0, w->cross_out_w[i], 2 * D, 0, w->cross_out_b[i], 0, ws.m, D, 0, 0, nullptr, 0, 0, 0,
@@ -589,7 +594,7 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
       c.kv_index = kv_index;
       c.tiles = attn_tiles_cls; c.num_tiles = (int32_t)num_attn_tiles_cls; c.kv_batches = kv_batches;
       c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = 1; c.Lk = (int32_t)N; c.scale = 0.125f;
-      CIR_TRY(cir_attention(ctx, &c));
+      CIR_TRY(tile_counts ? cir_attention_counted(ctx, &c, tile_counts + 1) : cir_attention(ctx, &c));
     }
     CIR_TRY(gemm(ctx, ws.ctxc, 2 * D, 0, w->cross_out_w[i], 2 * D, 0, w->cross_out_b[i], 0, ws.m, D, 0, 0, nullptr, 0, 0, 0,
                  T, D, 2 * D, 1, CIR_ACT_NONE));
@@ -699,4 +704,58 @@ extern "C" int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w
   return stage2_score_impl(ctx, w, nullptr, cand_list, C, a0 ? nullptr : z_t, a0 ? nullptr : ids, mask, Q, L, cache->num_tokens,
                            trip_query, trip_slot, T, attn_work, num_attn_work, attn_tiles, num_attn_tiles, attn_tiles_cls,
                            num_attn_tiles_cls, scores, feats, workspace, workspace_bytes, a0, qc0, cache);
+}
+
+// ------------------------------------------------------------------------------------------ re-ranking a device-resident top-K list
+constexpr int64_t RERANK_MAX_T = 16384;          // one planning CTA (stage2_plan.cu)
+constexpr int64_t RERANK_MAX_K = 2048;           // cir_rerank_sort
+
+struct RerankWs { int32_t *flat_pos, *kv_row, *trip_query, *tiles, *tiles_cls, *counts; float* sorted; void* s2; size_t s2_bytes, total; };
+static RerankWs rerank_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t Q, int64_t K, int64_t L, int64_t N) {
+  const int64_t T = Q * K;
+  Bump b(ws, bytes);
+  RerankWs w;
+  w.flat_pos = (int32_t*)b.take(T * 4);
+  w.kv_row = (int32_t*)b.take(T * 4);
+  w.trip_query = (int32_t*)b.take(T * 4);
+  w.tiles = (int32_t*)b.take(T * 16);
+  w.tiles_cls = (int32_t*)b.take(T * 16);
+  w.counts = (int32_t*)b.take(3 * 4);
+  w.sorted = (float*)b.take(T * 4);
+  w.s2_bytes = s2_plan(ctx, nullptr, 0, T, 0, Q, L, N, true).total;
+  w.s2 = b.take(w.s2_bytes);
+  w.total = align_up(b.off, 256);
+  return w;
+}
+extern "C" size_t cir_stage2_rerank_cached_workspace_bytes(const cir_ctx* ctx, int64_t Q, int64_t K, int64_t L, int64_t N) {
+  if (Q < 1 || K < 1 || L < 1 || N < 1) return 0;
+  return rerank_plan(ctx, nullptr, 0, Q, K, L, N).total;
+}
+
+extern "C" int cir_stage2_rerank_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache, const int32_t* cand,
+                                        int64_t Q, int64_t K, const void* z_t, const int32_t* ids, const int32_t* mask, int64_t L,
+                                        float* scores, int32_t* order, int32_t* ranked, int32_t* counts, void* workspace,
+                                        size_t workspace_bytes) {
+  CIR_ENTER(ctx);
+  CIR_CHECK_ARG(w && cache && cand && z_t && ids && mask && scores && order, "stage2_rerank_cached: NULL argument");
+  CIR_CHECK_ARG(cache->dtype == ctx->dtype, "stage2_rerank_cached: cache dtype %d, context dtype %d", cache->dtype, ctx->dtype);
+  CIR_CHECK_ARG(cache->rows >= 1, "stage2_rerank_cached: empty cache");
+  CIR_CHECK_ARG(Q >= 1 && K >= 1 && K <= RERANK_MAX_K && Q * K <= RERANK_MAX_T,
+                "stage2_rerank_cached: Q=%lld x K=%lld outside K <= %lld, Q*K <= %lld", (long long)Q, (long long)K,
+                (long long)RERANK_MAX_K, (long long)RERANK_MAX_T);
+  CIR_CHECK_ARG(L >= 1 && L <= 256, "stage2_rerank_cached: L=%lld outside [1, 256]", (long long)L);
+  CIR_CHECK_ARG(cache->rows < (1ll << 18) - 1, "stage2_rerank_cached: a cache of %lld rows (at most 2^18 - 2)", (long long)cache->rows);
+  const RerankWs ws = rerank_plan(ctx, workspace, workspace_bytes, Q, K, L, cache->num_tokens);
+  if (workspace_bytes < ws.total) { cir_set_error("stage2_rerank_cached: workspace %zu < %zu", workspace_bytes, ws.total); return CIR_EWORKSPACE; }
+  const int64_t T = Q * K;
+  int32_t* cnt = counts ? counts : ws.counts;
+  CIR_TRY(cir_stage2_plan_topk(ctx, cand, Q, K, L, cache->row0, cache->rows, ws.flat_pos, ws.kv_row, ws.trip_query, ws.tiles,
+                               ws.tiles_cls, cnt));
+  // one chunk of all T triplets, in the plan's candidate-major order: C is unused with a cache and the tile lists are bounded by T
+  CIR_TRY(stage2_score_impl(ctx, w, nullptr, nullptr, T, z_t, ids, mask, Q, L, cache->num_tokens, ws.trip_query, ws.kv_row, T,
+                            nullptr, 0, ws.tiles, T, ws.tiles_cls, T, ws.sorted, nullptr, ws.s2, ws.s2_bytes, nullptr, nullptr, cache, cnt));
+  CIR_TRY(cir_stage2_scatter_scores(ctx, ws.sorted, ws.flat_pos, T, cnt, scores));
+  CIR_TRY(cir_rerank_sort(ctx, scores, Q, K, order));
+  if (ranked) CIR_TRY(cir_stage2_gather_ranked(ctx, cand, order, Q, K, ranked));
+  return CIR_OK;
 }

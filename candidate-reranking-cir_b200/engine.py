@@ -18,6 +18,7 @@ from .schedule import build_attn_tiles, build_attn_work, plan_chunks
 
 HIDDEN, FFN, LAYERS, EMBED = 768, 3072, 12, 256
 NEG_FILL = -99999.99          # src/validate_stage2.py:123,258
+RERANK_MAX_TRIPLETS = 16384   # triplets per cir_stage2_rerank_cached call (one planning CTA)
 
 
 class Engine:
@@ -44,6 +45,8 @@ class Engine:
         self.max_candidates = int(os.environ.get("CIR_MAX_CANDIDATES", 64))
         self.query_prefix = True       # stage2_score_matrix: layer 0's query-only part once per query set (cir_stage2_prefix)
         self.prefix_batch = 8192       # queries per cir_stage2_prefix call (bounds its workspace: ~0.7 MB per query at L = 32)
+        self._rr_ws: Optional[torch.Tensor] = None    # stage2_rerank_cached's own workspace (never Engine.workspace: see there)
+        self._rr_retired: List[torch.Tensor] = []     # outgrown workspaces stay alive: a captured graph may still point at one
 
     # ------------------------------------------------------------------ plumbing
     def _sync_stream(self):
@@ -274,8 +277,9 @@ class Engine:
         return out
 
     def stage1_encode(self, w, gallery_tokens: torch.Tensor, ref_index, ids, mask, want_z=True, want_emb=True,
-                      normalize_twice=False, batch: int = 256):
-        """-> (z_t act [Q,L,768] | None, q_emb fp32 [Q,256] | None)"""
+                      normalize_twice=False, batch: int = 256, workspace: Optional[torch.Tensor] = None):
+        """-> (z_t act [Q,L,768] | None, q_emb fp32 [Q,256] | None).  ``workspace``: optional caller-owned uint8 device tensor of at
+        least cir_stage1_workspace_bytes for one batch (default: :meth:`workspace`)."""
         self._check_range(ref_index, gallery_tokens.shape[0], "stage1_encode ref_index")
         self._check_range(ids, getattr(self, "vocab_rows", None), "stage1_encode token ids")
         ref_index, ids, mask = self._i32(ref_index), self._i32(ids), self._i32(mask)
@@ -288,7 +292,7 @@ class Engine:
         for q0 in range(0, Q, batch):
             nq = min(batch, Q - q0)
             need = self._lib.cir_stage1_workspace_bytes(self.ctx, nq, L, n_tok)
-            ws = self.workspace(need)
+            ws = self.workspace(need) if workspace is None else workspace
             N.check(self._lib.cir_stage1_encode(
                 self.ctx, C.byref(w), N.ptr(gallery_tokens), N.ptr(ref_index[q0:q0 + nq]), N.ptr(ids[q0:q0 + nq]),
                 N.ptr(mask[q0:q0 + nq]), nq, L, n_tok, N.ptr(z[q0:q0 + nq]) if want_z else N.vp(0),
@@ -468,6 +472,45 @@ class Engine:
         out = torch.full((Q * K,), NEG_FILL, dtype=torch.float32, device=self.device)
         out.index_copy_(0, pos, s)
         return out.view(Q, K)
+
+    def stage2_rerank_cached(self, w, kv_cache: "Stage2KVCache", z_t, ids, mask, cand, out=None):
+        """Re-rank the candidate lists cand int [Q,K] (normally the idx of :meth:`Stage1Index.topk`, already on the device) through
+        the resident K/V gallery, with no host round trip (cir_stage2_rerank_cached): the candidate-major plan is built on the
+        device, so nothing is read back and the call can be captured in a CUDA graph.  z_t act [Q,L,768]; ids / mask [Q,L].
+        -> (scores fp32 [Q,K], order int32 [Q,K] = rerank_sort(scores), ranked int32 [Q,K] = cand[q, order[q, r]]).
+
+        The scores equal stage2_score_matrix(..., kv_cache=kv_cache) when that runs as one chunk, bit for bit.  Entries of -1 (the
+        padding of a filtered search) or outside the cache's rows score -99999.99 and rank last.  Query sets larger than
+        max(1, max_triplets // K) queries go through several calls; none synchronises.  The cache is checked against ``w`` on the
+        host, the candidates are not (they stay on the device).  ``out``: optional (scores, order, ranked) to fill; with device
+        int32 cand / ids / mask and ``out``, a warmed-up call allocates and uploads nothing."""
+        kv_cache._check_use(self, w, kv_cache.num_tokens)
+        cand, ids, mask = self._i32(cand), self._i32(ids), self._i32(mask)
+        assert cand.dim() == 2 and ids.dim() == 2 and mask.shape == ids.shape
+        Q, K = cand.shape
+        L = ids.shape[1]
+        assert ids.shape[0] == Q and z_t.shape == (Q, L, HIDDEN) and z_t.dtype == self.act_dtype and z_t.is_contiguous()
+        if out is None:
+            out = (torch.empty(Q, K, dtype=torch.float32, device=self.device), torch.empty(Q, K, dtype=torch.int32, device=self.device),
+                   torch.empty(Q, K, dtype=torch.int32, device=self.device))
+        scores, order, ranked = out
+        assert scores.shape == order.shape == ranked.shape == (Q, K) and scores.dtype == torch.float32
+        assert order.dtype == ranked.dtype == torch.int32 and all(t.is_contiguous() for t in out)
+        qb = max(1, min(self.max_triplets, RERANK_MAX_TRIPLETS) // K)
+        need = self._lib.cir_stage2_rerank_cached_workspace_bytes(self.ctx, min(qb, Q), K, L, kv_cache.num_tokens)
+        if self._rr_ws is None or self._rr_ws.numel() < need:
+            if self._rr_ws is not None:
+                self._rr_retired.append(self._rr_ws)
+            self._rr_ws = torch.empty(max(need, 256), dtype=torch.uint8, device=self.device)
+        ws = self._rr_ws
+        self._sync_stream()
+        for q0 in range(0, Q, qb):
+            n = min(qb, Q - q0)
+            N.check(self._lib.cir_stage2_rerank_cached(
+                self.ctx, C.byref(w), C.byref(kv_cache._s), N.ptr(cand[q0:q0 + n]), n, K, N.ptr(z_t[q0:q0 + n]), N.ptr(ids[q0:q0 + n]),
+                N.ptr(mask[q0:q0 + n]), L, N.ptr(scores[q0:q0 + n]), N.ptr(order[q0:q0 + n]), N.ptr(ranked[q0:q0 + n]), None,
+                N.ptr(ws), ws.numel()), "cir_stage2_rerank_cached")
+        return scores, order, ranked
 
     # ------------------------------------------------------------------ sort / top-K / recall
     def rerank_sort(self, scores: torch.Tensor) -> torch.Tensor:

@@ -186,6 +186,10 @@ _SIGS = {
     "cir_stage2_score_cached_workspace_bytes": (C.c_size_t, [vp, i64, i64, i64, i64]),
     "cir_stage2_score_cached": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, vp, vp, vp, vp, vp, i64, i64,
                                           vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, vp, vp, C.c_size_t]),
+    "cir_stage2_plan_topk": (C.c_int, [vp, vp, i64, i64, i64, i64, i64, vp, vp, vp, vp, vp, vp]),
+    "cir_stage2_rerank_cached_workspace_bytes": (C.c_size_t, [vp, i64, i64, i64, i64]),
+    "cir_stage2_rerank_cached": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, i64, vp, vp, vp, i64,
+                                           vp, vp, vp, vp, vp, C.c_size_t]),
 }
 
 _lib = None

@@ -446,6 +446,36 @@ int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir
                             const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                             float* scores, float* feats, void* workspace, size_t workspace_bytes);
 
+/* Re-ranking a top-K list that lives on the device (e.g. the top_idx of cir_stage1_index_topk) through a filled K/V cache, with no
+ * host round trip: every call below only enqueues kernels, never synchronises and never touches host memory, so the whole
+ * "stage-I search -> stage-II scores -> re-ranked list" sequence can be captured in one CUDA graph.
+ *   _plan_topk plans one call on the device: the candidate-major schedule that the host planner (schedule.plan_chunks as one chunk +
+ *        build_attn_tiles) computes for cand int32 [Q,K], T = Q*K <= 16,384, 1 <= L <= 256, a cache of rows [row0, row0 + rows),
+ *        rows <= 2^18 - 2.  Outputs (device, T entries each unless noted):
+ *          flat_pos    the triplets q*K+k sorted by candidate, ties in q*K+k order (a stable sort)
+ *          kv_row      cand[flat_pos] - row0 (the cross-attention's kv_index)
+ *          trip_query  flat_pos / K
+ *          tiles       int32 [<= T][4] tcgen05 tile list for RB = the smallest power of two >= L (cir_attn_args.tiles)
+ *          tiles_cls   int32 [<= T][4] tile list for one query row per triplet (RB = 1)
+ *          counts      int32 [3]: number of tiles, number of cls tiles, number of invalid entries
+ *        An entry is invalid if it is negative (-1: the padding of a filtered search) or outside the cache's rows.  Invalid entries
+ *        sort after every valid one and read kv_row 0; nothing traps.  Bad shapes or a NULL pointer: CIR_EINVAL.
+ *   _rerank_cached runs _plan_topk, the stage-II scoring of all T triplets as one chunk through the cache (layer-0 dedup as in
+ *        cir_stage2_score; the cross-attentions read the device tile counts), scatters the scores to scores fp32 [Q,K] (-99999.99
+ *        at invalid entries, src/validate_stage2.py:123,258), sorts them with cir_rerank_sort into order int32 [Q,K] and, when
+ *        ranked is not NULL, writes ranked[q,r] = cand[q, order[q,r]].  z_t act [Q,L,768], ids / mask int32 [Q,L].  counts
+ *        (optional, int32 [3]) receives the plan's counts, so a caller can check the invalid entries after the fact.  Scores and
+ *        order equal those of the host-planned cir_stage2_score_cached call of the same single chunk, bit for bit.
+ *        PRECONDITION (not checked on the device): the cache was filled with the K/V weights of `w`.  Q*K > 16,384, K > 2048,
+ *        L > 256, a cache of the other dtype or of more than 2^18 - 2 rows, or a NULL z_t / ids / mask: CIR_EINVAL before anything
+ *        is enqueued.  workspace: _rerank_cached_workspace_bytes(Q, K, L, cache->num_tokens). */
+int    cir_stage2_plan_topk(cir_ctx* ctx, const int32_t* cand, int64_t Q, int64_t K, int64_t L, int64_t row0, int64_t rows,
+                            int32_t* flat_pos, int32_t* kv_row, int32_t* trip_query, int32_t* tiles, int32_t* tiles_cls, int32_t* counts);
+size_t cir_stage2_rerank_cached_workspace_bytes(const cir_ctx* ctx, int64_t Q, int64_t K, int64_t L, int64_t N);
+int    cir_stage2_rerank_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache, const int32_t* cand,
+                                int64_t Q, int64_t K, const void* z_t, const int32_t* ids, const int32_t* mask, int64_t L,
+                                float* scores, int32_t* order, int32_t* ranked, int32_t* counts, void* workspace, size_t workspace_bytes);
+
 
 /* ---- weight packing: reference state_dict tensors -> the packed structs above ------------------------------------------
  * A consumer that does not go through the Python host layer binds the reference's checkpoints here: every field of a
