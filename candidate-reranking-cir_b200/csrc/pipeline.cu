@@ -228,6 +228,29 @@ static int self_attention(cir_ctx* ctx, const void* hin, const void* wqkv, const
   return CIR_OK;
 }
 
+// self_attention for query row 0 (CLS) of each caption only; its keys/values still come from all L rows.  ctxout: [batch][caps]
+// rows.  K | V for all rows (weight rows 768..2303 -> qkv columns 768..2303), Q for the CLS rows only (A row stride L*768 ->
+// qkv row 0 of each caption).
+static int self_attention_cls(cir_ctx* ctx, const void* hin, const void* wqkv, const float* bqkv, int batch, const int32_t* mask,
+                              const int32_t* mask_index, int64_t caps, int64_t L, void* qkv, void* ctxout) {
+  const size_t es = act_size(ctx);
+  const int64_t Mr = caps * L;
+  CIR_TRY(gemm(ctx, hin, D, Mr * D, at(const_cast<void*>(wqkv), D * D, es), D, 3 * D * D, bqkv + D, 3 * D,
+               at(qkv, D, es), 3 * D, Mr * 3 * D, 0, nullptr, 0, 0, 0, Mr, 2 * D, D, batch, CIR_ACT_NONE));
+  CIR_TRY(gemm(ctx, hin, L * D, Mr * D, wqkv, D, 3 * D * D, bqkv, 3 * D, qkv, L * 3 * D, Mr * 3 * D, 0,
+               nullptr, 0, 0, 0, caps, D, D, batch, CIR_ACT_NONE));
+  for (int s = 0; s < batch; s++) {
+    cir_attn_args a{};
+    void* qkv_s = at(qkv, s * Mr * 3 * D, es);
+    a.q = qkv_s; a.k = at(qkv_s, D, es); a.v = at(qkv_s, 2 * D, es); a.o = at(ctxout, s * caps * D, es);
+    a.q_bs = a.k_bs = a.v_bs = L * 3 * D; a.q_rs = a.k_rs = a.v_rs = 3 * D; a.o_bs = D; a.o_rs = D;
+    a.key_mask = mask; a.mask_index = mask_index;
+    a.B = (int32_t)caps; a.H = CIR_HEADS; a.Lq = 1; a.Lk = (int32_t)L; a.scale = 0.125f;
+    CIR_TRY(cir_attention(ctx, &a));
+  }
+  return CIR_OK;
+}
+
 // ========================================================================================== ViT
 struct VitWs { void *patches, *patch_out, *x, *y, *qkv, *ctx, *f; size_t total; };
 static VitWs vit_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t B, int64_t S) {
@@ -489,49 +512,37 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
   }
   // stream 1 = embeddings (nlvr_encoder.py:880-886), stream 0 = z_t WITHOUT embedding LayerNorm (:892);
   // both expanded over the query's triplets (blip_stage2.py:118-124)
-  const int full_layers = ctx->prune_last ? CIR_LAYERS - 1 : CIR_LAYERS;
   // The inputs of layer 0 -- and with them its whole self-attention block and its cross-attention query projection --
   // depend on the QUERY only, not on the candidate (both streams are expanded copies, blip_stage2.py:118-124): run them
   // once per unique query of the chunk ([2][Q*L] rows) and expand the results over the triplets.  Exact.
+  static_assert(CIR_LAYERS >= 2, "layer 0 is never the CLS-only last layer");
   const bool prefixed = a0 != nullptr;
-  CIR_CHECK_ARG(!prefixed || (qc0 && full_layers >= 1), "stage2: a0 and qc0 come as a pair");
-  const bool dedup0 = prefixed || (ctx->dedup_first && full_layers >= 1 && Q <= T);
+  CIR_CHECK_ARG(!prefixed || qc0, "stage2: a0 and qc0 come as a pair");
+  const bool dedup0 = prefixed || (ctx->dedup_first && Q <= T);
   const int64_t Mq = Q * L;
+  // layer 0's a / qc rows of the Q queries, [2][Q*L] rows each: precomputed for the whole query set (cir_stage2_prefix) or
+  // computed here once per unique query (stage2_query_block)
+  const void* a_q = a0;
+  const void* q_q = qc0;
   if (prefixed) {
     // nothing to prepare: layer 0 starts from the expanded a0 / qc0 rows
   } else if (dedup0) {
     CIR_TRY(stage2_query_inputs(ctx, w, z_t, ids, Q, L, ws.h));
+    // a_q -> ws.pre, its pre-LayerNorm scratch -> ws.x, q_q -> ws.qkv (written after the self-attention has read the
+    // QKV rows); all are [2][Q*L] rows and Q <= T, so the [2][T*L]-row buffers hold them
+    CIR_TRY(stage2_query_block(ctx, w, ws.h, mask, Q, L, ws.qkv, ws.ctx, ws.x, ws.pre, ws.qkv));
+    a_q = ws.pre; q_q = ws.qkv;
   } else {
     CIR_TRY(cir_bert_embeddings(ctx, ids, Q, L, w->word_emb, w->pos_emb, w->emb_ln_g, w->emb_ln_b, ws.emb));
     CIR_TRY(cir_gather_rows(ctx, z_t, trip_query, ws.h, T, L * D));
     CIR_TRY(cir_gather_rows(ctx, ws.emb, trip_query, at(ws.h, M * D, es), T, L * D));
   }
-  for (int i = 0; i < full_layers; i++) {                                                                          // nlvr_encoder.py:506
-    const bool per_query = dedup0 && i == 0;
-    if (per_query) {
-      // ---- layer 0, once per unique query (stage2_query_block), or precomputed for the whole query set (cir_stage2_prefix):
-      const void* a_q = a0;
-      const void* q_q = qc0;
-      if (!prefixed) {
-        // a_q -> ws.pre, its pre-LayerNorm scratch -> ws.x, q_q -> ws.qkv (written after the self-attention has read the
-        // QKV rows); all are [2][Q*L] rows and Q <= T, so the [2][T*L]-row buffers hold them
-        CIR_TRY(stage2_query_block(ctx, w, ws.h, mask, Q, L, ws.qkv, ws.ctx, ws.x, ws.pre, ws.qkv));
-        a_q = ws.pre; q_q = ws.qkv;
-      }
-      for (int s = 0; s < 2; s++) {                           // expand over the triplets (blip_stage2.py:118-124)
-        CIR_TRY(cir_gather_rows(ctx, at(const_cast<void*>(a_q), s * Mq * D, es), trip_query, at(ws.a, s * M * D, es), T, L * D));
-        CIR_TRY(cir_gather_rows(ctx, at(const_cast<void*>(q_q), s * Mq * D, es), trip_query, at(ws.qc, s * M * D, es), T, L * D));
-      }
-    } else {
-    // ---- twin self-attention (:281-289, :346-363): separate weights per stream, shared padding mask (:774)
-    CIR_TRY(self_attention(ctx, ws.h, w->self_qkv_w[i], w->self_qkv_b[i], 2, mask, trip_query, T, L, ws.qkv, ws.ctx));
-    // a_s = LayerNorm{A,B}(dense_s(ctx_s) + h_s)   (:261-264)
-    CIR_TRY(gemm_layernorm(ctx, ws.ctx, D, M * D, w->self_out_w[i], D, D * D, w->self_out_b[i], D, ws.h, D, M * D,
-                           w->self_ln_g[i], w->self_ln_b[i], BERT_EPS, ws.pre, ws.a, M, D, 2));
-    // ---- twin cross-attention onto the SAME candidate tokens (:322-339)
-    CIR_TRY(gemm(ctx, ws.a, D, M * D, w->cross_q_w[i], D, D * D, w->cross_q_b[i], D, ws.qc, D, M * D, 0, nullptr, 0, 0, 0,
-                 M, D, D, 2, CIR_ACT_NONE));
-    }   // !per_query
+  // ---- layer i from its cross-attention on: twin cross-attention onto the SAME candidate tokens (:322-339), merge, FFN, over the
+  // [2][T*Lq] rows of ws.a / ws.qc (Lq query rows per triplet) into ws.h.  tiles / work / counts: the cross-attention's tile list,
+  // work list and device tile count for Lq-row queries.
+  auto cross_ffn = [&](int i, int64_t Lq, const int32_t* tiles, int64_t num_tiles, const int32_t* work, int64_t num_work,
+                       const int32_t* counts) -> int {
+    const int64_t R = T * Lq;
     // K/V projections once per candidate image: rows K0|V0|K1|V1 (:158-159)
     void* kv = cache ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
     if (!cache)
@@ -539,69 +550,52 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                    C * N, 4 * D, D, 1, CIR_ACT_NONE));
     for (int s = 0; s < 2; s++) {
       cir_attn_args c{};
-      c.q = at(ws.qc, s * M * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
+      c.q = at(ws.qc, s * R * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
       c.o = at(ws.ctxc, s * D, es);
-      c.q_bs = L * D; c.q_rs = D; c.k_bs = c.v_bs = N * 4 * D; c.k_rs = c.v_rs = 4 * D; c.o_bs = L * 2 * D; c.o_rs = 2 * D;
+      c.q_bs = Lq * D; c.q_rs = D; c.k_bs = c.v_bs = N * 4 * D; c.k_rs = c.v_rs = 4 * D; c.o_bs = Lq * 2 * D; c.o_rs = 2 * D;
       c.kv_index = kv_index;
-      c.work = attn_work; c.num_work = (int32_t)num_attn_work;
-      c.tiles = attn_tiles; c.num_tiles = (int32_t)num_attn_tiles; c.kv_batches = kv_batches;
-      c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = (int32_t)L; c.Lk = (int32_t)N; c.scale = 0.125f;
-      CIR_TRY(tile_counts ? cir_attention_counted(ctx, &c, tile_counts) : cir_attention(ctx, &c));
+      c.work = work; c.num_work = (int32_t)num_work;
+      c.tiles = tiles; c.num_tiles = (int32_t)num_tiles; c.kv_batches = kv_batches;
+      c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = (int32_t)Lq; c.Lk = (int32_t)N; c.scale = 0.125f;
+      CIR_TRY(counts ? cir_attention_counted(ctx, &c, counts) : cir_attention(ctx, &c));
     }
     // m = merge(dense0(c0), dense1(c1)) folded into one K=1536 GEMM (:250-258); x_s = LayerNorm{A,B}(m + a_s) (:256,:260)
     CIR_TRY(gemm(ctx, ws.ctxc, 2 * D, 0, w->cross_out_w[i], 2 * D, 0, w->cross_out_b[i], 0, ws.m, D, 0, 0, nullptr, 0, 0, 0,
-                 M, D, 2 * D, 1, CIR_ACT_NONE));
-    CIR_TRY(cir_add_layernorm(ctx, ws.m, 0, M, ws.a, w->cross_ln_g[i], w->cross_ln_b[i], M, ws.x, 0, 2 * M, BERT_EPS));
-    // ---- FFN, weights shared by both streams (:469-476): both streams as 2M rows
-    CIR_TRY(gemm(ctx, ws.x, D, 0, w->ffn1_w[i], D, 0, w->ffn1_b[i], 0, ws.f, F, 0, 0, nullptr, 0, 0, 0, 2 * M, F, D, 1, CIR_ACT_GELU));
-    CIR_TRY(gemm_layernorm(ctx, ws.f, F, 0, w->ffn2_w[i], F, 0, w->ffn2_b[i], 0, ws.x, D, 0, w->ffn_ln_g[i], w->ffn_ln_b[i], BERT_EPS,
-                           ws.pre, ws.h, 2 * M, F, 1));
-  }
-  if (ctx->prune_last) {
-    // ---- last layer, CLS rows only.  The encoder returns cat(h0[:,0,:], h1[:,0,:]) (nlvr_encoder.py:906-909), so
-    // in layer 11 only the query row 0 of each stream feeds the result; its keys/values still come from all L
-    // rows (self) and all N image tokens (cross).  Everything after the K/V projections runs on [2][T] rows.
-    const int i = CIR_LAYERS - 1;
-    // self K | V for all rows (weight rows 768..2303 -> qkv columns 768..2303), self Q for the CLS rows only (A row stride
-    // L*768 -> qkv row 0 of each triplet)
-    CIR_TRY(gemm(ctx, ws.h, D, M * D, at(const_cast<void*>(w->self_qkv_w[i]), D * D, es), D, 3 * D * D, w->self_qkv_b[i] + D, 3 * D,
-                 at(ws.qkv, D, es), 3 * D, M * 3 * D, 0, nullptr, 0, 0, 0, M, 2 * D, D, 2, CIR_ACT_NONE));
-    CIR_TRY(gemm(ctx, ws.h, L * D, M * D, w->self_qkv_w[i], D, 3 * D * D, w->self_qkv_b[i], 3 * D, ws.qkv, L * 3 * D, M * 3 * D, 0,
-                 nullptr, 0, 0, 0, T, D, D, 2, CIR_ACT_NONE));
-    for (int s = 0; s < 2; s++) {
-      cir_attn_args a{};
-      void* qkv_s = at(ws.qkv, s * M * 3 * D, es);
-      a.q = qkv_s; a.k = at(qkv_s, D, es); a.v = at(qkv_s, 2 * D, es); a.o = at(ws.ctx, s * T * D, es);
-      a.q_bs = a.k_bs = a.v_bs = L * 3 * D; a.q_rs = a.k_rs = a.v_rs = 3 * D; a.o_bs = D; a.o_rs = D;
-      a.key_mask = mask; a.mask_index = trip_query;
-      a.B = (int32_t)T; a.H = CIR_HEADS; a.Lq = 1; a.Lk = (int32_t)L; a.scale = 0.125f;
-      CIR_TRY(cir_attention(ctx, &a));
+                 R, D, 2 * D, 1, CIR_ACT_NONE));
+    CIR_TRY(cir_add_layernorm(ctx, ws.m, 0, R, ws.a, w->cross_ln_g[i], w->cross_ln_b[i], R, ws.x, 0, 2 * R, BERT_EPS));
+    // ---- FFN, weights shared by both streams (:469-476): both streams as 2R rows
+    CIR_TRY(gemm(ctx, ws.x, D, 0, w->ffn1_w[i], D, 0, w->ffn1_b[i], 0, ws.f, F, 0, 0, nullptr, 0, 0, 0, 2 * R, F, D, 1, CIR_ACT_GELU));
+    return gemm_layernorm(ctx, ws.f, F, 0, w->ffn2_w[i], F, 0, w->ffn2_b[i], 0, ws.x, D, 0, w->ffn_ln_g[i], w->ffn_ln_b[i], BERT_EPS,
+                          ws.pre, ws.h, 2 * R, F, 1);
+  };
+  for (int i = 0; i < CIR_LAYERS; i++) {                                                                           // nlvr_encoder.py:506
+    // With prune_last, layer 11 runs on the CLS rows only: the encoder returns cat(h0[:,0,:], h1[:,0,:]) (nlvr_encoder.py:906-909),
+    // so there only query row 0 of each stream feeds the result; its keys/values still come from all L rows (self) and all N image
+    // tokens (cross).
+    const bool cls = ctx->prune_last && i == CIR_LAYERS - 1;
+    const int64_t Lq = cls ? 1 : L, R = T * Lq;
+    if (dedup0 && i == 0) {
+      for (int s = 0; s < 2; s++) {                           // expand over the triplets (blip_stage2.py:118-124)
+        CIR_TRY(cir_gather_rows(ctx, at(const_cast<void*>(a_q), s * Mq * D, es), trip_query, at(ws.a, s * M * D, es), T, L * D));
+        CIR_TRY(cir_gather_rows(ctx, at(const_cast<void*>(q_q), s * Mq * D, es), trip_query, at(ws.qc, s * M * D, es), T, L * D));
+      }
+    } else {
+      // ---- twin self-attention (:281-289, :346-363): separate weights per stream, shared padding mask (:774)
+      if (cls)
+        CIR_TRY(self_attention_cls(ctx, ws.h, w->self_qkv_w[i], w->self_qkv_b[i], 2, mask, trip_query, T, L, ws.qkv, ws.ctx));
+      else
+        CIR_TRY(self_attention(ctx, ws.h, w->self_qkv_w[i], w->self_qkv_b[i], 2, mask, trip_query, T, L, ws.qkv, ws.ctx));
+      // a_s = LayerNorm{A,B}(dense_s(ctx_s) + h_s)   (:261-264)
+      CIR_TRY(gemm_layernorm(ctx, ws.ctx, D, R * D, w->self_out_w[i], D, D * D, w->self_out_b[i], D, ws.h, cls ? L * D : D, M * D,
+                             w->self_ln_g[i], w->self_ln_b[i], BERT_EPS, ws.pre, ws.a, R, D, 2));
+      CIR_TRY(gemm(ctx, ws.a, D, R * D, w->cross_q_w[i], D, D * D, w->cross_q_b[i], D, ws.qc, D, R * D, 0, nullptr, 0, 0, 0,
+                   R, D, D, 2, CIR_ACT_NONE));
     }
-    CIR_TRY(gemm(ctx, ws.ctx, D, T * D, w->self_out_w[i], D, D * D, w->self_out_b[i], D, ws.pre, D, T * D, 0, ws.h, L * D, M * D, 0,
-                 T, D, D, 2, CIR_ACT_NONE));
-    CIR_TRY(cir_add_layernorm(ctx, ws.pre, 0, 2 * T, nullptr, w->self_ln_g[i], w->self_ln_b[i], T, ws.a, 0, 2 * T, BERT_EPS));
-    CIR_TRY(gemm(ctx, ws.a, D, T * D, w->cross_q_w[i], D, D * D, w->cross_q_b[i], D, ws.qc, D, T * D, 0, nullptr, 0, 0, 0,
-                 T, D, D, 2, CIR_ACT_NONE));
-    void* kv = cache ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
-    if (!cache)
-      CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
-                   C * N, 4 * D, D, 1, CIR_ACT_NONE));
-    for (int s = 0; s < 2; s++) {
-      cir_attn_args c{};
-      c.q = at(ws.qc, s * T * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
-      c.o = at(ws.ctxc, s * D, es);
-      c.q_bs = D; c.q_rs = D; c.k_bs = c.v_bs = N * 4 * D; c.k_rs = c.v_rs = 4 * D; c.o_bs = 2 * D; c.o_rs = 2 * D;
-      c.kv_index = kv_index;
-      c.tiles = attn_tiles_cls; c.num_tiles = (int32_t)num_attn_tiles_cls; c.kv_batches = kv_batches;
-      c.B = (int32_t)T; c.H = CIR_HEADS; c.Lq = 1; c.Lk = (int32_t)N; c.scale = 0.125f;
-      CIR_TRY(tile_counts ? cir_attention_counted(ctx, &c, tile_counts + 1) : cir_attention(ctx, &c));
-    }
-    CIR_TRY(gemm(ctx, ws.ctxc, 2 * D, 0, w->cross_out_w[i], 2 * D, 0, w->cross_out_b[i], 0, ws.m, D, 0, 0, nullptr, 0, 0, 0,
-                 T, D, 2 * D, 1, CIR_ACT_NONE));
-    CIR_TRY(cir_add_layernorm(ctx, ws.m, 0, T, ws.a, w->cross_ln_g[i], w->cross_ln_b[i], T, ws.x, 0, 2 * T, BERT_EPS));
-    CIR_TRY(gemm(ctx, ws.x, D, 0, w->ffn1_w[i], D, 0, w->ffn1_b[i], 0, ws.f, F, 0, 0, nullptr, 0, 0, 0, 2 * T, F, D, 1, CIR_ACT_GELU));
-    CIR_TRY(gemm(ctx, ws.f, F, 0, w->ffn2_w[i], F, 0, w->ffn2_b[i], 0, ws.pre, D, 0, 0, ws.x, D, 0, 0, 2 * T, D, F, 1, CIR_ACT_NONE));
-    CIR_TRY(cir_add_layernorm(ctx, ws.pre, 0, 2 * T, nullptr, w->ffn_ln_g[i], w->ffn_ln_b[i], 2 * T, ws.h, 0, 2 * T, BERT_EPS));
+    // the mma.sync work list describes L-row units: the CLS layer gets none
+    if (cls)
+      CIR_TRY(cross_ffn(i, Lq, attn_tiles_cls, num_attn_tiles_cls, nullptr, 0, tile_counts ? tile_counts + 1 : nullptr));
+    else
+      CIR_TRY(cross_ffn(i, Lq, attn_tiles, num_attn_tiles, attn_work, num_attn_work, tile_counts));
   }
   // cat(CLS0, CLS1) (:909) -> cls_head (blip_stage2.py:50-54,134-136)
   CIR_TRY(cir_gather_cls(ctx, ws.h, T, ctx->prune_last ? 1 : L, ws.feats, feats));
