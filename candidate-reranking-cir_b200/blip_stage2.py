@@ -97,11 +97,12 @@ class BLIP_NLVR(nn.Module):
         self._need_weights()
         return self.engine.stage2_rerank_cached(self._w, kv_cache, z_t, ids, mask, cand_idx, out=out)
 
-    def kv_cache(self, gallery_tokens, row0: int = 0, rows: Optional[int] = None):
+    def kv_cache(self, gallery_tokens, row0: int = 0, rows: Optional[int] = None, fp8: bool = False):
         """The cross-attention K/V of gallery rows [row0, row0 + rows) under this model's weights, computed once
-        (engine.Stage2KVCache): 42.5 MB per 384 px image in bf16.  Pass it as ``kv_cache=`` to score_triplets / the drivers."""
+        (engine.Stage2KVCache): 42.5 MB per 384 px image in bf16, 21.9 MB with ``fp8=True`` (MXFP8: e4m3 with a power-of-two scale
+        per 32 channels, bf16 models only).  Pass it as ``kv_cache=`` to score_triplets / rerank_topk / the drivers."""
         self._need_weights()
-        return self.engine.stage2_kv_cache(self._w, gallery_tokens, row0, rows)
+        return self.engine.stage2_kv_cache(self._w, gallery_tokens, row0, rows, fp8=fp8)
 
     def forward(self, *a, **k):
         raise NotImplementedError("use img_embed / img_txt_fusion_val / img_txt_fusion (the reference defines no forward())")

@@ -133,6 +133,13 @@ int cir_attention_counted(cir_ctx* ctx, const cir_attn_args* a, const int32_t* n
 // stage2_plan.cu: the two kernels after the scoring of an on-device plan (cir_stage2_rerank_cached)
 int cir_stage2_scatter_scores(cir_ctx* ctx, const float* sorted, const int32_t* flat_pos, int64_t T, const int32_t* counts, float* scores);
 int cir_stage2_gather_ranked(cir_ctx* ctx, const int32_t* cand, const int32_t* order, int64_t Q, int64_t K, int32_t* ranked);
+// stage2_plan.cu: run numbers of a plan's sorted kv_row (slot), the run -> gallery row list and its device length
+int cir_stage2_kv_runs(cir_ctx* ctx, const int32_t* kv_row, const int32_t* counts, int64_t T, int64_t row0, int32_t* slot,
+                       int32_t* run_row, int32_t* n_runs);
+// kv_fp8.cu: MXFP8 K/V cache (CIR_KV_MXFP8) quantisation of bf16 [rows][3072] and dequantisation of one layer's candidate rows
+int cir_kv_mxfp8_quantize(cir_ctx* ctx, const void* src, int64_t rows, void* elems, uint8_t* scales);
+int cir_kv_mxfp8_dequant(cir_ctx* ctx, const cir_stage2_kv_cache* cache, int i, const int32_t* cand_list, int64_t C,
+                         const int32_t* count, void* dst);
 bool cir_qkv_attention_supported(const cir_ctx* ctx, int64_t L);   // qkv_attention.cu
 // stage1_topk_tc.cu: tensor-core candidate filter + exact fp32 re-check, per-query exact fallback on the device (never synchronises).
 // A gallery "view" is the fp32 rows, their bf16 copy and gmax = {max ||g||, max ||g - bf16(g)||} as float bits.

@@ -12,6 +12,7 @@ int cir_vit_assemble(cir_ctx* ctx, const float* patch, const float* cls, const f
 int cir_gather_cls(cir_ctx* ctx, const void* h, int64_t T, int64_t L, void* feats, float* feats_f32);
 int cir_head_dot(cir_ctx* ctx, const float* hidden, const float* w, const float* b, float* scores, int64_t rows);
 
+#include <algorithm>
 #include <vector>
 struct ProfState {
   std::vector<cudaEvent_t> ev;      // pairs: [2i] start, [2i+1] end
@@ -387,15 +388,25 @@ extern "C" int cir_stage1_gallery_embed(cir_ctx* ctx, const cir_stage1_weights* 
 }
 
 // ========================================================================================== stage II
-// cached = K/V read from a cir_stage2_kv_cache: no candidate tokens / K/V rows in the workspace, one int32 cache row per triplet
+// Where a stage-II call's cross-attention K/V come from:
+//   KV_PROJECT      the chunk's candidate tokens, gathered and projected per layer into the workspace
+//   KV_CACHE        a bf16 / fp32 cir_stage2_kv_cache, read in place: one int32 cache row per triplet in the workspace
+//   KV_CACHE_MXFP8  an MXFP8 cache: the K/V of the C candidates dequantised per layer into the workspace (the KV_PROJECT layout)
+enum KvSrc { KV_PROJECT, KV_CACHE, KV_CACHE_MXFP8 };
+static KvSrc kv_src(const cir_stage2_kv_cache* c) { return !c ? KV_PROJECT : c->dtype == CIR_KV_MXFP8 ? KV_CACHE_MXFP8 : KV_CACHE; }
+// a cache of the context's dtype, or an MXFP8 cache in a bf16 context
+static bool kv_cache_serves(const cir_ctx* ctx, const cir_stage2_kv_cache* c) {
+  return c->dtype == ctx->dtype || (c->dtype == CIR_KV_MXFP8 && ctx->dtype == CIR_DTYPE_BF16);
+}
+
 struct S2Ws { void *cand, *kv, *emb, *h, *qkv, *ctx, *pre, *a, *qc, *ctxc, *m, *x, *f, *feats; float *hid; int32_t* kv_row; size_t total; };
-static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64_t C, int64_t Q, int64_t L, int64_t N, bool cached = false) {
+static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64_t C, int64_t Q, int64_t L, int64_t N, KvSrc src = KV_PROJECT) {
   const size_t es = act_size(ctx);
   const int64_t M = T * L;
   Bump b(ws, bytes);
   S2Ws w;
-  w.cand = cached ? nullptr : b.take(C * N * D * es);
-  w.kv = cached ? nullptr : b.take(C * N * 4 * D * es);
+  w.cand = src == KV_PROJECT ? b.take(C * N * D * es) : nullptr;
+  w.kv = src == KV_CACHE ? nullptr : b.take(C * N * 4 * D * es);
   w.emb = b.take(Q * L * D * es);
   w.h = b.take(2 * M * D * es);
   w.qkv = b.take(2 * M * 3 * D * es);
@@ -409,7 +420,7 @@ static S2Ws s2_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t T, int64
   w.f = b.take(2 * M * F * es);
   w.feats = b.take(T * 2 * D * es);
   w.hid = (float*)b.take(T * D * 4);
-  w.kv_row = cached ? (int32_t*)b.take(T * 4) : nullptr;
+  w.kv_row = src == KV_CACHE ? (int32_t*)b.take(T * 4) : nullptr;
   w.total = align_up(b.off, 256);
   return w;
 }
@@ -476,10 +487,12 @@ static const void* kv_cache_layer(const cir_stage2_kv_cache* c, int i, size_t es
 }
 
 // cache == NULL: the chunk's candidate tokens are gathered and their K/V projected per layer into the workspace (attention reads
-// K/V batch trip_slot[t] of C); otherwise the K/V rows come from the cache (K/V batch kv_row[t] of cache->rows).
+// K/V batch trip_slot[t] of C); a bf16 / fp32 cache: the K/V rows come from the cache (K/V batch kv_row[t] of cache->rows); an
+// MXFP8 cache: the K/V of the C candidates are dequantised per layer into the workspace (K/V batch trip_slot[t] of C).
 // tile_counts (cached only; NULL from every host-planned caller): device {tiles, cls tiles} of an on-device plan
-// (cir_stage2_plan_topk).  trip_slot then holds each triplet's cache row, and attn_tiles / attn_tiles_cls hold at most T entries,
-// of which the two cross-attentions read as many as the device counts say.
+// (cir_stage2_plan_topk).  attn_tiles / attn_tiles_cls then hold at most T entries, of which the two cross-attentions read as many
+// as the device counts say, and trip_slot holds each triplet's cache row -- or, with an MXFP8 cache, its run number, cand_list the
+// runs' gallery rows and cand_count (device) how many of the C entries the plan filled.
 static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const void* gallery_tokens,
                              const int32_t* cand_list, int64_t C, const void* z_t, const int32_t* ids,
                              const int32_t* mask, int64_t Q, int64_t L, int64_t N,
@@ -489,24 +502,26 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                              const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                              float* scores, float* feats, void* workspace, size_t workspace_bytes,
                              const void* a0, const void* qc0,              // optional cir_stage2_prefix results of the Q queries
-                             const cir_stage2_kv_cache* cache, const int32_t* tile_counts = nullptr) {
+                             const cir_stage2_kv_cache* cache, const int32_t* tile_counts = nullptr,
+                             const int32_t* cand_count = nullptr) {
   if (T == 0) return CIR_OK;
   CIR_CHECK_ARG(C >= 1 && Q >= 1, "stage2: need at least one candidate and one query");
   CIR_CHECK_ARG(L >= 1 && L <= 512 && N >= 1 && N <= 1024, "stage2: L=%lld N=%lld out of range", (long long)L, (long long)N);
-  S2Ws ws = s2_plan(ctx, workspace, workspace_bytes, T, C, Q, L, N, cache != nullptr);
+  const KvSrc src = kv_src(cache);
+  S2Ws ws = s2_plan(ctx, workspace, workspace_bytes, T, C, Q, L, N, src);
   if (workspace_bytes < ws.total) { cir_set_error("stage2: workspace %zu < %zu", workspace_bytes, ws.total); return CIR_EWORKSPACE; }
   const size_t es = act_size(ctx);
   const int64_t M = T * L;
   const int32_t* kv_index = trip_slot;
   int32_t kv_batches = (int32_t)C;
-  if (cache && tile_counts) {
+  if (src == KV_CACHE && tile_counts) {
     kv_batches = (int32_t)cache->rows;               // trip_slot already holds the cache rows
-  } else if (cache) {
+  } else if (src == KV_CACHE) {
     stage2_kv_rows_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(cand_list, trip_slot, cache->row0, T, ws.kv_row);
     CIR_LAUNCH_CHECK(ctx);
     kv_index = ws.kv_row;
     kv_batches = (int32_t)cache->rows;
-  } else {
+  } else if (src == KV_PROJECT) {
     // candidate tokens of this chunk, contiguous [C*N, 768] (validate_stage2.py:251 gather, once per unique image)
     CIR_TRY(cir_gather_rows(ctx, gallery_tokens, cand_list, ws.cand, C, N * D));
   }
@@ -544,10 +559,12 @@ static int stage2_score_impl(cir_ctx* ctx, const cir_stage2_weights* w, const vo
                        const int32_t* counts) -> int {
     const int64_t R = T * Lq;
     // K/V projections once per candidate image: rows K0|V0|K1|V1 (:158-159)
-    void* kv = cache ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
-    if (!cache)
+    void* kv = src == KV_CACHE ? const_cast<void*>(kv_cache_layer(cache, i, es)) : ws.kv;
+    if (src == KV_PROJECT)
       CIR_TRY(gemm(ctx, ws.cand, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, ws.kv, 4 * D, 0, 0, nullptr, 0, 0, 0,
                    C * N, 4 * D, D, 1, CIR_ACT_NONE));
+    else if (src == KV_CACHE_MXFP8)
+      CIR_TRY(cir_kv_mxfp8_dequant(ctx, cache, i, cand_list, C, cand_count, ws.kv));
     for (int s = 0; s < 2; s++) {
       cir_attn_args c{};
       c.q = at(ws.qc, s * R * D, es); c.k = at(kv, s * 2 * D, es); c.v = at(kv, s * 2 * D + D, es);
@@ -640,17 +657,35 @@ extern "C" size_t cir_stage2_kv_cache_bytes(const cir_ctx* ctx, int64_t rows, in
   return align_up((size_t)CIR_LAYERS * rows * N * 4 * D * act_size(ctx), 256);
 }
 
+// MXFP8: one e4m3 byte per element plus one E8M0 byte per 32 elements
+extern "C" size_t cir_stage2_kv_cache_bytes_mxfp8(const cir_ctx*, int64_t rows, int64_t N) {
+  if (rows < 0 || N < 0) return 0;
+  return align_up((size_t)CIR_LAYERS * rows * N * (4 * D + 4 * D / 32), 256);
+}
+
+// the checks and record of _init / _init_mxfp8; `need` is the blob size of the cache format `fmt`
+static int kv_cache_init(const char* what, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N, size_t need, int fmt,
+                         cir_stage2_kv_cache* out) {
+  CIR_CHECK_ARG(out != nullptr, "%s: out is NULL", what);
+  CIR_CHECK_ARG(row0 >= 0 && rows >= 0 && row0 + rows <= (1ll << 31) && N >= 1 && N <= 1024,
+                "%s: bad range row0=%lld rows=%lld N=%lld", what, (long long)row0, (long long)rows, (long long)N);
+  CIR_CHECK_ARG(rows * N < (1ll << 31), "%s: rows * N must stay below 2^31 (attention row index)", what);
+  CIR_CHECK_ARG(rows == 0 || (blob && ((uintptr_t)blob & 255) == 0), "%s: blob must be 256-byte aligned", what);
+  CIR_CHECK_ARG(bytes >= need, "%s: blob %zu < %zu bytes", what, bytes, need);
+  out->row0 = row0; out->rows = rows; out->num_tokens = N; out->dtype = fmt; out->kv = blob;
+  return CIR_OK;
+}
+
 extern "C" int cir_stage2_kv_cache_init(cir_ctx* ctx, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N,
                                         cir_stage2_kv_cache* out) {
-  CIR_CHECK_ARG(out != nullptr, "stage2_kv_cache_init: out is NULL");
-  CIR_CHECK_ARG(row0 >= 0 && rows >= 0 && row0 + rows <= (1ll << 31) && N >= 1 && N <= 1024,
-                "stage2_kv_cache_init: bad range row0=%lld rows=%lld N=%lld", (long long)row0, (long long)rows, (long long)N);
-  CIR_CHECK_ARG(rows * N < (1ll << 31), "stage2_kv_cache_init: rows * N must stay below 2^31 (attention row index)");
-  const size_t need = cir_stage2_kv_cache_bytes(ctx, rows, N);
-  CIR_CHECK_ARG(rows == 0 || (blob && ((uintptr_t)blob & 255) == 0), "stage2_kv_cache_init: blob must be 256-byte aligned");
-  CIR_CHECK_ARG(bytes >= need, "stage2_kv_cache_init: blob %zu < %zu bytes", bytes, need);
-  out->row0 = row0; out->rows = rows; out->num_tokens = N; out->dtype = ctx->dtype; out->kv = blob;
-  return CIR_OK;
+  return kv_cache_init("stage2_kv_cache_init", blob, bytes, row0, rows, N, cir_stage2_kv_cache_bytes(ctx, rows, N), ctx->dtype, out);
+}
+
+extern "C" int cir_stage2_kv_cache_init_mxfp8(cir_ctx* ctx, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N,
+                                              cir_stage2_kv_cache* out) {
+  CIR_CHECK_ARG(ctx->dtype == CIR_DTYPE_BF16, "stage2_kv_cache_init_mxfp8: an MXFP8 cache needs a bf16 context (dtype %d)", ctx->dtype);
+  return kv_cache_init("stage2_kv_cache_init_mxfp8", blob, bytes, row0, rows, N, cir_stage2_kv_cache_bytes_mxfp8(ctx, rows, N),
+                       CIR_KV_MXFP8, out);
 }
 
 extern "C" int cir_stage2_kv_cache_fill(cir_ctx* ctx, const cir_stage2_weights* w, cir_stage2_kv_cache* cache, const void* tokens,
@@ -677,8 +712,56 @@ extern "C" int cir_stage2_kv_cache_fill(cir_ctx* ctx, const cir_stage2_weights* 
   return rc;
 }
 
+extern "C" size_t cir_stage2_kv_cache_fill_mxfp8_workspace_bytes(const cir_ctx*, const cir_stage2_kv_cache* cache, int64_t slice_rows) {
+  if (!cache || slice_rows < 0) return 0;
+  return align_up((size_t)slice_rows * cache->num_tokens * 4 * D * sizeof(bf16), 256);
+}
+
+extern "C" int cir_stage2_kv_cache_fill_mxfp8(cir_ctx* ctx, const cir_stage2_weights* w, cir_stage2_kv_cache* cache, const void* tokens,
+                                              int64_t first, int64_t n, void* workspace, size_t workspace_bytes) {
+  CIR_ENTER(ctx);
+  CIR_CHECK_ARG(w && cache, "stage2_kv_cache_fill_mxfp8: NULL weights or cache");
+  CIR_CHECK_ARG(cache->dtype == CIR_KV_MXFP8 && ctx->dtype == CIR_DTYPE_BF16,
+                "stage2_kv_cache_fill_mxfp8: cache format %d, context dtype %d (needs an MXFP8 cache and a bf16 context)", cache->dtype,
+                ctx->dtype);
+  CIR_CHECK_ARG(n >= 0 && first >= cache->row0 && first + n <= cache->row0 + cache->rows,
+                "stage2_kv_cache_fill_mxfp8: rows [%lld, %lld) outside the cache's [%lld, %lld)", (long long)first,
+                (long long)(first + n), (long long)cache->row0, (long long)(cache->row0 + cache->rows));
+  if (n == 0) return CIR_OK;
+  CIR_CHECK_ARG(tokens != nullptr, "stage2_kv_cache_fill_mxfp8: tokens is NULL");
+  const int64_t N = cache->num_tokens, rn = cache->rows * N;
+  const size_t row_bytes = (size_t)N * 4 * D * sizeof(bf16);
+  const int64_t slice = workspace ? std::min<int64_t>(n, (int64_t)(workspace_bytes / row_bytes)) : 0;
+  if (slice < 1) {
+    cir_set_error("stage2_kv_cache_fill_mxfp8: workspace %zu < %zu (one row)", workspace ? workspace_bytes : 0, row_bytes);
+    return CIR_EWORKSPACE;
+  }
+  uint8_t* elems = (uint8_t*)cache->kv;
+  uint8_t* scales = elems + CIR_LAYERS * rn * 4 * D;
+  // per slice and layer: the bf16 K/V of _fill (the pair tile whatever the slice is) into the workspace, then quantised
+  ctx->gemm_force_pair = 1;
+  int rc = CIR_OK;
+  for (int64_t s0 = 0; s0 < n && rc == CIR_OK; s0 += slice) {
+    const int64_t m = std::min(slice, n - s0), r = (first - cache->row0 + s0) * N;
+    const void* tok = at(const_cast<void*>(tokens), s0 * N * D, sizeof(bf16));
+    for (int i = 0; i < CIR_LAYERS && rc == CIR_OK; i++) {
+      rc = gemm(ctx, tok, D, 0, w->cross_kv_w[i], D, 0, w->cross_kv_b[i], 0, workspace, 4 * D, 0, 0, nullptr, 0, 0, 0, m * N, 4 * D, D, 1,
+                CIR_ACT_NONE);
+      if (rc == CIR_OK) rc = cir_kv_mxfp8_quantize(ctx, workspace, m * N, elems + (i * rn + r) * 4 * D, scales + (i * rn + r) * (4 * D / 32));
+    }
+  }
+  ctx->gemm_force_pair = 0;
+  return rc;
+}
+
+extern "C" size_t cir_stage2_kv_score_workspace_bytes(const cir_ctx* ctx, const cir_stage2_kv_cache* cache, int64_t T, int64_t C, int64_t Q,
+                                                      int64_t L) {
+  if (!cache) return 0;
+  return s2_plan(ctx, nullptr, 0, T, C, Q, L, cache->num_tokens, kv_src(cache)).total;
+}
+
 extern "C" size_t cir_stage2_score_cached_workspace_bytes(const cir_ctx* ctx, int64_t T, int64_t Q, int64_t L, int64_t N) {
-  return s2_plan(ctx, nullptr, 0, T, 0, Q, L, N, true).total;
+  return s2_plan(ctx, nullptr, 0, T, 0, Q, L, N, KV_CACHE).total;
 }
 
 extern "C" int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache,
@@ -691,7 +774,7 @@ extern "C" int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w
                                        float* scores, float* feats, void* workspace, size_t workspace_bytes) {
   CIR_ENTER(ctx);
   CIR_CHECK_ARG(cache != nullptr, "stage2_score_cached: cache is NULL");
-  CIR_CHECK_ARG(cache->dtype == ctx->dtype, "stage2_score_cached: cache dtype %d, context dtype %d", cache->dtype, ctx->dtype);
+  CIR_CHECK_ARG(kv_cache_serves(ctx, cache), "stage2_score_cached: cache format %d, context dtype %d", cache->dtype, ctx->dtype);
   CIR_CHECK_ARG(!a0 == !qc0, "stage2_score_cached: a0 and qc0 come as a pair");
   CIR_CHECK_ARG(T == 0 || a0 || (z_t && ids), "stage2_score_cached: z_t and ids are required without the a0 / qc0 prefix");
   CIR_CHECK_ARG(T == 0 || cache->rows >= 1, "stage2_score_cached: empty cache");
@@ -704,8 +787,12 @@ extern "C" int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w
 constexpr int64_t RERANK_MAX_T = 16384;          // one planning CTA (stage2_plan.cu)
 constexpr int64_t RERANK_MAX_K = 2048;           // cir_rerank_sort
 
-struct RerankWs { int32_t *flat_pos, *kv_row, *trip_query, *tiles, *tiles_cls, *counts; float* sorted; void* s2; size_t s2_bytes, total; };
-static RerankWs rerank_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t Q, int64_t K, int64_t L, int64_t N) {
+// slot / run_row / n_runs: MXFP8 caches only (cir_stage2_kv_runs), whose dequantised K/V of up to T runs sit in s2
+struct RerankWs {
+  int32_t *flat_pos, *kv_row, *trip_query, *tiles, *tiles_cls, *counts; float* sorted; void* s2; int32_t *slot, *run_row, *n_runs;
+  size_t s2_bytes, total;
+};
+static RerankWs rerank_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t Q, int64_t K, int64_t L, int64_t N, KvSrc src = KV_CACHE) {
   const int64_t T = Q * K;
   Bump b(ws, bytes);
   RerankWs w;
@@ -716,14 +803,22 @@ static RerankWs rerank_plan(const cir_ctx* ctx, void* ws, size_t bytes, int64_t 
   w.tiles_cls = (int32_t*)b.take(T * 16);
   w.counts = (int32_t*)b.take(3 * 4);
   w.sorted = (float*)b.take(T * 4);
-  w.s2_bytes = s2_plan(ctx, nullptr, 0, T, 0, Q, L, N, true).total;
+  w.s2_bytes = s2_plan(ctx, nullptr, 0, T, T, Q, L, N, src).total;
   w.s2 = b.take(w.s2_bytes);
+  const bool runs = src == KV_CACHE_MXFP8;
+  w.slot = runs ? (int32_t*)b.take(T * 4) : nullptr;
+  w.run_row = runs ? (int32_t*)b.take(T * 4) : nullptr;
+  w.n_runs = runs ? (int32_t*)b.take(4) : nullptr;
   w.total = align_up(b.off, 256);
   return w;
 }
 extern "C" size_t cir_stage2_rerank_cached_workspace_bytes(const cir_ctx* ctx, int64_t Q, int64_t K, int64_t L, int64_t N) {
   if (Q < 1 || K < 1 || L < 1 || N < 1) return 0;
   return rerank_plan(ctx, nullptr, 0, Q, K, L, N).total;
+}
+extern "C" size_t cir_stage2_kv_rerank_workspace_bytes(const cir_ctx* ctx, const cir_stage2_kv_cache* cache, int64_t Q, int64_t K, int64_t L) {
+  if (!cache || Q < 1 || K < 1 || L < 1 || cache->num_tokens < 1) return 0;
+  return rerank_plan(ctx, nullptr, 0, Q, K, L, cache->num_tokens, kv_src(cache)).total;
 }
 
 extern "C" int cir_stage2_rerank_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir_stage2_kv_cache* cache, const int32_t* cand,
@@ -732,22 +827,30 @@ extern "C" int cir_stage2_rerank_cached(cir_ctx* ctx, const cir_stage2_weights* 
                                         size_t workspace_bytes) {
   CIR_ENTER(ctx);
   CIR_CHECK_ARG(w && cache && cand && z_t && ids && mask && scores && order, "stage2_rerank_cached: NULL argument");
-  CIR_CHECK_ARG(cache->dtype == ctx->dtype, "stage2_rerank_cached: cache dtype %d, context dtype %d", cache->dtype, ctx->dtype);
+  CIR_CHECK_ARG(kv_cache_serves(ctx, cache), "stage2_rerank_cached: cache format %d, context dtype %d", cache->dtype, ctx->dtype);
   CIR_CHECK_ARG(cache->rows >= 1, "stage2_rerank_cached: empty cache");
   CIR_CHECK_ARG(Q >= 1 && K >= 1 && K <= RERANK_MAX_K && Q * K <= RERANK_MAX_T,
                 "stage2_rerank_cached: Q=%lld x K=%lld outside K <= %lld, Q*K <= %lld", (long long)Q, (long long)K,
                 (long long)RERANK_MAX_K, (long long)RERANK_MAX_T);
   CIR_CHECK_ARG(L >= 1 && L <= 256, "stage2_rerank_cached: L=%lld outside [1, 256]", (long long)L);
   CIR_CHECK_ARG(cache->rows < (1ll << 18) - 1, "stage2_rerank_cached: a cache of %lld rows (at most 2^18 - 2)", (long long)cache->rows);
-  const RerankWs ws = rerank_plan(ctx, workspace, workspace_bytes, Q, K, L, cache->num_tokens);
+  const KvSrc src = kv_src(cache);
+  const RerankWs ws = rerank_plan(ctx, workspace, workspace_bytes, Q, K, L, cache->num_tokens, src);
   if (workspace_bytes < ws.total) { cir_set_error("stage2_rerank_cached: workspace %zu < %zu", workspace_bytes, ws.total); return CIR_EWORKSPACE; }
   const int64_t T = Q * K;
   int32_t* cnt = counts ? counts : ws.counts;
   CIR_TRY(cir_stage2_plan_topk(ctx, cand, Q, K, L, cache->row0, cache->rows, ws.flat_pos, ws.kv_row, ws.trip_query, ws.tiles,
                                ws.tiles_cls, cnt));
-  // one chunk of all T triplets, in the plan's candidate-major order: C is unused with a cache and the tile lists are bounded by T
-  CIR_TRY(stage2_score_impl(ctx, w, nullptr, nullptr, T, z_t, ids, mask, Q, L, cache->num_tokens, ws.trip_query, ws.kv_row, T,
-                            nullptr, 0, ws.tiles, T, ws.tiles_cls, T, ws.sorted, nullptr, ws.s2, ws.s2_bytes, nullptr, nullptr, cache, cnt));
+  // one chunk of all T triplets, in the plan's candidate-major order: C is unused with a bf16 / fp32 cache and the tile lists are
+  // bounded by T.  An MXFP8 cache needs the chunk's unique candidates: the runs of the sorted cache rows, at most T.
+  const int32_t* trip_slot = ws.kv_row;
+  if (src == KV_CACHE_MXFP8) {
+    CIR_TRY(cir_stage2_kv_runs(ctx, ws.kv_row, cnt, T, cache->row0, ws.slot, ws.run_row, ws.n_runs));
+    trip_slot = ws.slot;
+  }
+  CIR_TRY(stage2_score_impl(ctx, w, nullptr, ws.run_row, T, z_t, ids, mask, Q, L, cache->num_tokens, ws.trip_query, trip_slot, T,
+                            nullptr, 0, ws.tiles, T, ws.tiles_cls, T, ws.sorted, nullptr, ws.s2, ws.s2_bytes, nullptr, nullptr, cache, cnt,
+                            ws.n_runs));
   CIR_TRY(cir_stage2_scatter_scores(ctx, ws.sorted, ws.flat_pos, T, cnt, scores));
   CIR_TRY(cir_rerank_sort(ctx, scores, Q, K, order));
   if (ranked) CIR_TRY(cir_stage2_gather_ranked(ctx, cand, order, Q, K, ranked));

@@ -137,6 +137,32 @@ __global__ void stage2_scatter_kernel(const float* __restrict__ sorted, const in
   if (i < T) scores[flat_pos[i]] = i < T - counts[2] ? sorted[i] : NEG_FILL;      // invalid entries trail the sorted list
 }
 
+// The unique-candidate list of a plan, for caches whose K/V are dequantised per chunk (CIR_KV_MXFP8).  kv_row holds the plan's
+// sorted cache rows, its first T - counts[2] entries valid: slot[t] = run number of t among them (invalid entries: 0),
+// run_row[r] = row0 + the cache row of run r, *n_runs = number of runs.  Without a valid entry run 0 is cache row 0, so every
+// slot names a dequantised row.
+__global__ void __launch_bounds__(PLAN_THREADS)
+stage2_kv_runs_kernel(const int32_t* __restrict__ kv_row, const int32_t* __restrict__ counts, int T, int64_t row0,
+                      int32_t* __restrict__ slot, int32_t* __restrict__ run_row, int32_t* __restrict__ n_runs) {
+  __shared__ int s_warp[32];
+  const int V = T - counts[2];
+  const int per = (T + PLAN_THREADS - 1) / PLAN_THREADS;
+  const int lo = min((int)threadIdx.x * per, T), hi = min(lo + per, T);
+  auto is_start = [&](int i) { return i < V && (i == 0 || kv_row[i] != kv_row[i - 1]); };
+  int starts = 0;
+  for (int i = lo; i < hi; i++) starts += is_start(i);
+  int total;
+  int r = block_scan_excl(starts, 0, SumOp{}, s_warp, &total) - 1;
+  for (int i = lo; i < hi; i++) {
+    if (is_start(i)) run_row[++r] = (int32_t)(row0 + kv_row[i]);
+    slot[i] = i < V ? r : 0;
+  }
+  if (threadIdx.x == 0) {
+    if (total == 0) run_row[0] = (int32_t)row0;
+    *n_runs = max(total, 1);
+  }
+}
+
 __global__ void stage2_gather_ranked_kernel(const int32_t* __restrict__ cand, const int32_t* __restrict__ order, int64_t n, int64_t K,
                                             int32_t* __restrict__ ranked) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -173,6 +199,13 @@ extern "C" int cir_stage2_plan_topk(cir_ctx* ctx, const int32_t* cand, int64_t Q
 
 int cir_stage2_scatter_scores(cir_ctx* ctx, const float* sorted, const int32_t* flat_pos, int64_t T, const int32_t* counts, float* scores) {
   stage2_scatter_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(sorted, flat_pos, T, counts, scores);
+  CIR_LAUNCH_CHECK(ctx);
+  return CIR_OK;
+}
+
+int cir_stage2_kv_runs(cir_ctx* ctx, const int32_t* kv_row, const int32_t* counts, int64_t T, int64_t row0, int32_t* slot,
+                       int32_t* run_row, int32_t* n_runs) {
+  stage2_kv_runs_kernel<<<1, PLAN_THREADS, 0, ctx->stream>>>(kv_row, counts, (int)T, row0, slot, run_row, n_runs);
   CIR_LAUNCH_CHECK(ctx);
   return CIR_OK;
 }

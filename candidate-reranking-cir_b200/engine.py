@@ -19,6 +19,10 @@ from .schedule import build_attn_tiles, build_attn_work, plan_chunks
 HIDDEN, FFN, LAYERS, EMBED = 768, 3072, 12, 256
 NEG_FILL = -99999.99          # src/validate_stage2.py:123,258
 RERANK_MAX_TRIPLETS = 16384   # triplets per cir_stage2_rerank_cached call (one planning CTA)
+# triplets per cir_stage2_rerank_cached call through an MXFP8 cache: the call dequantises the K/V of up to T candidates into its
+# workspace (T * N * 3072 bf16), which this bounds to 7.3 GB at N = 577
+RERANK_FP8_MAX_TRIPLETS = 2048
+KV_FILL_SLICE_ROWS = 16       # gallery rows per slice of an MXFP8 fill (bf16 K/V workspace: 56.7 MB at N = 577)
 
 
 class Engine:
@@ -315,7 +319,8 @@ class Engine:
         ``attn_work``: optional int32 [W,4] K/V-sharing work list (schedule.build_attn_work).
         ``prefix``: optional (a0, qc0) from :meth:`stage2_prefix` for the same Q queries as ids/mask (z_t is then unused).
         ``kv_cache``: optional :class:`Stage2KVCache` holding every candidate of ``cand_list`` (cir_stage2_score_cached; not checked
-        here -- :meth:`stage2_score_pairs` checks it); ``gallery_tokens`` is then unused and may be None."""
+        here -- :meth:`stage2_score_pairs` checks it); ``gallery_tokens`` is then unused and may be None.  An MXFP8 cache puts the
+        dequantised K/V of the C candidates in the workspace, as the uncached path does with its projections."""
         cand_list, ids, mask = self._i32(cand_list), self._i32(ids), self._i32(mask)
         trip_query, trip_slot = self._i32(trip_query), self._i32(trip_slot)
         T, Cn, (Q, L) = trip_query.numel(), cand_list.numel(), ids.shape
@@ -326,7 +331,7 @@ class Engine:
             assert gallery_tokens.dtype == self.act_dtype and gallery_tokens.is_contiguous()
             need = self._lib.cir_stage2_workspace_bytes(self.ctx, T, Cn, Q, L, n_tok)
         else:
-            need = self._lib.cir_stage2_score_cached_workspace_bytes(self.ctx, T, Q, L, kv_cache.num_tokens)
+            need = self._lib.cir_stage2_kv_score_workspace_bytes(self.ctx, C.byref(kv_cache._s), T, Cn, Q, L)
         scores = torch.empty(T, dtype=torch.float32, device=self.device) if out is None else out
         assert scores.is_contiguous() and scores.numel() == T and scores.dtype == torch.float32
         feats = torch.empty(T, 2 * HIDDEN, dtype=torch.float32, device=self.device) if want_feats else None
@@ -414,7 +419,8 @@ class Engine:
         rank's contiguous candidate range (schedule.candidate_partition): every candidate's K/V projections stay on ONE rank,
         so the per-GPU K/V reuse does not fall with the number of GPUs.  z_t act [Q,L,768] / ids / mask [Q,L] cover ALL Q queries.
         ``kv_cache``: a :class:`Stage2KVCache` filled with ``w`` that holds every candidate this process scores: the chunks then
-        read their K/V from it (cir_stage2_score_cached) and are bounded by ``max_triplets`` only.  It is checked against ``w``,
+        read their K/V from it (cir_stage2_score_cached) and are bounded by ``max_triplets`` only -- an MXFP8 cache (``fp8=True``)
+        also by ``max_candidates``, as its dequantised K/V live in the workspace.  It is checked against ``w``,
         the token count of ``gallery_tokens`` and the candidates before anything launches (CirError).
         -> (flat_pos int64 [n] = q*K+k of each scored triplet, scores fp32 [n]) on the device."""
         cand_np = cand_idx.cpu().numpy() if isinstance(cand_idx, torch.Tensor) else np.asarray(cand_idx)
@@ -425,8 +431,8 @@ class Engine:
         info: dict = {}
         if kv_cache is not None:
             kv_cache._check_use(self, w, gallery_tokens.shape[1])
-        # the cached path keeps no per-chunk K/V, so nothing bounds the unique candidates of a chunk
-        max_cand = self.max_candidates if kv_cache is None else max(1, Q * K)
+        # a bf16 / fp32 cache keeps no per-chunk K/V, so nothing bounds the unique candidates of a chunk
+        max_cand = self.max_candidates if kv_cache is None or kv_cache.fp8 else max(1, Q * K)
         chunks = plan_chunks(cand_np, act_np, self.max_triplets, max_cand, part=part, info=info)
         if kv_cache is not None and chunks:
             kv_cache._check_rows(min(int(c.cand_list[0]) for c in chunks), max(int(c.cand_list[-1]) for c in chunks))
@@ -481,7 +487,8 @@ class Engine:
 
         The scores equal stage2_score_matrix(..., kv_cache=kv_cache) when that runs as one chunk, bit for bit.  Entries of -1 (the
         padding of a filtered search) or outside the cache's rows score -99999.99 and rank last.  Query sets larger than
-        max(1, max_triplets // K) queries go through several calls; none synchronises.  The cache is checked against ``w`` on the
+        max(1, max_triplets // K) queries (through an MXFP8 cache: at most RERANK_FP8_MAX_TRIPLETS triplets per call) go through
+        several calls; none synchronises.  The cache is checked against ``w`` on the
         host, the candidates are not (they stay on the device).  ``out``: optional (scores, order, ranked) to fill; with device
         int32 cand / ids / mask and ``out``, a warmed-up call allocates and uploads nothing."""
         kv_cache._check_use(self, w, kv_cache.num_tokens)
@@ -496,8 +503,8 @@ class Engine:
         scores, order, ranked = out
         assert scores.shape == order.shape == ranked.shape == (Q, K) and scores.dtype == torch.float32
         assert order.dtype == ranked.dtype == torch.int32 and all(t.is_contiguous() for t in out)
-        qb = max(1, min(self.max_triplets, RERANK_MAX_TRIPLETS) // K)
-        need = self._lib.cir_stage2_rerank_cached_workspace_bytes(self.ctx, min(qb, Q), K, L, kv_cache.num_tokens)
+        qb = max(1, min(self.max_triplets, RERANK_FP8_MAX_TRIPLETS if kv_cache.fp8 else RERANK_MAX_TRIPLETS) // K)
+        need = self._lib.cir_stage2_kv_rerank_workspace_bytes(self.ctx, C.byref(kv_cache._s), min(qb, Q), K, L)
         if self._rr_ws is None or self._rr_ws.numel() < need:
             if self._rr_ws is not None:
                 self._rr_retired.append(self._rr_ws)
@@ -546,14 +553,16 @@ class Engine:
                                           N.ptr(ti), N.ptr(ws), ws.numel()), "cir_stage1_topk")
         return td, ti
 
-    def stage2_kv_cache(self, w, gallery_tokens: torch.Tensor, row0: int = 0, rows: Optional[int] = None) -> "Stage2KVCache":
+    def stage2_kv_cache(self, w, gallery_tokens: torch.Tensor, row0: int = 0, rows: Optional[int] = None,
+                        fp8: bool = False) -> "Stage2KVCache":
         """A resident cross-attention K/V gallery (cir_stage2_kv_cache) of gallery rows [row0, row0 + rows) (default: to the end of
-        ``gallery_tokens``, act [G,N,768]), filled with the packed stage-II weights ``w``: 42.5 MB per image in bf16 at N = 577."""
+        ``gallery_tokens``, act [G,N,768]), filled with the packed stage-II weights ``w``: 42.5 MB per image in bf16 at N = 577,
+        21.9 MB with ``fp8=True`` (MXFP8, bf16 engines only)."""
         G, n_tok = gallery_tokens.shape[0], gallery_tokens.shape[1]
         rows = G - row0 if rows is None else rows
         if row0 < 0 or rows < 0 or row0 + rows > G:
             raise N.CirError(f"stage2_kv_cache: rows [{row0}, {row0 + rows}) outside the gallery's [0, {G})")
-        cache = Stage2KVCache(self, w, rows, n_tok, row0=row0)
+        cache = Stage2KVCache(self, w, rows, n_tok, row0=row0, fp8=fp8)
         return cache.fill(gallery_tokens[row0:row0 + rows], row0)
 
     def stage1_index(self, capacity: int) -> "Stage1Index":
@@ -705,18 +714,24 @@ class Stage2KVCache:
     per-chunk token gather and K/V GEMMs (32.7 GF per candidate load) and return the same scores bit for bit.
 
     The cache remembers the packed weights it is filled with (``weights``; their blob must stay alive, as for any scoring call)
-    and refuses to serve other weights.  ``blob``: optional caller-provided uint8 device tensor of at least ``nbytes``."""
+    and refuses to serve other weights.  ``blob``: optional caller-provided uint8 device tensor of at least ``nbytes``.
 
-    def __init__(self, eng: Engine, w, rows: int, num_tokens: int, row0: int = 0, blob: Optional[torch.Tensor] = None):
-        self.eng, self.weights = eng, w
+    ``fp8=True`` (bf16 engines): the MXFP8 format (CIR_KV_MXFP8) -- e4m3 elements with a power-of-two scale per 32 channels, half
+    the bytes.  Scores through it equal those through a bf16 cache holding its exactly dequantised K/V; every scoring call and the
+    online path take it unchanged."""
+
+    def __init__(self, eng: Engine, w, rows: int, num_tokens: int, row0: int = 0, blob: Optional[torch.Tensor] = None,
+                 fp8: bool = False):
+        self.eng, self.weights, self.fp8 = eng, w, bool(fp8)
         self._key = _kv_weights_key(w)
-        need = eng._lib.cir_stage2_kv_cache_bytes(eng.ctx, rows, num_tokens)
+        sfx = "_mxfp8" if self.fp8 else ""
+        need = getattr(eng._lib, "cir_stage2_kv_cache_bytes" + sfx)(eng.ctx, rows, num_tokens)
         self._blob = torch.empty(max(need, 256), dtype=torch.uint8, device=eng.device) if blob is None else blob
         if self._blob.device != eng.device or self._blob.dtype != torch.uint8:
             raise N.CirError(f"Stage2KVCache: the blob must be a uint8 tensor on {eng.device}")
         self._s = N.Stage2KVCache()
-        N.check(eng._lib.cir_stage2_kv_cache_init(eng.ctx, N.ptr(self._blob), self._blob.numel(), row0, rows, num_tokens,
-                                                  C.byref(self._s)), "cir_stage2_kv_cache_init")
+        N.check(getattr(eng._lib, "cir_stage2_kv_cache_init" + sfx)(eng.ctx, N.ptr(self._blob), self._blob.numel(), row0, rows,
+                                                                    num_tokens, C.byref(self._s)), "cir_stage2_kv_cache_init" + sfx)
 
     @property
     def row0(self) -> int:
@@ -732,12 +747,18 @@ class Stage2KVCache:
 
     @property
     def nbytes(self) -> int:
-        """Bytes of K/V the cache holds (12 layers x rows x N x 3072 activations)."""
-        return int(self.eng._lib.cir_stage2_kv_cache_bytes(self.eng.ctx, self.rows, self.num_tokens))
+        """Bytes of K/V the cache holds (12 layers x rows x N x 3072 activations, or e4m3 bytes + one scale byte per 32)."""
+        fn = self.eng._lib.cir_stage2_kv_cache_bytes_mxfp8 if self.fp8 else self.eng._lib.cir_stage2_kv_cache_bytes
+        return int(fn(self.eng.ctx, self.rows, self.num_tokens))
 
-    def layer(self, i: int) -> torch.Tensor:
-        """View of layer i's K/V rows: act [rows * N, 3072] (K0 | V0 | K1 | V1 columns)."""
+    def layer(self, i: int):
+        """View of layer i's K/V rows: act [rows * N, 3072] (K0 | V0 | K1 | V1 columns); for an MXFP8 cache the pair
+        (elements float8_e4m3fn [rows * N, 3072], scales uint8 [rows * N, 96]), scale j covering channels 32j .. 32j + 31."""
         n = self.rows * self.num_tokens * 4 * HIDDEN
+        if self.fp8:
+            e = self._blob[i * n:(i + 1) * n].view(torch.float8_e4m3fn).view(-1, 4 * HIDDEN)
+            s0 = LAYERS * n + i * (n // 32)
+            return e, self._blob[s0:s0 + n // 32].view(-1, 4 * HIDDEN // 32)
         es = 2 if self.eng.act_dtype == torch.bfloat16 else 4
         return self._blob[i * n * es:(i + 1) * n * es].view(self.eng.act_dtype).view(self.rows * self.num_tokens, 4 * HIDDEN)
 
@@ -751,6 +772,14 @@ class Stage2KVCache:
         if tokens.dtype != eng.act_dtype or tokens.device != eng.device:
             raise N.CirError(f"Stage2KVCache.fill: tokens must be {eng.act_dtype} on {eng.device}")
         t = tokens.contiguous()
+        if self.fp8:
+            # the fill's own slice workspace: Engine.workspace may be in use by a captured graph
+            ws = torch.empty(max(256, eng._lib.cir_stage2_kv_cache_fill_mxfp8_workspace_bytes(
+                eng.ctx, C.byref(self._s), min(t.shape[0], KV_FILL_SLICE_ROWS))), dtype=torch.uint8, device=eng.device)
+            eng._sync_stream()
+            N.check(eng._lib.cir_stage2_kv_cache_fill_mxfp8(eng.ctx, C.byref(self.weights), C.byref(self._s), N.ptr(t), first, t.shape[0],
+                                                            N.ptr(ws), ws.numel()), "cir_stage2_kv_cache_fill_mxfp8")
+            return self
         eng._sync_stream()
         N.check(eng._lib.cir_stage2_kv_cache_fill(eng.ctx, C.byref(self.weights), C.byref(self._s), N.ptr(t), first, t.shape[0]),
                 "cir_stage2_kv_cache_fill")

@@ -13,6 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CIR_B200_LIB") or os.path.join(HERE, "csrc", "libcir_b200.so")   # override: A/B of kernel builds
 
 DTYPE_F32, DTYPE_BF16 = 0, 1
+KV_MXFP8 = 2                  # cir_stage2_kv_cache.dtype of an MXFP8 K/V cache
 GEMM_AUTO, GEMM_SIMT, GEMM_TCGEN05, GEMM_TCGEN05_1CTA = 0, 1, 2, 3
 ACT_NONE, ACT_GELU, ACT_RELU = 0, 1, 2
 PROF_GEMM, PROF_ATTN_TC, PROF_ATTN_SELF, PROF_LAYERNORM, PROF_QKV_ATTN = 0, 1, 2, 3, 4
@@ -186,6 +187,12 @@ _SIGS = {
     "cir_stage2_score_cached_workspace_bytes": (C.c_size_t, [vp, i64, i64, i64, i64]),
     "cir_stage2_score_cached": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, vp, vp, vp, vp, vp, i64, i64,
                                           vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, vp, vp, C.c_size_t]),
+    "cir_stage2_kv_cache_bytes_mxfp8": (C.c_size_t, [vp, i64, i64]),
+    "cir_stage2_kv_cache_init_mxfp8": (C.c_int, [vp, vp, C.c_size_t, i64, i64, i64, C.POINTER(Stage2KVCache)]),
+    "cir_stage2_kv_cache_fill_mxfp8_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage2KVCache), i64]),
+    "cir_stage2_kv_cache_fill_mxfp8": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, i64, vp, C.c_size_t]),
+    "cir_stage2_kv_score_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage2KVCache), i64, i64, i64, i64]),
+    "cir_stage2_kv_rerank_workspace_bytes": (C.c_size_t, [vp, C.POINTER(Stage2KVCache), i64, i64, i64]),
     "cir_stage2_plan_topk": (C.c_int, [vp, vp, i64, i64, i64, i64, i64, vp, vp, vp, vp, vp, vp]),
     "cir_stage2_rerank_cached_workspace_bytes": (C.c_size_t, [vp, i64, i64, i64, i64]),
     "cir_stage2_rerank_cached": (C.c_int, [vp, C.POINTER(Stage2Weights), C.POINTER(Stage2KVCache), vp, i64, i64, vp, vp, vp, i64,

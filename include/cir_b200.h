@@ -423,7 +423,7 @@ int cir_stage2_score_prefixed(cir_ctx* ctx, const cir_stage2_weights* w, const v
 typedef struct cir_stage2_kv_cache {
   int64_t row0, rows;     /* gallery rows [row0, row0 + rows) */
   int64_t num_tokens;     /* N (577 at 384 px) */
-  int32_t dtype;          /* CIR_DTYPE_* of the context that initialised it */
+  int32_t dtype;          /* CIR_DTYPE_* of the context that initialised it, or CIR_KV_MXFP8 (below) */
   void*   kv;             /* act dtype, per layer i: [rows * N][3072] = K0|V0|K1|V1, at kv + i * rows * N * 3072 */
 } cir_stage2_kv_cache;
 size_t cir_stage2_kv_cache_bytes(const cir_ctx* ctx, int64_t rows, int64_t N);
@@ -445,6 +445,37 @@ int cir_stage2_score_cached(cir_ctx* ctx, const cir_stage2_weights* w, const cir
                             const int32_t* attn_work, int64_t num_attn_work, const int32_t* attn_tiles, int64_t num_attn_tiles,
                             const int32_t* attn_tiles_cls, int64_t num_attn_tiles_cls,
                             float* scores, float* feats, void* workspace, size_t workspace_bytes);
+
+/* MXFP8 K/V gallery: the same K0|V0|K1|V1 rows in 8-bit floating point with one power-of-two scale per 32 channels, half the bytes of
+ * a bf16 cache (21.9 MB per image at N = 577 against 42.5 MB), so twice as many gallery images fit one GPU.  A cache format, not a
+ * context dtype: cir_stage2_kv_cache.dtype = CIR_KV_MXFP8, in bf16 contexts only (fp32 context: CIR_EINVAL).  Blob layout:
+ *   elements  per layer i: uint8 [rows * N][3072] e4m3 (OCP e4m3fn: no infinities, max 448), row (r - row0) * N + t as in the bf16
+ *             cache, at kv + i * rows * N * 3072 bytes
+ *   scales    after the 12 element layers, per layer i: uint8 [rows * N][96] E8M0 (2^(b - 127)) of channels 32j .. 32j + 31, at
+ *             kv + 12 * rows * N * 3072 + i * rows * N * 96 bytes
+ * Quantisation of the bf16 K/V x the fill GEMM writes (the bytes a bf16 cache would hold): per block of 32 channels with largest
+ * magnitude amax, k = max(-127, smallest integer with amax <= 448 * 2^k) (amax = 0: k = -127), element e4m3_rne(x * 2^-k) (exact
+ * in fp32, never above 448), scale byte k + 127.  Dequantisation bf16(float(e) * 2^k) is exact.
+ *   _bytes_mxfp8 / _init_mxfp8  as their bf16 twins (same range, alignment and size checks).
+ *   _fill_mxfp8 projects rows [first, first + n) in slices that fit the workspace (_fill_mxfp8_workspace_bytes of slice_rows rows;
+ *        at least one row): per slice and layer the cross_kv_w GEMM (pair tile, as _fill) writes bf16 into the workspace and one
+ *        kernel quantises it into the cache.  A row's bytes do not depend on the slicing.  Workspace too small for one row:
+ *        CIR_EWORKSPACE.  cir_stage2_kv_cache_fill rejects an MXFP8 cache (CIR_EINVAL) and this one any other.
+ * Scoring: cir_stage2_score_cached and cir_stage2_rerank_cached accept an MXFP8 cache.  Per layer one kernel dequantises the K/V of
+ * the chunk's unique candidates into the workspace (C * N * 3072 bf16; C <= T on the device-planned path) and the cross-attentions
+ * read them as in cir_stage2_score.  Scores equal those through a bf16 cache holding the dequantised K/V, bit for bit.  Size the
+ * workspaces with the cache-aware functions below, which return the older functions' values for bf16 and fp32 caches. */
+#define CIR_KV_MXFP8 2
+size_t cir_stage2_kv_cache_bytes_mxfp8(const cir_ctx* ctx, int64_t rows, int64_t N);
+int    cir_stage2_kv_cache_init_mxfp8(cir_ctx* ctx, void* blob, size_t bytes, int64_t row0, int64_t rows, int64_t N,
+                                      cir_stage2_kv_cache* out);
+size_t cir_stage2_kv_cache_fill_mxfp8_workspace_bytes(const cir_ctx* ctx, const cir_stage2_kv_cache* cache, int64_t slice_rows);
+int    cir_stage2_kv_cache_fill_mxfp8(cir_ctx* ctx, const cir_stage2_weights* w, cir_stage2_kv_cache* cache, const void* tokens,
+                                      int64_t first, int64_t n, void* workspace, size_t workspace_bytes);
+/* workspace of cir_stage2_score_cached (T triplets, C unique candidates, Q queries) / cir_stage2_rerank_cached (Q x K) with `cache` */
+size_t cir_stage2_kv_score_workspace_bytes(const cir_ctx* ctx, const cir_stage2_kv_cache* cache, int64_t T, int64_t C, int64_t Q,
+                                           int64_t L);
+size_t cir_stage2_kv_rerank_workspace_bytes(const cir_ctx* ctx, const cir_stage2_kv_cache* cache, int64_t Q, int64_t K, int64_t L);
 
 /* Re-ranking a top-K list that lives on the device (e.g. the top_idx of cir_stage1_index_topk) through a filled K/V cache, with no
  * host round trip: every call below only enqueues kernels, never synchronises and never touches host memory, so the whole
